@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # CPU arm: the oracle port on the host cores
+    python bench.py ... --dump-outputs DIR                    # + what the last timed step computed, as DIR/*.npy
 
 One "step" = one pass of the hot path over the rank's whole batch: the on-device random-valid
 policy (`sy_sample_actions`) + `sy_step` (dynamics, budgets/tolls, capture/termination, rewards,
@@ -106,6 +107,37 @@ class ClockSampler:
         self.stop = True
         return {"sm_mhz": statistics.median(self.samples) if self.samples else None, "sm_max_mhz": self.max_mhz,
                 "reasons": sorted(self.reasons), "samples": len(self.samples)}
+
+
+DUMP_BYTES = 48 << 20  # per-env arrays of --dump-outputs: one sample of envs, sized to stay under 64 MB in all
+
+
+def dump_outputs(out_dir, env, actions, stats):
+    """`--dump-outputs DIR`: what the timed path hands its caller after its last step, as DIR/<name>.npy, so that two
+    builds run with the same arguments can be compared output for output.  Per-env arrays (the policy's actions, the
+    step's reward and flags, the dynamic observation entries) are float32 rows of a fixed, seeded sample of envs whose
+    indices are `env_index`; `episode_stats` (float64, named by STAT_NAMES) covers the whole batch."""
+    import numpy as np
+    import torch
+
+    from student_mechanism_design_b200._cabi import STAT_NAMES
+
+    obs = env.observation()
+    per_env = {"actions": actions, "reward": env.reward, "terminated": env.terminated, "truncated": env.truncated,
+               "done": env.done_flags, "winner": env.winner}
+    for k in ("agent_position", "Currency", "agent_budget", "MrX_revealed", "graph_id", "action_mask", "node_features",
+              "belief_map"):
+        if k in obs:
+            per_env[k] = obs[k]
+    B = env.num_envs
+    n = min(B, DUMP_BYTES // sum(4 * t[0].numel() for t in per_env.values()))
+    idx = np.sort(np.random.default_rng(0).choice(B, size=n, replace=False))
+    sel = torch.from_numpy(idx).to(env.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in per_env.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.index_select(0, sel).float().cpu().numpy())
+    np.save(os.path.join(out_dir, "env_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "episode_stats.npy"), np.asarray([stats[k] for k in STAT_NAMES], dtype=np.float64))
 
 
 # --------------------------------------------------------------------------------------------
@@ -371,6 +403,8 @@ def run_cuda_arm(args, wl):
     ev1.record()
     barrier()
     stats_ms = max_over_ranks(ev0.elapsed_time(ev1))
+    if args.dump_outputs and rank == 0:  # before the roofline steps below move the env on
+        dump_outputs(args.dump_outputs, env, actions, stats_total)
 
     # ---- duration of the sy_step call alone (its two kernels), CUDA events around every call, for the roofline
     Kk = min(K, 300)
@@ -582,10 +616,14 @@ def main():
                     help="issue the timed steps with one sy_rollout_random call instead of replaying a captured CUDA graph of "
                          "50-step segments (the default for the random policy: no launch gaps between the kernels)")
     ap.add_argument("--python-loop", action="store_true", help="issue every step from Python instead of sy_rollout_random")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed passes, write what their last step computed as DIR/<name>.npy (CUDA arm, rank 0)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     wl = dict(WORKLOADS[args.workload], name=args.workload)
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of the CUDA arm")
         run_reference_arm(args, wl)
     else:
         run_cuda_arm(args, wl)

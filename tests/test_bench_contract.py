@@ -1,7 +1,12 @@
-"""CPU checks of bench.py's accounting and of the committed bench lines (the contract of the driver's JSON line)."""
+"""Checks of bench.py: its accounting and the committed bench lines (the contract of its JSON line) on the CPU, the
+outputs it dumps on the GPU."""
 import importlib.util
 import json
 import os
+import subprocess
+import sys
+
+import pytest
 
 from conftest import ROOT
 
@@ -73,3 +78,51 @@ def test_round2_bench_lines_carry_the_contract_keys():
     ref = json.loads(open(os.path.join(ROOT, "profiles", "r02_bench_c3_reference_arm.json")).read().strip().splitlines()[-1])
     assert ref["impl"] == "reference" and ref["e2e"]["h2d_bytes_per_step"] == 0 and ref["cpu_baseline"]["kind"] == "port"
     assert ref["config"]["envs_per_gpu"] == n1["config"]["envs_per_gpu"]  # the CPU arm steps the same batch
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_those_of_the_last_timed_step(tmp_path):
+    """--dump-outputs: the same arguments give the same inputs, so two runs write identical float32 / float64 arrays
+    (under 64 MB in all); they equal the C oracle's after exactly the steps the benchmark has run at the end of its timed
+    passes, and two more timed steps per pass add exactly that many steps."""
+    import numpy as np
+
+    import sy_oracle as so
+    import sy_oracle_c as oc
+    from student_mechanism_design_b200.graphs import generate_graph_pool
+
+    B, warmup, passes = 1024, 3, 2  # c2: 50 nodes, 110 edges, 3 police, budget 10, no tolls, no belief, reveal every 5
+
+    def run(tag, steps):
+        out = tmp_path / tag
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--workload", "c2", "--steps", str(steps),
+                            "--warmup", str(warmup), "--passes", str(passes), "--no-cpu-baseline", "--e2e-steps", "3",
+                            "--dump-outputs", str(out)], capture_output=True, text=True, cwd=tmp_path)
+        assert p.returncode == 0, p.stderr[-2000:]
+        assert json.loads(p.stdout.strip().splitlines()[-1])["steps"] == steps
+        return {f.stem: np.load(f) for f in sorted(out.glob("*.npy"))}
+
+    a, b, c = run("a", 7), run("b", 7), run("c", 9)
+    assert set(a) == set(b) == set(c) >= {"actions", "reward", "terminated", "agent_position", "action_mask", "node_features",
+                                          "env_index", "episode_stats"}
+    assert sum(x.nbytes for x in a.values()) <= 64 << 20
+    for k in a:
+        assert a[k].dtype in (np.float32, np.float64), k
+        assert np.array_equal(a[k], b[k]), k
+    # 7 and 9 have no divisor among bench.py's segment lengths (50, 25, 20, 10, 5, 4, 2), so the timed passes replay a
+    # 1-step graph, which also ran once when it was captured and once to upload it: at the dump the env has taken
+    # warmup + 2 + passes * steps steps.  Other step counts change that count of untimed steps.
+    T = warmup + 2 + passes * 7
+    assert a["episode_stats"][0] == B * T and c["episode_stats"][0] == B * (T + passes * (9 - 7))  # STAT_NAMES[0] = env_steps
+    pool = [so.Graph(g.num_nodes, g.edge_links, g.edges) for g in generate_graph_pool(1, 50, 110, seed=0)]
+    ob = oc.CBatch(so.OracleConfig(num_police=3, agent_money=10, toll=0, belief=False, reveal_interval=5), pool, B, seed=0)
+    ob.steps(T - 1)
+    acts = ob.sample_actions(T - 1)
+    want = ob.step(acts)
+    idx = a["env_index"].astype(np.int64)
+    assert np.array_equal(idx, np.arange(B))  # the whole c2 batch fits the sample
+    expect = {"actions": acts, "agent_position": ob.pos(), "Currency": ob.money()[:, 1:], "MrX_revealed": ob.revealed(),
+              "reward": want["reward"].astype(np.float32), "terminated": np.repeat(want["terminated"][:, None], 4, 1),
+              "winner": want["winner"], "action_mask": ob.masks(), "node_features": ob.node_features()}
+    for k, v in expect.items():
+        np.testing.assert_array_equal(a[k], np.asarray(v, dtype=np.float32)[idx], err_msg=k)
