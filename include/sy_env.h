@@ -334,6 +334,35 @@ int sy_sample_actions(SyEnv* env, const SyState* state, uint32_t step_counter, i
  * step kernel's atomics do not serialise on one cache line). */
 int sy_stats(SyEnv* env, int64_t* stats, sy_stream_t stream);
 
+/* Mechanism groups: one handle evaluates up to SY_MAX_GROUPS mechanisms side by side.  Every env belongs to one group,
+ * and a group replaces, for its envs, the config's reward weights (fp32 reward mode uses (float)w), police start budget
+ * (agent_money) and reveal schedule (reveal_interval, reveal_skip_prob).  Everything else stays one value per handle.
+ * Group membership enters no random stream, so a group equal to the config reproduces a handle without groups bit for
+ * bit.  Every step path runs with groups (its GROUPS instantiation) except the split step of SY_OPT_NF_FILL, which acts
+ * as off while groups are set (results are the same).  The statistics are also summed per group (sy_group_stats).
+ * The library's group buffers are allocated once and updated in place, but a CUDA graph captured before a
+ * sy_set_groups call carries the groups of its capture: recapture it after changing the groups. */
+#define SY_MAX_GROUPS 1024
+typedef struct SyGroup {
+  uint64_t struct_bytes; /* = sizeof(SyGroup) */
+  double reward_weights[SY_NUM_REWARD_WEIGHTS];
+  int32_t agent_money, reveal_interval;
+  float reveal_skip_prob;
+  int32_t reserved0;
+} SyGroup;
+/* groups: HOST table [num_groups]; group_id: DEVICE int32 [B], or NULL = (env_offset + b) % num_groups (every group then
+ * sees the same graph mix, and a sharded batch is assigned as the unsharded one); num_groups = 0 clears the groups.
+ * Validates (the table on the host, the ids with one small kernel + one synchronise of `stream`) and copies both into
+ * library-owned memory; a rejected call keeps the previous groups.  The new groups take effect at the next sy_reset of
+ * every env (NULL reset_mask, or one with every byte set): until then the step and rollout entry points fail with
+ * SY_ERR_STATE (so a state saved under groups cannot be resumed mid-episode: the reset starts new episodes).  Fails with
+ * SY_ERR_STATE while observations are pending.  Clears the per-group statistics. */
+int sy_set_groups(SyEnv* env, int32_t num_groups, const SyGroup* groups, const int32_t* group_id, sy_stream_t stream);
+/* Add the per-group statistics accumulated since the last call to `stats` (DEVICE int64 [num_groups, SY_NUM_STATS],
+ * caller-owned, cumulative) and clear the accumulators; num_groups must be the number set.  They are collected by the
+ * same steps as sy_stats, with the same integer sums, so the sum over groups equals the handle-wide vector. */
+int sy_group_stats(SyEnv* env, int32_t num_groups, int64_t* stats, sy_stream_t stream);
+
 /* The path's one collective (SURVEY.md 8(e)): fold the accumulated statistics into `stats_local` (device, int64
  * [SY_NUM_STATS], this rank's cumulative vector, as sy_stats does) and write their sum over all ranks of `nccl_comm`
  * (an `ncclComm_t`, passed as void*) to `stats_global` (device, int64 [SY_NUM_STATS]) with one ncclAllReduce on `stream`

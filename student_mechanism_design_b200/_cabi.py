@@ -13,6 +13,7 @@ SY_ABI_VERSION = 4
 SY_NUM_REWARD_WEIGHTS = 11
 SY_MAX_AGENTS = 16
 SY_NUM_STATS = 16
+SY_MAX_GROUPS = 1024
 SY_REWARD_FP64, SY_REWARD_FP32 = 0, 1
 STAT_NAMES = [
     "env_steps", "episodes", "mrx_wins", "police_wins", "truncations", "out_of_money",
@@ -62,6 +63,13 @@ class SyHostOut(_PtrStruct):
         "reward", "terminated", "truncated", "done", "winner", "status")]
 
 
+class SyGroup(C.Structure):
+    _fields_ = [
+        ("struct_bytes", C.c_uint64), ("reward_weights", C.c_double * SY_NUM_REWARD_WEIGHTS),
+        ("agent_money", C.c_int32), ("reveal_interval", C.c_int32), ("reveal_skip_prob", C.c_float), ("reserved0", C.c_int32),
+    ]
+
+
 # name -> (restype, argtypes); must list every function include/sy_env.h declares
 SIGNATURES = {
     "sy_abi_version": (C.c_int, []),
@@ -100,6 +108,8 @@ SIGNATURES = {
     "sy_sample_actions": (C.c_int, [C.c_void_p, C.POINTER(SyState), C.c_uint32, C.c_void_p, C.c_void_p]),
     "sy_copy_segments": (C.c_int, [C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sy_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "sy_set_groups": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(SyGroup), C.c_void_p, C.c_void_p]),
+    "sy_group_stats": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
     "sy_allreduce_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sy_rollout_random_dev": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(SyState), C.POINTER(SyObs),
                                         C.POINTER(SyOut), C.c_void_p]),

@@ -65,6 +65,7 @@ int fail(int code, const char* fmt, ...) {
   } while (0)
 
 constexpr int STAT_REPLICAS = 64;  // statistics accumulator lines (128 B each) the tiles are spread over
+constexpr int GROUP_STAT_LINES = 4096;  // per-group statistics lines of a handle (replicas x groups)
 constexpr int TILE = 32;       // envs per observe CTA / per logic warp (lane = env)
 #ifndef SY_BEL_WARPS
 #define SY_BEL_WARPS 8
@@ -166,6 +167,21 @@ struct Params {
   const int32_t* init_pos;
   const int32_t* init_gid;
   int restart;
+  // mechanism groups (sy_set_groups; read only by the GROUPS instantiations): per-env reward weights, police budget and
+  // reveal schedule.  Appended so that the offsets of every field above stay where the default kernels expect them.
+  const struct GroupRow* grp;        // [grp_n] library-owned table
+  const int32_t* grp_id;             // [B] group of each env
+  int grp_n, grp_rep;                // groups; replicas of the per-group statistics lines
+  unsigned long long* grp_stats;     // [grp_rep, grp_n, SY_NUM_STATS] per-group statistics accumulators
+};
+
+// one mechanism group as the kernels read it (SyGroup prepared on the host: fp32 weights and the reveal-skip threshold
+// precomputed exactly as fill_params does for the handle's config)
+struct GroupRow {
+  double w64[SY_NUM_REWARD_WEIGHTS];
+  float w32[SY_NUM_REWARD_WEIGHTS];
+  int agent_money, reveal;
+  unsigned long long reveal_skip_thresh;
 };
 
 
@@ -220,11 +236,22 @@ __device__ void philox_start_positions(const Params& p, unsigned env, unsigned e
 
 // reveal schedule (src/eval/run_ablations.py:225-229) with the robustness hook of src/eval/ood_eval.py:227-229: a scheduled
 // reveal is skipped with probability reveal_skip_prob, one Philox(seed; env, timestep, RNG_REVEAL_SKIP, episode) draw
-__device__ __forceinline__ bool reveal_now(const Params& p, unsigned env, int t, int episode) {
-  if (p.reveal <= 0 || t <= 0 || (t % p.reveal) != 0) return false;
-  if (p.reveal_skip_thresh == 0) return true;
-  const uint4 r = philox4x32(make_uint4(env, (unsigned)t, RNG_REVEAL_SKIP, (unsigned)episode), make_uint2(p.seed_lo, p.seed_hi));
-  return (unsigned long long)r.x >= p.reveal_skip_thresh;
+// (GROUPS: the schedule of the env's mechanism group `gr` instead of the handle's)
+template <int GROUPS = 0>
+__device__ __forceinline__ bool reveal_now(const Params& p, unsigned env, int t, int episode, const GroupRow* gr = nullptr) {
+  if constexpr (GROUPS) {
+    const int reveal = __ldg(&gr->reveal);
+    if (reveal <= 0 || t <= 0 || (t % reveal) != 0) return false;
+    const unsigned long long thresh = __ldg(&gr->reveal_skip_thresh);
+    if (thresh == 0) return true;
+    const uint4 r = philox4x32(make_uint4(env, (unsigned)t, RNG_REVEAL_SKIP, (unsigned)episode), make_uint2(p.seed_lo, p.seed_hi));
+    return (unsigned long long)r.x >= thresh;
+  } else {
+    if (p.reveal <= 0 || t <= 0 || (t % p.reveal) != 0) return false;
+    if (p.reveal_skip_thresh == 0) return true;
+    const uint4 r = philox4x32(make_uint4(env, (unsigned)t, RNG_REVEAL_SKIP, (unsigned)episode), make_uint2(p.seed_lo, p.seed_hi));
+    return (unsigned long long)r.x >= p.reveal_skip_thresh;
+  }
 }
 
 __device__ __forceinline__ int philox_graph_choice(const Params& p, unsigned env, unsigned episode) {
@@ -416,10 +443,13 @@ struct RewardInputs {
 };
 
 // reward of agent a (reward_calculator.py:26-92 endings, :94-266 shaped), float64 value (fp32 mode: the float, widened)
-template <int MODE, int MAXA>
+// GROUPS: the weights of the env's mechanism group `gr` instead of the handle's
+template <int MODE, int MAXA, int GROUPS = 0>
 __device__ __forceinline__ double agent_reward(const Params& p, const RewardTables& rt, const RewardInputs<MAXA>& in, int t, int status,
-                                               int a, int visits_here) {
+                                               int a, int visits_here, const GroupRow* gr = nullptr) {
   const Tables& tb = p.tb;
+  auto w64 = [&](int k) { return GROUPS ? __ldg(&gr->w64[k]) : p.w64[k]; };
+  auto w32 = [&](int k) { return GROUPS ? __ldg(&gr->w32[k]) : p.w32[k]; };
   const int P = p.P;
   if (status == ST_CAPTURE) return (a == 0) ? -1.0 : 1.0;
   if (status != ST_RUNNING) return (a == 0) ? 1.0 : 0.0;
@@ -445,13 +475,13 @@ __device__ __forceinline__ double agent_reward(const Params& p, const RewardTabl
     const double x3 = (double)in.mob;
     const double x4 = __dmul_rn(0.1, tt);
     if (MODE == SY_REWARD_FP64) {
-      const double t1 = __dmul_rn(p.w64[4], x1), t2 = __dmul_rn(p.w64[5], x2), t3 = __dmul_rn(p.w64[6], x3);
-      const double t4 = __dmul_rn(__dsub_rn(1.0, p.w64[7]), x4);
+      const double t1 = __dmul_rn(w64(4), x1), t2 = __dmul_rn(w64(5), x2), t3 = __dmul_rn(w64(6), x3);
+      const double t4 = __dmul_rn(__dsub_rn(1.0, w64(7)), x4);
       return __dadd_rn(__dadd_rn(__dadd_rn(t1, t2), t3), t4);
     } else {
-      const float t1 = __fmul_rn(p.w32[4], (float)x1), t2 = __fmul_rn(p.w32[5], (float)x2);
-      const float t3 = __fmul_rn(p.w32[6], (float)x3);
-      const float t4 = __fmul_rn(__fsub_rn(1.0f, p.w32[7]), (float)x4);
+      const float t1 = __fmul_rn(w32(4), (float)x1), t2 = __fmul_rn(w32(5), (float)x2);
+      const float t3 = __fmul_rn(w32(6), (float)x3);
+      const float t4 = __fmul_rn(__fsub_rn(1.0f, w32(7)), (float)x4);
       return (double)__fadd_rn(__fadd_rn(__fadd_rn(t1, t2), t3), t4);
     }
   }
@@ -476,16 +506,16 @@ __device__ __forceinline__ double agent_reward(const Params& p, const RewardTabl
   }
   const double x4 = __dmul_rn(0.05, tt);
   if (MODE == SY_REWARD_FP64) {
-    const double u1 = __dmul_rn(p.w64[0], dx), u2 = __dmul_rn(p.w64[1], grp), u3 = __dmul_rn(p.w64[2], mob);
-    const double u4 = __dmul_rn(__dsub_rn(1.0, p.w64[3]), x4);
-    const double u5 = __dmul_rn(p.w64[9], prox), u6 = __dmul_rn(p.w64[10], ov), u7 = __dmul_rn(p.w64[8], cov);
+    const double u1 = __dmul_rn(w64(0), dx), u2 = __dmul_rn(w64(1), grp), u3 = __dmul_rn(w64(2), mob);
+    const double u4 = __dmul_rn(__dsub_rn(1.0, w64(3)), x4);
+    const double u5 = __dmul_rn(w64(9), prox), u6 = __dmul_rn(w64(10), ov), u7 = __dmul_rn(w64(8), cov);
     return __dadd_rn(__dsub_rn(__dadd_rn(__dadd_rn(__dadd_rn(__dadd_rn(u1, u2), u3), u4), u5), u6), u7);
   } else {
-    const float u1 = __fmul_rn(p.w32[0], (float)dx), u2 = __fmul_rn(p.w32[1], (float)grp);
-    const float u3 = __fmul_rn(p.w32[2], (float)mob);
-    const float u4 = __fmul_rn(__fsub_rn(1.0f, p.w32[3]), (float)x4);
-    const float u5 = __fmul_rn(p.w32[9], (float)prox), u6 = __fmul_rn(p.w32[10], (float)ov);
-    const float u7 = __fmul_rn(p.w32[8], (float)cov);
+    const float u1 = __fmul_rn(w32(0), (float)dx), u2 = __fmul_rn(w32(1), (float)grp);
+    const float u3 = __fmul_rn(w32(2), (float)mob);
+    const float u4 = __fmul_rn(__fsub_rn(1.0f, w32(3)), (float)x4);
+    const float u5 = __fmul_rn(w32(9), (float)prox), u6 = __fmul_rn(w32(10), (float)ov);
+    const float u7 = __fmul_rn(w32(8), (float)cov);
     return (double)__fadd_rn(__fsub_rn(__fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(u1, u2), u3), u4), u5), u6), u7);
   }
 }
@@ -572,7 +602,9 @@ struct LogicSmem {
 // LAG_BAR, LAGT threads: the observation warps arrive, the dynamics warps wait -- long after the arrival in practice).
 constexpr int LAG_BAR = 4;
 constexpr int LAG_CSR_BAR = 6;  // lagged kernel: the writers' staged graph is complete (writers arrive, dynamics warps wait)
-template <int MODE, int MAXA, int BAR, int LAGT = 0, int CSRT = 0>
+// GROUPS: mechanism groups are set -- every env reads its group's row (reward weights, police budget, reveal schedule)
+// once per step through the read-only path, and the statistics are also summed per group
+template <int MODE, int MAXA, int BAR, int LAGT = 0, int CSRT = 0, int GROUPS = 0>
 __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm, int b0, int tid, const SharedGraph* sgp = nullptr,
                                            const int* sg_valid = nullptr, unsigned extra_ctr = 0, bool draw_next = true) {
   constexpr int DS = LogicSmem<MAXA>::DS;
@@ -643,6 +675,12 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
   u16* pos = sm.pos + lane * HS;
   int* money = sm.money + lane * AS;
   const int* act = sm.act + lane * AS;
+  const GroupRow* gr = nullptr;  // this env's mechanism group (GROUPS only)
+  int grp = -1;
+  if constexpr (GROUPS) {
+    grp = live ? __ldg(p.grp_id + b) : -1;
+    gr = p.grp + max(grp, 0);
+  }
 
   // ---- P1, four warps in parallel:
   //   warp 0    the order-dependent moves + ending
@@ -736,7 +774,7 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
           const int c = min(mny - p.toll, p.tb.wcap);
           if (c > 0) in.mob = sm.cnt_staged ? (int)sm.cnt[u * (p.tb.wcap + 1) + c] : move_count(p.tb, N, g, u, mny, p.toll);
         }
-        r64 = agent_reward<MODE, MAXA>(p, sm.rt, in, t, status, a, visits_here);
+        r64 = agent_reward<MODE, MAXA, GROUPS>(p, sm.rt, in, t, status, a, visits_here, gr);
       }
       p.out.reward[(size_t)b * A + a] = (float)r64;
       if (p.out.reward64) p.out.reward64[(size_t)b * A + a] = r64;
@@ -770,7 +808,8 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
         p.out.winner[b] = (int8_t)(status == ST_CAPTURE ? SY_WINNER_POLICE : (status == ST_RUNNING ? SY_WINNER_NONE : SY_WINNER_MRX));
         bel = BEL_PROPAGATE;
         if (status != ST_RUNNING) {
-          ep_spent = P * p.agent_money;  // every police starts an episode with agent_money (yard.py:117-119)
+          const int agent_money = GROUPS ? __ldg(&gr->agent_money) : p.agent_money;
+          ep_spent = P * agent_money;  // every police starts an episode with agent_money (yard.py:117-119)
           for (int i = 1; i <= P; ++i) ep_spent -= money[i];
           if (p.auto_reset) {  // same-step auto-reset: the observation describes the fresh episode
             episode += 1;
@@ -778,7 +817,7 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
             money[0] = p.mrx_money;
             pos[0] = sm.reset_pos[lane * HS];
             for (int i = 1; i <= P; ++i) {
-              money[i] = p.agent_money;
+              money[i] = agent_money;
               pos[i] = sm.reset_pos[lane * HS + i];
             }
             t_new = 0;
@@ -792,9 +831,10 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
         p.out.winner[b] = SY_WINNER_NONE;
       }
       // reveal schedule (src/eval/run_ablations.py:225-229) on the new timestep
-      const bool rev = reveal_now(p, (unsigned)(p.env_offset + (unsigned long long)b), t_new, episode);
+      const bool rev = reveal_now<GROUPS>(p, (unsigned)(p.env_offset + (unsigned long long)b), t_new, episode, gr);
       if (rev && bel == BEL_PROPAGATE) bel = BEL_DELTA;
-      revealed = (p.reveal <= 0 || rev) ? (int)pos[0] : -1;
+      if constexpr (GROUPS) revealed = (__ldg(&gr->reveal) <= 0 || rev) ? (int)pos[0] : -1;
+      else revealed = (p.reveal <= 0 || rev) ? (int)pos[0] : -1;
     }
     sm.t_new[lane] = t_new;
     sm.gid[lane] = gnew;
@@ -822,6 +862,19 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
     int n_trunc = fin && st == ST_TIMEOUT, n_broke = fin && st == ST_NO_MONEY;
     int len_sum = len, len_sq = len * len, len_pol = n_pol ? len : 0, len_mrx = n_mrx ? len : 0;
     int ep_spent = sm.ep_spent[lane], spent = sm.spent[lane], moves = sm.moves[lane];
+    if constexpr (GROUPS) {
+      // per-group sums: the lanes of each distinct group reduce together, one leader adds them to the group's line
+      const int v[SY_STAT_POLICE_MOVES + 1] = {n_step, n_ep, n_mrx, n_pol, n_trunc, n_broke, len_sum, spent,
+                                               len_sq, len_pol, len_mrx, ep_spent, moves};
+      const unsigned same = __match_any_sync(FULL, grp);
+      const bool leader = grp >= 0 && lane == __ffs(same) - 1;
+      unsigned long long* line = p.grp_stats + ((size_t)(blockIdx.x % p.grp_rep) * p.grp_n + max(grp, 0)) * SY_NUM_STATS;
+#pragma unroll
+      for (int k = 0; k <= SY_STAT_POLICE_MOVES; ++k) {
+        const int sum = __reduce_add_sync(same, v[k]);
+        if (leader && sum) atomicAdd(line + k, (unsigned long long)sum);
+      }
+    }
     // per-tile sums -> one of STAT_REPLICAS library-owned accumulator lines (sy_stats folds them into the caller's
     // vector): with a single shared line the 13 atomics of all 2048 tiles serialised in one L2 slice (8 us per step)
     n_step = __reduce_add_sync(FULL, n_step);
@@ -932,11 +985,11 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
   PHASE_MARK(7);
 }
 
-template <int MODE, int MAXA>
+template <int MODE, int MAXA, int GROUPS = 0>
 __global__ void __launch_bounds__(LOGIC_THREADS, SY_LOGIC_MIN_CTAS) sy_logic_kernel(const Params p) {
   __shared__ LogicSmem<MAXA> sm;
   pdl_launch_dependents();  // the observation kernel's CTAs may take the slots the last wave of this grid leaves free
-  logic_tile<MODE, MAXA, 3>(p, sm, blockIdx.x * 32, threadIdx.x);
+  logic_tile<MODE, MAXA, 3, 0, 0, GROUPS>(p, sm, blockIdx.x * 32, threadIdx.x);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -972,6 +1025,8 @@ __global__ void __launch_bounds__(FILL_THREADS) sy_fill_kernel(uint8_t* dst, siz
 // ---------------------------------------------------------------------------------------------
 // reset kernel (yard.py:80-142): re-initialise the masked envs (same warp = 32 envs layout)
 // ---------------------------------------------------------------------------------------------
+// GROUPS: police budgets and reveal schedule of each env's mechanism group
+template <int GROUPS = 0>
 __global__ void __launch_bounds__(LOGIC_THREADS) sy_reset_kernel(const Params p) {
   __shared__ WarpTile wts[LOGIC_THREADS / 32];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -988,7 +1043,8 @@ __global__ void __launch_bounds__(LOGIC_THREADS) sy_reset_kernel(const Params p)
     const int e = (i * p.inv_A) >> 16, a = i - e * A;  // i / A without a division (i < 512, A <= 16)
     const size_t o = (size_t)b0 * A + i;
     if ((rst_mask >> e) & 1u) {
-      wt.money[e * AS + a] = (a == 0) ? p.mrx_money : p.agent_money;  // yard.py:117-119
+      const int agent_money = GROUPS ? __ldg(&p.grp[__ldg(p.grp_id + b0 + e)].agent_money) : p.agent_money;
+      wt.money[e * AS + a] = (a == 0) ? p.mrx_money : agent_money;  // yard.py:117-119
       wt.pos[e * AS + a] = p.init_pos ? p.init_pos[o] : 0;
     } else {
       wt.money[e * AS + a] = p.st.money[o];
@@ -1013,8 +1069,10 @@ __global__ void __launch_bounds__(LOGIC_THREADS) sy_reset_kernel(const Params p)
       done = p.st.done[b];
       g = p.st.graph_id[b];
     }
-    const bool rev = reveal_now(p, (unsigned)(p.env_offset + (unsigned long long)b), t, episode);
-    revealed = (p.reveal <= 0 || rev) ? wt.pos[lane * AS] : -1;
+    const GroupRow* gr = GROUPS ? p.grp + __ldg(p.grp_id + b) : nullptr;
+    const bool rev = reveal_now<GROUPS>(p, (unsigned)(p.env_offset + (unsigned long long)b), t, episode, gr);
+    if constexpr (GROUPS) revealed = (__ldg(&gr->reveal) <= 0 || rev) ? wt.pos[lane * AS] : -1;
+    else revealed = (p.reveal <= 0 || rev) ? wt.pos[lane * AS] : -1;
   }
   store_state(p, wt, b0, nEnv, lane, t, g, episode, done, rst ? BEL_UNIFORM : BEL_KEEP, revealed, rst);
 }
@@ -1567,17 +1625,32 @@ constexpr float CE_Q = 16777216.0f;  // 2^24
 
 __device__ __forceinline__ float ce_clip(float v) { return fminf(fmaxf(v, CE_CLIP), 1.0f); }
 
-// lanes hold partial clipped sums `S` and (one lane) the clipped value at the true node `vx`
-__device__ __forceinline__ void ce_record(CeAcc& acc, float S, float vx) {
+// lanes hold partial clipped sums `S` and (one lane) the clipped value at the true node `vx`.  GROUPS: the score of env
+// b also goes straight into its mechanism group's line (reveals are a fraction of the steps: one atomic triple each)
+template <int GROUPS = 0>
+__device__ __forceinline__ void ce_record(CeAcc& acc, float S, float vx, const Params* p = nullptr, int b = 0, int lane = 0) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
     S += __shfl_xor_sync(FULL, S, o);
     vx = fmaxf(vx, __shfl_xor_sync(FULL, vx, o));
   }
   const float ce = logf(S) - logf(vx);  // -log(vx / S); both logs are of normal floats (vx >= 1e-8)
-  acc.n += 1;
-  acc.sum_q += __float2ll_rn(ce * CE_Q);
-  acc.sq_q += __float2ll_rn(ce * ce * CE_Q);
+  if constexpr (!GROUPS) {
+    acc.n += 1;
+    acc.sum_q += __float2ll_rn(ce * CE_Q);
+    acc.sq_q += __float2ll_rn(ce * ce * CE_Q);
+  } else {
+    const long long q = __float2ll_rn(ce * CE_Q), sq = __float2ll_rn(ce * ce * CE_Q);
+    acc.n += 1;
+    acc.sum_q += q;
+    acc.sq_q += sq;
+    if (lane == 0) {
+      unsigned long long* line = p->grp_stats + ((size_t)(blockIdx.x % p->grp_rep) * p->grp_n + __ldg(p->grp_id + b)) * SY_NUM_STATS;
+      atomicAdd(line + SY_STAT_REVEALS, 1ull);
+      atomicAdd(line + SY_STAT_SUM_BELIEF_CE_Q24, (unsigned long long)q);
+      atomicAdd(line + SY_STAT_SUM_SQ_BELIEF_CE_Q24, (unsigned long long)sq);
+    }
+  }
 }
 
 __device__ __forceinline__ void ce_flush(const Params& p, const CeAcc& acc, int lane) {
@@ -1598,7 +1671,9 @@ struct SharedCsr {  // the writer warps' staged copy of the tile's graph (null r
   const uint16_t* perm;  // nodes by degree: the 32 lanes of a gather step walk lists of (nearly) equal length
 };
 
-__device__ void belief_env_generic(const Params& p, float* sb, int b, int op, int g, int x, int lane, CeAcc& ce, const SharedCsr sc) {
+template <int GROUPS>
+__device__ __forceinline__ void belief_env_generic_t(const Params& p, float* sb, int b, int op, int g, int x, int lane, CeAcc& ce,
+                                                     const SharedCsr sc) {
   const int N = p.N;
   const Tables& tb = p.tb;
   float* bel = p.st.belief + (size_t)b * N;
@@ -1713,7 +1788,8 @@ __device__ void belief_env_generic(const Params& p, float* sb, int b, int op, in
       }
     }
     if (score) {
-      ce_record(ce, S, vx);
+      if constexpr (GROUPS) ce_record<1>(ce, S, vx, &p, b, lane);
+      else ce_record(ce, S, vx);
       _Pragma("unroll 1") for (int j = lane; j < N; j += 32) bel[j] = (j == x) ? 1.0f : 0.0f;
     } else if (p.belief_hint && op == BEL_PROPAGATE && tot != 0.0f) {
       // observation hint (belief_module.py:102-106) on the row this warp just wrote (every lane re-reads its own stores)
@@ -1728,7 +1804,16 @@ __device__ void belief_env_generic(const Params& p, float* sb, int b, int op, in
   }
 }
 
-template <int BW, int LAGT = 0>
+// one env's belief row, warp-wide (an out-of-line function, as the kernels were tuned with; GROUPS: its own copy)
+__device__ void belief_env_generic(const Params& p, float* sb, int b, int op, int g, int x, int lane, CeAcc& ce, const SharedCsr sc) {
+  belief_env_generic_t<0>(p, sb, b, op, g, x, lane, ce, sc);
+}
+__device__ void belief_env_generic_groups(const Params& p, float* sb, int b, int op, int g, int x, int lane, CeAcc& ce,
+                                          const SharedCsr sc) {
+  belief_env_generic_t<1>(p, sb, b, op, g, x, lane, ce, sc);
+}
+
+template <int BW, int LAGT = 0, int GROUPS = 0>
 __device__ __forceinline__ void belief_role(const Params& p, unsigned char* dyn, int tile0, int nEnv, int w, int lane) {
   const int N = p.N;
   // every belief warp reads the same 32 flags / graph ids, so the branches below are uniform across the role
@@ -1767,8 +1852,12 @@ __device__ __forceinline__ void belief_role(const Params& p, unsigned char* dyn,
       sc.pptr = reinterpret_cast<const uint16_t*>(dyn + p.wr_off_csr + p.wr_off_pad);
       sc.pcol = sc.pptr + ((N + 1 + 3) & ~3);
     }
-    for (int e = w; e < nEnv; e += BW)
-      belief_env_generic(p, sb, tile0 + e, __shfl_sync(FULL, op, e), __shfl_sync(FULL, g, e), __shfl_sync(FULL, xm, e), lane, ce, sc);
+    for (int e = w; e < nEnv; e += BW) {
+      if constexpr (GROUPS)
+        belief_env_generic_groups(p, sb, tile0 + e, __shfl_sync(FULL, op, e), __shfl_sync(FULL, g, e), __shfl_sync(FULL, xm, e), lane, ce, sc);
+      else
+        belief_env_generic(p, sb, tile0 + e, __shfl_sync(FULL, op, e), __shfl_sync(FULL, g, e), __shfl_sync(FULL, xm, e), lane, ce, sc);
+    }
     ce_flush(p, ce, lane);
     return;
   }
@@ -1892,7 +1981,8 @@ __device__ __forceinline__ void belief_role(const Params& p, unsigned char* dyn,
             if (j == x) vx = c;
           }
         }
-        ce_record(ce, S, vx);
+        if constexpr (GROUPS) ce_record<1>(ce, S, vx, &p, tile0 + e, lane);
+        else ce_record(ce, S, vx);
       }
       _Pragma("unroll 1") for (int j = lane; j < N; j += 32) bel[j] = (j == x) ? 1.0f : 0.0f;
     }
@@ -1908,7 +1998,9 @@ __device__ __forceinline__ void belief_role(const Params& p, unsigned char* dyn,
 // <BW, 0> / <0, WRW>: one role per launch (the split step runs them as two concurrent kernels; the role hand-over
 // barrier of the large-N belief path counts THREADS, so that path keeps both roles in one launch)
 enum { WV_LSU = 0, WV_BULK = 1, WV_ONES = 2 };
-template <int BW, int WRW, int WV = WV_LSU>
+// GROUPS: the belief scores at reveal steps are also summed per mechanism group (only launched while groups are set and
+// the step collects scored statistics)
+template <int BW, int WRW, int WV = WV_LSU, int GROUPS = 0>
 __global__ void __launch_bounds__((BW + WRW) * 32) sy_observe_kernel(const Params p) {
   static_assert((BW + WRW) * 32 == THREADS || BW == 0 || WRW == 0, "the role hand-over barrier counts THREADS");
   extern __shared__ __align__(16) unsigned char dyn[];
@@ -1931,7 +2023,7 @@ __global__ void __launch_bounds__((BW + WRW) * 32) sy_observe_kernel(const Param
   const long long t0 = FCLK_NOW();
   if (warp < nbw) {
     if constexpr (BW > 0) {
-      if (!(p.dbg_skip & 4)) belief_role<BW>(p, dyn, tile0, nEnv, warp, lane);
+      if (!(p.dbg_skip & 4)) belief_role<BW, 0, GROUPS>(p, dyn, tile0, nEnv, warp, lane);
       if (warp == 0) FCLK_ADD(3, FCLK_NOW() - t0);
     }
   } else if (!(p.dbg_skip & 1)) {
@@ -1963,7 +2055,7 @@ constexpr int GEN_BEL_WARPS = THREADS / 32 >= 16 ? 12 : BEL_WARPS, GEN_WR_WARPS 
 // agents) sees the new state after every launch; action_mask / node_features / belief_map trail it by one step until
 // sy_flush_observations (or any non-deferred call) brings them up to date.
 // ---------------------------------------------------------------------------------------------
-template <int MODE, int MAXA, int BW, int WRW>
+template <int MODE, int MAXA, int BW, int WRW, int GROUPS = 0>
 __global__ void __launch_bounds__((BW + WRW + LOGIC_WARPS) * 32, 2) sy_step_lagged_kernel(const Params p) {
   constexpr int NT = (BW + WRW + LOGIC_WARPS) * 32;
   extern __shared__ __align__(16) unsigned char dyn[];
@@ -1975,7 +2067,7 @@ __global__ void __launch_bounds__((BW + WRW + LOGIC_WARPS) * 32, 2) sy_step_lagg
   __shared__ int staged_flag;
   const long long t0 = FCLK_NOW();
   if (warp < BW) {
-    if constexpr (BW > 0) belief_role<BW, NT>(p, dyn, tile0, nEnv, warp, lane);
+    if constexpr (BW > 0) belief_role<BW, NT, GROUPS>(p, dyn, tile0, nEnv, warp, lane);
     if (warp == 0) FCLK_ADD(3, FCLK_NOW() - t0);
   } else if (warp < BW + WRW) {
     writer_role<WRW, false, NT, CSRT>(p, dyn, tile0, nEnv, warp - BW, lane, &staged_flag);
@@ -1984,7 +2076,7 @@ __global__ void __launch_bounds__((BW + WRW + LOGIC_WARPS) * 32, 2) sy_step_lagg
     const int* s_rp = reinterpret_cast<const int*>(dyn + p.wr_off_csr);
     const uint16_t* s_col = reinterpret_cast<const uint16_t*>(s_rp + p.N + 1);
     const SharedGraph sg{s_rp, s_col, reinterpret_cast<const uint8_t*>(s_col + p.tb.nnz_stride)};
-    logic_tile<MODE, MAXA, 5, NT, CSRT>(p, lsm, tile0, threadIdx.x - (BW + WRW) * 32, &sg, &staged_flag);
+    logic_tile<MODE, MAXA, 5, NT, CSRT, GROUPS>(p, lsm, tile0, threadIdx.x - (BW + WRW) * 32, &sg, &staged_flag);
     if (warp == BW + WRW) {
       FCLK_ADD(4, FCLK_NOW() - t0);
       FCLK_ADD(5, 1);
@@ -1999,7 +2091,7 @@ __global__ void __launch_bounds__((BW + WRW + LOGIC_WARPS) * 32, 2) sy_step_lagg
 // the iteration (the new state is visible to the CTA's own roles, shared memory may be reused).  K + 1 iterations: the
 // first without observations (they are current on entry), the last without dynamics.
 constexpr int ROLL_BAR = 7;
-template <int MODE, int MAXA, int BW, int WRW>
+template <int MODE, int MAXA, int BW, int WRW, int GROUPS = 0>
 __global__ void __launch_bounds__((BW + WRW + LOGIC_WARPS) * 32, 2) sy_rollout_lagged_kernel(const Params p, const int K) {
   constexpr int NT = (BW + WRW + LOGIC_WARPS) * 32;
   constexpr int CSRT = (WRW + LOGIC_WARPS) * 32;
@@ -2013,7 +2105,7 @@ __global__ void __launch_bounds__((BW + WRW + LOGIC_WARPS) * 32, 2) sy_rollout_l
     const bool do_obs = it > 0, do_logic = it < K;
     if (warp < BW) {
       if constexpr (BW > 0) {
-        if (do_obs) belief_role<BW, NT>(p, dyn, tile0, nEnv, warp, lane);
+        if (do_obs) belief_role<BW, NT, GROUPS>(p, dyn, tile0, nEnv, warp, lane);
         else asm volatile("bar.arrive %0, %1;\n" ::"n"(LAG_BAR), "n"(NT) : "memory");
       }
     } else if (warp < BW + WRW) {
@@ -2030,7 +2122,7 @@ __global__ void __launch_bounds__((BW + WRW + LOGIC_WARPS) * 32, 2) sy_rollout_l
         const uint16_t* s_col = reinterpret_cast<const uint16_t*>(s_rp + p.N + 1);
         const SharedGraph sg{s_rp, s_col, reinterpret_cast<const uint8_t*>(s_col + p.tb.nnz_stride)};
         // (the last step draws nothing: `actions` keeps the actions of the last step, as sy_rollout_random documents)
-        logic_tile<MODE, MAXA, 5, NT, CSRT>(p, lsm, tile0, threadIdx.x - (BW + WRW) * 32, &sg, &staged_flag, (unsigned)it, it + 1 < K);
+        logic_tile<MODE, MAXA, 5, NT, CSRT, GROUPS>(p, lsm, tile0, threadIdx.x - (BW + WRW) * 32, &sg, &staged_flag, (unsigned)it, it + 1 < K);
       } else {  // complete the two hand-shakes of the observation roles
         asm volatile("bar.sync %0, %1;\n" ::"n"(LAG_CSR_BAR), "n"(CSRT) : "memory");
         asm volatile("bar.sync %0, %1;\n" ::"n"(LAG_BAR), "n"(NT) : "memory");
@@ -2341,7 +2433,7 @@ __device__ __forceinline__ void fused_writer_role(const Params& p, unsigned char
   for (int q = 0; q < pending; ++q) owed_ones(ring_k[q], ring_item[q], ring_fast[q]);
 }
 
-template <int MODE, int MAXA, int BW>
+template <int MODE, int MAXA, int BW, int GROUPS = 0>
 __global__ void __launch_bounds__((BW + FUSED_WR + LOGIC_WARPS) * 32, 2) sy_step_fused_kernel(const Params p) {
   extern __shared__ __align__(16) unsigned char dyn[];
   __shared__ LogicSmem<MAXA> lsm;
@@ -2357,7 +2449,7 @@ __global__ void __launch_bounds__((BW + FUSED_WR + LOGIC_WARPS) * 32, 2) sy_step
       for (int k = 0, t = blockIdx.x; t < ntiles; t += gridDim.x, ++k) {
         if (k) named_barrier(1, BW * 32);  // every belief warp has left the previous tile's scratch
         wait_tiles_done(&tiles_done, (unsigned)k, lane, warp == 0 ? 2 : -1);
-        belief_role<BW>(p, dyn, t * TILE, min(TILE, p.B - t * TILE), warp, lane);
+        belief_role<BW, 0, GROUPS>(p, dyn, t * TILE, min(TILE, p.B - t * TILE), warp, lane);
       }
       if (warp == 0) FCLK_ADD(3, FCLK_NOW() - t0);
     }
@@ -2370,7 +2462,7 @@ __global__ void __launch_bounds__((BW + FUSED_WR + LOGIC_WARPS) * 32, 2) sy_step
     unsigned k = 0;
     const long long t0 = FCLK_NOW();
     for (int t = blockIdx.x; t < ntiles; t += gridDim.x) {
-      logic_tile<MODE, MAXA, 3>(p, lsm, t * TILE, tid);
+      logic_tile<MODE, MAXA, 3, 0, 0, GROUPS>(p, lsm, t * TILE, tid);
       __threadfence_block();
       named_barrier(3, LOGIC_THREADS);  // every logic thread's stores of the tile are ordered; lsm may be reused
       ++k;
@@ -2393,6 +2485,37 @@ __global__ void sy_fold_stats_kernel(unsigned long long* rep, long long* out) {
     rep[r * SY_NUM_STATS + k] = 0;
   }
   out[k] += (long long)sum;
+}
+
+// per-group statistics: fold the replicas of each group's line into the caller's [n, SY_NUM_STATS] table and clear them
+__global__ void sy_fold_group_stats_kernel(unsigned long long* rep, int n, int reps, long long* out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;  // = group * SY_NUM_STATS + statistic
+  if (i >= n * SY_NUM_STATS) return;
+  unsigned long long sum = 0;
+  for (int r = 0; r < reps; ++r) {
+    sum += rep[(size_t)r * n * SY_NUM_STATS + i];
+    rep[(size_t)r * n * SY_NUM_STATS + i] = 0;
+  }
+  out[i] += (long long)sum;
+}
+
+// sy_set_groups: group ids in range ([B] -> count of ids outside [0, n)), or the default assignment (env_offset + b) % n
+__global__ void sy_group_ids_kernel(const int32_t* in, int32_t* out, int B, int n, unsigned long long env_offset, int* bad) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  if (in) {
+    const int g = in[b];
+    if (g < 0 || g >= n) atomicAdd(bad, 1);
+    out[b] = g;
+  } else {
+    out[b] = (int32_t)((env_offset + (unsigned long long)b) % (unsigned long long)n);
+  }
+}
+
+// sy_reset after sy_set_groups: envs the mask leaves out
+__global__ void sy_count_unset_kernel(const uint8_t* mask, int B, int* unset) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b < B && mask[b] == 0) atomicAdd(unset, 1);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -2849,6 +2972,16 @@ struct SyEnv {
   int lag_slots = 0;  // resident CTAs of the lagged kernel (occupancy x SMs)
   int opt_pdl = 0;  // sy_set_option(SY_OPT_PDL): dynamics / observation kernels launched with programmatic stream serialisation
   int opt_rollout_kernel = 1;  // sy_set_option(SY_OPT_ROLLOUT_KERNEL): random rollouts of single-wave batches as ONE launch
+  // mechanism groups (sy_set_groups).  While they are set, steps run the GROUPS instantiations of the dynamics kernel (and
+  // of the observation kernel when belief scores are collected) as two launches: the fused / lagged / one-launch rollout
+  // kernels and the split step are not instantiated for groups
+  int grp_n = 0, grp_rep = 0;
+  void* d_grp = nullptr;         // GroupRow [SY_MAX_GROUPS], rows [0, grp_n) in use
+  void* d_grp_id = nullptr;      // int32 [B]
+  void* d_grp_id_new = nullptr;  // int32 [B] staging of sy_set_groups (validated before it replaces d_grp_id)
+  void* d_grp_bad = nullptr;     // int: ids out of range
+  void* d_grp_stats = nullptr;   // u64 [GROUP_STAT_LINES, SY_NUM_STATS]: [grp_rep, grp_n] lines in use
+  bool grp_need_reset = false;  // groups changed: steps are refused until a full sy_reset
 };
 
 namespace {
@@ -2911,14 +3044,18 @@ int plan_bulk_chunk(size_t S, int cap, int wr_warps) {
 }
 
 using FusedFn = void (*)(const Params);
-template <int BW>
+template <int BW, int GR>
 FusedFn fused_fn_bw(int reward_mode, int A) {
   const bool f64 = reward_mode == SY_REWARD_FP64;
-  if (A <= 4) return f64 ? sy_step_fused_kernel<SY_REWARD_FP64, 4, BW> : sy_step_fused_kernel<SY_REWARD_FP32, 4, BW>;
-  if (A <= 8) return f64 ? sy_step_fused_kernel<SY_REWARD_FP64, 8, BW> : sy_step_fused_kernel<SY_REWARD_FP32, 8, BW>;
-  return f64 ? sy_step_fused_kernel<SY_REWARD_FP64, 16, BW> : sy_step_fused_kernel<SY_REWARD_FP32, 16, BW>;
+  if (A <= 4) return f64 ? sy_step_fused_kernel<SY_REWARD_FP64, 4, BW, GR> : sy_step_fused_kernel<SY_REWARD_FP32, 4, BW, GR>;
+  if (A <= 8) return f64 ? sy_step_fused_kernel<SY_REWARD_FP64, 8, BW, GR> : sy_step_fused_kernel<SY_REWARD_FP32, 8, BW, GR>;
+  return f64 ? sy_step_fused_kernel<SY_REWARD_FP64, 16, BW, GR> : sy_step_fused_kernel<SY_REWARD_FP32, 16, BW, GR>;
 }
-FusedFn fused_fn(int bw, int reward_mode, int A) { return bw ? fused_fn_bw<BEL_WARPS>(reward_mode, A) : fused_fn_bw<0>(reward_mode, A); }
+// groups: the GROUPS instantiation (mechanism groups are set)
+FusedFn fused_fn(int bw, int reward_mode, int A, bool groups = false) {
+  if (groups) return bw ? fused_fn_bw<BEL_WARPS, 1>(reward_mode, A) : fused_fn_bw<0, 1>(reward_mode, A);
+  return bw ? fused_fn_bw<BEL_WARPS, 0>(reward_mode, A) : fused_fn_bw<0, 0>(reward_mode, A);
+}
 
 // shared-memory plan, grid and eligibility of the fused step kernel for this handle's shape (called with the tables)
 int plan_fused(SyEnv* e, int nnz_stride) {
@@ -2945,7 +3082,8 @@ int plan_fused(SyEnv* e, int nnz_stride) {
   e->f_smem = (size_t)e->f_off_nbr4 + (e->f_epc ? (size_t)N * 16 : 0);
   if (e->f_smem > 200 * 1024) return SY_OK;
   FusedFn fn = fused_fn(e->f_bw, e->cfg.reward_mode, A);
-  if (cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess) {
+  if (cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess ||
+      cudaFuncSetAttribute(fused_fn(e->f_bw, e->cfg.reward_mode, A, true), cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess) {
     cudaGetLastError();
     return SY_OK;
   }
@@ -2962,26 +3100,29 @@ int plan_fused(SyEnv* e, int nnz_stride) {
   return SY_OK;
 }
 
-template <int BW>
+template <int BW, int GR>
 FusedFn lagged_fn_bw(int reward_mode, int A) {
   const bool f64 = reward_mode == SY_REWARD_FP64;
-  if (A <= 4) return f64 ? sy_step_lagged_kernel<SY_REWARD_FP64, 4, BW, WR_WARPS> : sy_step_lagged_kernel<SY_REWARD_FP32, 4, BW, WR_WARPS>;
-  if (A <= 8) return f64 ? sy_step_lagged_kernel<SY_REWARD_FP64, 8, BW, WR_WARPS> : sy_step_lagged_kernel<SY_REWARD_FP32, 8, BW, WR_WARPS>;
-  return f64 ? sy_step_lagged_kernel<SY_REWARD_FP64, 16, BW, WR_WARPS> : sy_step_lagged_kernel<SY_REWARD_FP32, 16, BW, WR_WARPS>;
+  if (A <= 4) return f64 ? sy_step_lagged_kernel<SY_REWARD_FP64, 4, BW, WR_WARPS, GR> : sy_step_lagged_kernel<SY_REWARD_FP32, 4, BW, WR_WARPS, GR>;
+  if (A <= 8) return f64 ? sy_step_lagged_kernel<SY_REWARD_FP64, 8, BW, WR_WARPS, GR> : sy_step_lagged_kernel<SY_REWARD_FP32, 8, BW, WR_WARPS, GR>;
+  return f64 ? sy_step_lagged_kernel<SY_REWARD_FP64, 16, BW, WR_WARPS, GR> : sy_step_lagged_kernel<SY_REWARD_FP32, 16, BW, WR_WARPS, GR>;
 }
 using RolloutFn = void (*)(const Params, const int);
-template <int BW>
+template <int BW, int GR>
 RolloutFn rollout_fn_bw(int reward_mode, int A) {
   const bool f64 = reward_mode == SY_REWARD_FP64;
-  if (A <= 4) return f64 ? sy_rollout_lagged_kernel<SY_REWARD_FP64, 4, BW, WR_WARPS> : sy_rollout_lagged_kernel<SY_REWARD_FP32, 4, BW, WR_WARPS>;
-  if (A <= 8) return f64 ? sy_rollout_lagged_kernel<SY_REWARD_FP64, 8, BW, WR_WARPS> : sy_rollout_lagged_kernel<SY_REWARD_FP32, 8, BW, WR_WARPS>;
-  return f64 ? sy_rollout_lagged_kernel<SY_REWARD_FP64, 16, BW, WR_WARPS> : sy_rollout_lagged_kernel<SY_REWARD_FP32, 16, BW, WR_WARPS>;
+  if (A <= 4) return f64 ? sy_rollout_lagged_kernel<SY_REWARD_FP64, 4, BW, WR_WARPS, GR> : sy_rollout_lagged_kernel<SY_REWARD_FP32, 4, BW, WR_WARPS, GR>;
+  if (A <= 8) return f64 ? sy_rollout_lagged_kernel<SY_REWARD_FP64, 8, BW, WR_WARPS, GR> : sy_rollout_lagged_kernel<SY_REWARD_FP32, 8, BW, WR_WARPS, GR>;
+  return f64 ? sy_rollout_lagged_kernel<SY_REWARD_FP64, 16, BW, WR_WARPS, GR> : sy_rollout_lagged_kernel<SY_REWARD_FP32, 16, BW, WR_WARPS, GR>;
 }
-RolloutFn rollout_fn(const SyEnv* e) {
-  return e->cfg.belief ? rollout_fn_bw<BEL_WARPS>(e->cfg.reward_mode, e->A) : rollout_fn_bw<0>(e->cfg.reward_mode, e->A);
+// groups: the GROUPS instantiation (mechanism groups are set)
+RolloutFn rollout_fn(const SyEnv* e, bool groups = false) {
+  if (groups) return e->cfg.belief ? rollout_fn_bw<BEL_WARPS, 1>(e->cfg.reward_mode, e->A) : rollout_fn_bw<0, 1>(e->cfg.reward_mode, e->A);
+  return e->cfg.belief ? rollout_fn_bw<BEL_WARPS, 0>(e->cfg.reward_mode, e->A) : rollout_fn_bw<0, 0>(e->cfg.reward_mode, e->A);
 }
-FusedFn lagged_fn(const SyEnv* e) {
-  return e->cfg.belief ? lagged_fn_bw<BEL_WARPS>(e->cfg.reward_mode, e->A) : lagged_fn_bw<0>(e->cfg.reward_mode, e->A);
+FusedFn lagged_fn(const SyEnv* e, bool groups = false) {
+  if (groups) return e->cfg.belief ? lagged_fn_bw<BEL_WARPS, 1>(e->cfg.reward_mode, e->A) : lagged_fn_bw<0, 1>(e->cfg.reward_mode, e->A);
+  return e->cfg.belief ? lagged_fn_bw<BEL_WARPS, 0>(e->cfg.reward_mode, e->A) : lagged_fn_bw<0, 0>(e->cfg.reward_mode, e->A);
 }
 int lagged_threads(const SyEnv* e) { return ((e->cfg.belief ? BEL_WARPS : 0) + WR_WARPS + LOGIC_WARPS) * 32; }
 
@@ -2999,7 +3140,9 @@ int plan_lagged(SyEnv* e) {
     size_t& cur = limit[e->cfg.device & 63][slot];
     if (e->obs_smem > cur) {
       if (cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e->obs_smem) != cudaSuccess ||
-          cudaFuncSetAttribute(rollout_fn(e), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e->obs_smem) != cudaSuccess) {
+          cudaFuncSetAttribute(rollout_fn(e), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e->obs_smem) != cudaSuccess ||
+          cudaFuncSetAttribute(lagged_fn(e, true), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e->obs_smem) != cudaSuccess ||
+          cudaFuncSetAttribute(rollout_fn(e, true), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e->obs_smem) != cudaSuccess) {
         cudaGetLastError();
         return SY_OK;
       }
@@ -3035,6 +3178,10 @@ int raise_observe_smem_limit(int device, size_t bytes) {
   CUDA_TRY(cudaFuncSetAttribute(sy_observe_kernel<GEN_BEL_WARPS, GEN_WR_WARPS, WV_BULK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
   CUDA_TRY(cudaFuncSetAttribute(sy_observe_kernel<BEL_WARPS, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
   CUDA_TRY(cudaFuncSetAttribute(sy_observe_kernel<0, WR_WARPS, WV_ONES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+  CUDA_TRY(cudaFuncSetAttribute(sy_observe_kernel<BEL_WARPS, WR_WARPS, WV_LSU, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+  CUDA_TRY(cudaFuncSetAttribute(sy_observe_kernel<GEN_BEL_WARPS, GEN_WR_WARPS, WV_LSU, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+  CUDA_TRY(cudaFuncSetAttribute(sy_observe_kernel<BEL_WARPS, WR_WARPS, WV_BULK, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+  CUDA_TRY(cudaFuncSetAttribute(sy_observe_kernel<GEN_BEL_WARPS, GEN_WR_WARPS, WV_BULK, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
   cur = bytes;
   return SY_OK;
 }
@@ -3075,7 +3222,15 @@ void launch_observe(const SyEnv* e, const Params& p0, unsigned grid, cudaStream_
       grid = (unsigned)(full + rest * k);
     }
   }
-  if (p.wr_bulk) {
+  if (p.grp_n && p.belief_score && p.out.stats) {  // mechanism groups: belief scores also summed per group
+    if (p.wr_bulk) {
+      if (gen) sy_observe_kernel<GEN_BEL_WARPS, GEN_WR_WARPS, WV_BULK, 1><<<grid, THREADS, e->obs_smem, s>>>(p);
+      else sy_observe_kernel<BEL_WARPS, WR_WARPS, WV_BULK, 1><<<grid, THREADS, e->obs_smem, s>>>(p);
+    } else {
+      if (gen) launch_ex(sy_observe_kernel<GEN_BEL_WARPS, GEN_WR_WARPS, WV_LSU, 1>, grid, THREADS, e->obs_smem, s, e->opt_pdl != 0, p);
+      else launch_ex(sy_observe_kernel<BEL_WARPS, WR_WARPS, WV_LSU, 1>, grid, THREADS, e->obs_smem, s, e->opt_pdl != 0, p);
+    }
+  } else if (p.wr_bulk) {
     if (gen) sy_observe_kernel<GEN_BEL_WARPS, GEN_WR_WARPS, WV_BULK><<<grid, THREADS, e->obs_smem, s>>>(p);
     else sy_observe_kernel<BEL_WARPS, WR_WARPS, WV_BULK><<<grid, THREADS, e->obs_smem, s>>>(p);
   } else {
@@ -3152,6 +3307,13 @@ int fill_params(const SyEnv* env, const SyState* st, const SyObs* ob, const SyOu
     p.wr_c_mask = env->wr_c_mask;
     p.wr_c_nf = ob->node_features_u8 ? env->wr_c_nf8 : env->wr_c_nf32;
     p.wr_img_bytes = env->wr_img_bytes;
+  }
+  if (env->grp_n) {
+    p.grp = (const GroupRow*)env->d_grp;
+    p.grp_id = (const int32_t*)env->d_grp_id;
+    p.grp_n = env->grp_n;
+    p.grp_rep = env->grp_rep;
+    p.grp_stats = (unsigned long long*)env->d_grp_stats;
   }
   return SY_OK;
 }
@@ -3241,6 +3403,8 @@ void sy_destroy(SyEnv* e) {
   if (e->d_cov) cudaFree(e->d_cov);
   if (e->d_bel_flags) cudaFree(e->d_bel_flags);
   if (e->d_stats_rep) cudaFree(e->d_stats_rep);
+  for (void* ptr : {e->d_grp, e->d_grp_id, e->d_grp_id_new, e->d_grp_bad, e->d_grp_stats})
+    if (ptr) cudaFree(ptr);
   if (e->aux_stream) cudaStreamDestroy(e->aux_stream);
   if (e->split_stream) cudaStreamDestroy(e->split_stream);
   for (cudaEvent_t ev : {e->ev_split_start, e->ev_split_logic, e->ev_split_belief})
@@ -3631,9 +3795,22 @@ int sy_reset(SyEnv* e, const uint8_t* reset_mask, const int32_t* init_pos, const
     CUDA_TRY(cudaGetLastError());
     e->obs_pending = false;
   }
-  sy_reset_kernel<<<(unsigned)((p.B + LOGIC_THREADS - 1) / LOGIC_THREADS), LOGIC_THREADS, 0, s>>>(p);
+  const unsigned rgrid = (unsigned)((p.B + LOGIC_THREADS - 1) / LOGIC_THREADS);
+  if (p.grp_n) sy_reset_kernel<1><<<rgrid, LOGIC_THREADS, 0, s>>>(p);
+  else sy_reset_kernel<<<rgrid, LOGIC_THREADS, 0, s>>>(p);
   g_launches++;
   CUDA_TRY(cudaGetLastError());
+  if (e->grp_need_reset && reset_mask) {  // does the mask cover every env?  (once after sy_set_groups: one synchronise)
+    int unset = 0;
+    CUDA_TRY(cudaMemsetAsync(e->d_grp_bad, 0, sizeof(int), s));
+    sy_count_unset_kernel<<<(unsigned)((p.B + 255) / 256), 256, 0, s>>>(reset_mask, p.B, (int*)e->d_grp_bad);
+    g_launches++;
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaMemcpyAsync(&unset, e->d_grp_bad, sizeof(int), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    if (unset == 0) e->grp_need_reset = false;
+  }
+  if (!reset_mask) e->grp_need_reset = false;  // every env starts an episode under its (new) group
   launch_observe(e, p, (unsigned)((p.B + TILE - 1) / TILE), s);
   g_launches++;
   CUDA_TRY(cudaGetLastError());
@@ -3654,6 +3831,12 @@ bool fused_eligible(const SyEnv* e, const SyObs* ob) {
 // next_actions (+ counter): a fused launch also draws the next step's random actions; *fused_sampled reports whether it did
 void launch_logic(const SyEnv* e, const Params& p, unsigned grid, cudaStream_t ls) {
   const bool f64 = e->cfg.reward_mode == SY_REWARD_FP64, pdl = e->opt_pdl != 0;
+  if (p.grp_n) {  // mechanism groups
+    if (p.A <= 4) launch_ex(f64 ? sy_logic_kernel<SY_REWARD_FP64, 4, 1> : sy_logic_kernel<SY_REWARD_FP32, 4, 1>, grid, LOGIC_THREADS, 0, ls, pdl, p);
+    else if (p.A <= 8) launch_ex(f64 ? sy_logic_kernel<SY_REWARD_FP64, 8, 1> : sy_logic_kernel<SY_REWARD_FP32, 8, 1>, grid, LOGIC_THREADS, 0, ls, pdl, p);
+    else launch_ex(f64 ? sy_logic_kernel<SY_REWARD_FP64, 16, 1> : sy_logic_kernel<SY_REWARD_FP32, 16, 1>, grid, LOGIC_THREADS, 0, ls, pdl, p);
+    return;
+  }
   if (p.A <= 4) {
     if (f64) launch_ex(sy_logic_kernel<SY_REWARD_FP64, 4>, grid, LOGIC_THREADS, 0, ls, pdl, p);
     else launch_ex(sy_logic_kernel<SY_REWARD_FP32, 4>, grid, LOGIC_THREADS, 0, ls, pdl, p);
@@ -3681,6 +3864,7 @@ int step_impl(SyEnv* e, const int64_t* actions, const int32_t* actions32, const 
   if (!e || (!actions && !actions32 && !actions16)) return fail(SY_ERR_INVALID_ARGUMENT, "NULL env / actions");
   if (actions16 && e->cfg.num_nodes > 32767) return fail(SY_ERR_INVALID_ARGUMENT, "int16 actions need num_nodes <= 32767");
   e->aux_after_logic = false;
+  if (e->grp_need_reset) return fail(SY_ERR_STATE, "mechanism groups changed: a sy_reset of every env (NULL or all-set mask) must come before the next step");
   if (!out) return fail(SY_ERR_INVALID_ARGUMENT, "SyOut is NULL");
   if (out->struct_bytes != sizeof(SyOut)) return fail(SY_ERR_INVALID_ARGUMENT, "SyOut size mismatch: got %llu, library expects %zu (ABI %d)", (unsigned long long)out->struct_bytes, sizeof(SyOut), SY_ABI_VERSION);
   if (!out->reward || !out->terminated || !out->truncated || !out->done || !out->winner)
@@ -3714,7 +3898,7 @@ int step_impl(SyEnv* e, const int64_t* actions, const int32_t* actions32, const 
     p.next_counter = next_counter;
     p.next_counter_base = next_counter_base;
     if (e->obs_pending && use_lagged(e) && !p.wr_bulk && !p.dbg_skip) {
-      lagged_fn(e)<<<grid, lagged_threads(e), e->obs_smem, s>>>(p);
+      lagged_fn(e, p.grp_n > 0)<<<grid, lagged_threads(e), e->obs_smem, s>>>(p);
     } else {
       if (e->obs_pending) {
         launch_observe(e, p, grid, s);
@@ -3755,7 +3939,7 @@ int step_impl(SyEnv* e, const int64_t* actions, const int32_t* actions32, const 
     p.f_off_nbr4 = e->f_off_nbr4;
     p.wr_epc = e->f_epc;
     const int threads = (e->f_bw + FUSED_WR + LOGIC_WARPS) * 32;
-    fused_fn(e->f_bw, e->cfg.reward_mode, p.A)<<<(unsigned)e->f_grid, threads, e->f_smem, s>>>(p);
+    fused_fn(e->f_bw, e->cfg.reward_mode, p.A, p.grp_n > 0)<<<(unsigned)e->f_grid, threads, e->f_smem, s>>>(p);
     g_launches++;
     CUDA_TRY(cudaGetLastError());
     if (after_logic) CUDA_TRY(cudaEventRecord(after_logic, s));
@@ -3767,7 +3951,7 @@ int step_impl(SyEnv* e, const int64_t* actions, const int32_t* actions32, const 
   // the belief propagation (split stream) and the writers of the ones (caller's stream) run next to each other.  Both
   // join on the caller's stream before step_impl returns (events; capturable in a CUDA graph as a DAG).
   const bool split = e->opt_fill && !ob->node_features_u8 && !p.wr_bulk && (reinterpret_cast<uintptr_t>(ob->node_features) & 15u) == 0 &&
-                     !p.dbg_skip && !e->bel_share_csr && e->cfg.num_envs >= SPLIT_MIN_ENVS;
+                     !p.dbg_skip && !e->bel_share_csr && e->cfg.num_envs >= SPLIT_MIN_ENVS && !e->grp_n;
   cudaStream_t ls = s;  // stream of the dynamics kernel
   if (split) {
     if (!e->split_stream) {
@@ -3981,6 +4165,7 @@ int sy_host_rollout_random(SyEnv* e, int32_t num_steps, uint32_t step_counter0, 
                            int32_t bytes_per_action, const SyState* st, const SyObs* ob, const SyOut* out,
                            const SyHostOut* ho, sy_stream_t stream) {
   if (!e || num_steps < 0) return fail(SY_ERR_INVALID_ARGUMENT, "NULL env or negative num_steps");
+  if (e->grp_need_reset) return fail(SY_ERR_STATE, "mechanism groups changed: a sy_reset of every env (NULL or all-set mask) must come before the next step");
   for (int32_t k = 0; k < num_steps; ++k) {
     int rc = sy_sample_actions_host(e, st, step_counter0 + (uint32_t)k, actions_dev, actions_host, bytes_per_action, stream);
     if (rc) return rc;
@@ -4012,6 +4197,80 @@ int sy_stats(SyEnv* e, int64_t* stats, sy_stream_t stream) {
   if (!e || !stats) return fail(SY_ERR_INVALID_ARGUMENT, "NULL env / stats");
   CUDA_TRY(cudaSetDevice(e->cfg.device));
   sy_fold_stats_kernel<<<1, 32, 0, (cudaStream_t)stream>>>((unsigned long long*)e->d_stats_rep, reinterpret_cast<long long*>(stats));
+  g_launches++;
+  CUDA_TRY(cudaGetLastError());
+  return SY_OK;
+}
+
+int sy_set_groups(SyEnv* e, int32_t n, const SyGroup* groups, const int32_t* group_id, sy_stream_t stream) {
+  if (!e) return fail(SY_ERR_INVALID_ARGUMENT, "NULL env");
+  if (e->obs_pending) return fail(SY_ERR_STATE, "sy_set_groups: observations are pending (sy_flush_observations first)");
+  if (n < 0 || n > SY_MAX_GROUPS) return fail(SY_ERR_INVALID_ARGUMENT, "num_groups must be in [0, %d], got %d", SY_MAX_GROUPS, n);
+  if (n > 0 && !groups) return fail(SY_ERR_INVALID_ARGUMENT, "SyGroup table is NULL");
+  std::vector<GroupRow> rows((size_t)n);
+  for (int g = 0; g < n; ++g) {
+    const SyGroup& q = groups[g];
+    if (q.struct_bytes != sizeof(SyGroup))
+      return fail(SY_ERR_INVALID_ARGUMENT, "SyGroup size mismatch in group %d: got %llu, library expects %zu (ABI %d)", g, (unsigned long long)q.struct_bytes, sizeof(SyGroup), SY_ABI_VERSION);
+    if (q.agent_money < 0 || q.reveal_interval < 0) return fail(SY_ERR_INVALID_ARGUMENT, "group %d: negative agent_money / reveal_interval", g);
+    if (!(q.reveal_skip_prob >= 0.0f && q.reveal_skip_prob <= 1.0f)) return fail(SY_ERR_INVALID_ARGUMENT, "group %d: reveal_skip_prob must be in [0, 1]", g);
+    for (int i = 0; i < SY_NUM_REWARD_WEIGHTS; ++i) {
+      if (!std::isfinite(q.reward_weights[i])) return fail(SY_ERR_INVALID_ARGUMENT, "group %d: reward weight %d is not finite", g, i);
+      rows[g].w64[i] = q.reward_weights[i];
+      rows[g].w32[i] = (float)q.reward_weights[i];
+    }
+    rows[g].agent_money = q.agent_money;
+    rows[g].reveal = q.reveal_interval;
+    rows[g].reveal_skip_thresh = q.reveal_skip_prob > 0.0f ? (unsigned long long)((double)fminf(q.reveal_skip_prob, 1.0f) * 4294967296.0) : 0ull;
+  }
+  CUDA_TRY(cudaSetDevice(e->cfg.device));
+  cudaStream_t s = (cudaStream_t)stream;
+  const int B = e->cfg.num_envs;
+  // The buffers are allocated once, at their largest, and updated in place: kernels in flight, and CUDA graphs captured
+  // earlier, never see a freed address (a graph captured under other groups still has to be recaptured -- its launches
+  // carry the old group count and kernel choice)
+  if (!e->d_grp) {
+    if (cudaMalloc(&e->d_grp, (size_t)SY_MAX_GROUPS * sizeof(GroupRow)) != cudaSuccess ||
+        cudaMalloc(&e->d_grp_id, (size_t)B * sizeof(int32_t)) != cudaSuccess ||
+        cudaMalloc(&e->d_grp_id_new, (size_t)B * sizeof(int32_t)) != cudaSuccess ||
+        cudaMalloc(&e->d_grp_stats, (size_t)GROUP_STAT_LINES * SY_NUM_STATS * sizeof(unsigned long long)) != cudaSuccess ||
+        cudaMalloc(&e->d_grp_bad, sizeof(int)) != cudaSuccess) {
+      for (void** ptr : {&e->d_grp, &e->d_grp_id, &e->d_grp_id_new, &e->d_grp_stats, &e->d_grp_bad}) {
+        if (*ptr) cudaFree(*ptr);
+        *ptr = nullptr;
+      }
+      return fail(SY_ERR_CUDA, "cudaMalloc of the mechanism group buffers failed");
+    }
+  }
+  if (n > 0) {
+    // ids into the staging buffer first: a rejected call leaves the handle's groups as they were
+    int bad = 0;
+    CUDA_TRY(cudaMemsetAsync(e->d_grp_bad, 0, sizeof(int), s));
+    sy_group_ids_kernel<<<(unsigned)((B + 255) / 256), 256, 0, s>>>(group_id, (int32_t*)e->d_grp_id_new, B, n,
+                                                                    (unsigned long long)e->cfg.env_offset, (int*)e->d_grp_bad);
+    g_launches++;
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaMemcpyAsync(&bad, e->d_grp_bad, sizeof(int), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    if (bad) return fail(SY_ERR_INVALID_ARGUMENT, "%d group ids outside [0, %d)", bad, n);
+    CUDA_TRY(cudaMemcpyAsync(e->d_grp_id, e->d_grp_id_new, (size_t)B * sizeof(int32_t), cudaMemcpyDeviceToDevice, s));
+    CUDA_TRY(cudaMemcpyAsync(e->d_grp, rows.data(), (size_t)n * sizeof(GroupRow), cudaMemcpyHostToDevice, s));
+  }
+  CUDA_TRY(cudaMemsetAsync(e->d_grp_stats, 0, (size_t)GROUP_STAT_LINES * SY_NUM_STATS * sizeof(unsigned long long), s));
+  CUDA_TRY(cudaStreamSynchronize(s));  // (the host table is a local)
+  e->grp_n = n;
+  // per-group lines spread like the handle-wide replicas: rep * n <= GROUP_STAT_LINES for every n <= SY_MAX_GROUPS
+  e->grp_rep = n ? std::max(1, std::min(STAT_REPLICAS, GROUP_STAT_LINES / n)) : 0;
+  e->grp_need_reset = true;
+  return SY_OK;
+}
+
+int sy_group_stats(SyEnv* e, int32_t n, int64_t* stats, sy_stream_t stream) {
+  if (!e || !stats) return fail(SY_ERR_INVALID_ARGUMENT, "NULL env / stats");
+  if (n != e->grp_n || n == 0) return fail(SY_ERR_INVALID_ARGUMENT, "sy_group_stats: num_groups %d, but the handle holds %d groups", n, e->grp_n);
+  CUDA_TRY(cudaSetDevice(e->cfg.device));
+  const int total = n * SY_NUM_STATS;
+  sy_fold_group_stats_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>((unsigned long long*)e->d_grp_stats, n, e->grp_rep, reinterpret_cast<long long*>(stats));
   g_launches++;
   CUDA_TRY(cudaGetLastError());
   return SY_OK;
@@ -4095,7 +4354,7 @@ int rollout_one_launch(SyEnv* e, int32_t num_steps, int64_t* actions, uint32_t n
   p.next_counter_base = next_counter_base;
   CUDA_TRY(cudaSetDevice(e->cfg.device));
   e->aux_after_logic = false;
-  rollout_fn(e)<<<(unsigned)((p.B + TILE - 1) / TILE), lagged_threads(e), e->obs_smem, s>>>(p, (int)num_steps);
+  rollout_fn(e, p.grp_n > 0)<<<(unsigned)((p.B + TILE - 1) / TILE), lagged_threads(e), e->obs_smem, s>>>(p, (int)num_steps);
   g_launches++;
   CUDA_TRY(cudaGetLastError());
   return SY_OK;
@@ -4113,6 +4372,7 @@ extern "C" {
 int sy_rollout_random(SyEnv* e, int32_t num_steps, uint32_t step_counter0, int64_t* actions, const SyState* st, const SyObs* ob,
                       const SyOut* out, sy_stream_t stream) {
   if (!e || !actions || num_steps < 0) return fail(SY_ERR_INVALID_ARGUMENT, "NULL env / actions or negative num_steps");
+  if (e->grp_need_reset) return fail(SY_ERR_STATE, "mechanism groups changed: a sy_reset of every env (NULL or all-set mask) must come before the next step");
   if (num_steps >= 2 && one_launch_rollout(e, ob)) {
     int rc = sy_flush_observations(e, st, ob, stream);
     if (!rc) rc = sy_sample_actions(e, st, step_counter0, actions, stream);
@@ -4137,6 +4397,7 @@ int sy_rollout_random(SyEnv* e, int32_t num_steps, uint32_t step_counter0, int64
 int sy_rollout_random_dev(SyEnv* e, int32_t num_steps, uint32_t* step_counter_dev, int64_t* actions, const SyState* st,
                           const SyObs* ob, const SyOut* out, sy_stream_t stream) {
   if (!e || !actions || !step_counter_dev || num_steps < 0) return fail(SY_ERR_INVALID_ARGUMENT, "NULL env / actions / counter or negative num_steps");
+  if (e->grp_need_reset) return fail(SY_ERR_STATE, "mechanism groups changed: a sy_reset of every env (NULL or all-set mask) must come before the next step");
   cudaStream_t s = (cudaStream_t)stream;
   int rc = SY_OK;
   if (num_steps >= 2 && one_launch_rollout(e, ob)) {

@@ -36,6 +36,51 @@ MAX_MONEY_LIMIT = 1000  # yard.py:11
 N_EXP_TABLE = 1100  # exp(-d) underflows to 0 beyond d = 745
 
 
+MECHANISM_KEYS = ("reward_weights", "agent_money", "reveal_interval", "reveal_skip_prob")
+
+
+def pack_mechanism(mech: Dict, base) -> "_cabi.SyGroup":
+    """One mechanism dict (keys of MECHANISM_KEYS, all optional) as the SyGroup of sy_set_groups; missing keys and
+    missing reward-weight names take `base`'s values (an env, or anything with `reward_weights`, `agent_money`,
+    `reveal_interval` and `config.reveal_skip_prob`).  Raises ValueError / KeyError on what the library would refuse."""
+    if not isinstance(mech, dict):
+        raise TypeError(f"a mechanism is a dict, got {type(mech).__name__}")
+    unknown = set(mech) - set(MECHANISM_KEYS)
+    if unknown:
+        raise KeyError(f"unknown mechanism keys {sorted(unknown)}; expected {list(MECHANISM_KEYS)}")
+    weights = dict(base.reward_weights)
+    given = mech.get("reward_weights", {}) or {}
+    bad = set(given) - set(REWARD_WEIGHT_NAMES)
+    if bad:
+        raise KeyError(f"unknown reward weights {sorted(bad)}")
+    weights.update(given)
+    w = [float(weights[k].detach()) if isinstance(weights[k], torch.Tensor) else float(weights[k]) for k in REWARD_WEIGHT_NAMES]
+    if not all(np.isfinite(w)):
+        raise ValueError("reward weights must be finite")
+    money = mech.get("agent_money", base.agent_money)
+    reveal = mech.get("reveal_interval", base.reveal_interval)
+    skip = float(mech.get("reveal_skip_prob", base.config.reveal_skip_prob))
+    if int(money) != money or int(money) < 0:
+        raise ValueError(f"agent_money must be a non-negative integer, got {money}")
+    if int(reveal) != reveal or int(reveal) < 0:
+        raise ValueError(f"reveal_interval must be a non-negative integer, got {reveal}")
+    if not 0.0 <= skip <= 1.0:
+        raise ValueError(f"reveal_skip_prob must be in [0, 1], got {skip}")
+    g = _cabi.SyGroup()
+    g.struct_bytes = C.sizeof(_cabi.SyGroup)
+    for i, v in enumerate(w):
+        g.reward_weights[i] = v
+    g.agent_money, g.reveal_interval, g.reveal_skip_prob = int(money), int(reveal), skip
+    return g
+
+
+def unpack_mechanism(g: "_cabi.SyGroup") -> Dict:
+    """The complete mechanism dict of a SyGroup (float weights)"""
+    return dict(reward_weights={k: float(g.reward_weights[i]) for i, k in enumerate(REWARD_WEIGHT_NAMES)},
+                agent_money=int(g.agent_money), reveal_interval=int(g.reveal_interval),
+                reveal_skip_prob=float(g.reveal_skip_prob))
+
+
 def numpy_reward_tables(max_timestep: int = 250):
     """The two float64 tables the kernels read instead of calling exp/log1p, computed by NumPy
     on this host so the rewards equal the reference's `np.exp` bit for bit
@@ -205,6 +250,9 @@ class BatchedScotlandYardEnv:
         self._static = None
         self._sample_counter = 0
         self._is_reset = False
+        self._need_full_reset = False
+        self._mechanisms, self._group_id, self.group_stats_vec = None, None, None  # set_mechanisms
+        self._groups_generation = 0  # set_mechanisms calls: captured rollout graphs check it
 
     # ------------------------------------------------------------------ plumbing
     def _result_bytes(self) -> int:
@@ -309,6 +357,8 @@ class BatchedScotlandYardEnv:
             restart = not self._is_reset
         if not self._is_reset and m is not None:
             raise _cabi.SyError("the first reset must cover every env")
+        if self._need_full_reset and m is not None and not bool(m.all()):
+            raise _cabi.SyError("the first reset after set_mechanisms must cover every env")
         if gi is None and not self._is_reset and not self.config.resample_graph:
             # blocks of 32 consecutive envs share a graph: the kernels' 32-env tiles then stay on the single-graph fast
             # paths (shared-memory CSR, lane = env belief propagation) for pools of up to B / 32 graphs
@@ -318,6 +368,7 @@ class BatchedScotlandYardEnv:
             _cabi.check(self._lib.sy_reset(self._handle, _ptr(m), _ptr(ip), _ptr(gi), int(bool(restart)),
                                            C.byref(self._state), C.byref(self._obs), self._stream()))
         self._is_reset = True
+        self._need_full_reset = False
         self._keep = (m, ip, gi)  # keep inputs alive until the stream has consumed them
         return self.observation()
 
@@ -367,6 +418,45 @@ class BatchedScotlandYardEnv:
     @property
     def observations_pending(self) -> bool:
         return bool(self._lib.sy_observations_pending(self._handle))
+
+    # ------------------------------------------------------------------ mechanism groups
+    def set_mechanisms(self, mechanisms, group_id=None):
+        """Evaluate several mechanisms in this one batch (sy_set_groups).  `mechanisms`: a sequence of dicts with the
+        optional keys `reward_weights` (a dict keyed by REWARD_WEIGHT_NAMES, floats or 0-dim tensors; missing names keep
+        the constructor's weight), `agent_money`, `reveal_interval` and `reveal_skip_prob` (a missing key keeps the
+        constructor's value).  `group_id`: int tensor [B] (env -> index into `mechanisms`), or None for
+        (env_offset + b) % len(mechanisms).  `mechanisms=None` clears the groups.  Pending observations are flushed
+        first; the new mechanisms take effect at the next full `reset()`, which `step` and the rollouts require."""
+        self.flush_observations()
+        if mechanisms is None:
+            table, gid = [], None
+        else:
+            table = [pack_mechanism(m, self) for m in mechanisms]
+            if not 1 <= len(table) <= _cabi.SY_MAX_GROUPS:
+                raise ValueError(f"between 1 and {_cabi.SY_MAX_GROUPS} mechanisms, got {len(table)}")
+            gid = None if group_id is None else self._dev(group_id, torch.int32, (self.num_envs,))
+        arr = (_cabi.SyGroup * max(len(table), 1))(*table)
+        with torch.cuda.device(self.device):
+            _cabi.check(self._lib.sy_set_groups(self._handle, len(table), arr, _ptr(gid), self._stream()))
+        self._mechanisms = None if mechanisms is None else tuple(unpack_mechanism(g) for g in table)
+        self._group_id = None
+        if table:
+            self._group_id = gid.clone() if gid is not None else (
+                (torch.arange(self.num_envs, device=self.device, dtype=torch.int64) + self.env_offset) % len(table)).to(torch.int32)
+        self.group_stats_vec = torch.zeros(len(table), _cabi.SY_NUM_STATS, dtype=torch.int64, device=self.device) \
+            if table and self.stats_vec is not None else None
+        self._need_full_reset = True  # the next reset() covers every env
+        self._groups_generation += 1
+
+    @property
+    def mechanisms(self):
+        """The mechanism groups as set (tuple of complete dicts), or None"""
+        return self._mechanisms
+
+    @property
+    def group_id(self) -> Optional[torch.Tensor]:
+        """int32 [B] group of each env while mechanism groups are set (a copy), else None"""
+        return None if self._group_id is None else self._group_id.clone()
 
     def sample_actions(self, out: Optional[torch.Tensor] = None, step_counter: Optional[int] = None) -> torch.Tensor:
         """Uniform random valid action per agent on the device (-1 when an agent cannot move)."""
@@ -426,7 +516,7 @@ class BatchedScotlandYardEnv:
         with torch.cuda.device(self.device), torch.cuda.graph(graph, stream=side):
             issue()
         self._rollout_graph_keepalive = (actions, counter)
-        return graph, counter
+        return _RolloutGraph(graph, self), counter
 
     def _host_buffers(self):
         if getattr(self, "_host", None) is None:
@@ -639,13 +729,23 @@ class BatchedScotlandYardEnv:
         d = int(self.graph_tables(g)[1][node1, node2])
         return float("inf") if d == 0xFFFF else float(d)
 
-    def stats(self, reduce_group=None) -> Dict[str, int]:
+    def stats(self, reduce_group=None, by_group: bool = False):
         """Episode statistics accumulated on the device; with `reduce_group` (or an initialised
         default process group and reduce_group=True) they are summed over ranks with one
-        all-reduce (NCCL over NVLink on a GPU box)."""
+        all-reduce (NCCL over NVLink on a GPU box).  by_group=True: one dict per mechanism group."""
         if self.stats_vec is None:
             raise _cabi.SyError("collect_stats=False")
         self._fold_stats()
+        if by_group:
+            if self.group_stats_vec is None:
+                raise _cabi.SyError("no mechanism groups are set")
+            t = self.group_stats_vec
+            if reduce_group is not None:
+                import torch.distributed as dist
+
+                t = t.clone()
+                dist.all_reduce(t, group=None if reduce_group is True else reduce_group)
+            return [{k: int(row[i]) for i, k in enumerate(_cabi.STAT_NAMES)} for row in t.cpu().tolist()]
         if reduce_group is not None:
             from .sharding import allreduce_stats
 
@@ -653,12 +753,25 @@ class BatchedScotlandYardEnv:
         h = self.stats_vec.cpu().tolist()
         return {k: int(h[i]) for i, k in enumerate(_cabi.STAT_NAMES)}
 
-    def metrics(self, reduce_group=None) -> Dict[str, float]:
+    def metrics(self, reduce_group=None, by_group: bool = False):
         """The aggregates of the reference's MetricsTracker.get_aggregated_metrics (src/eval/metrics.py:168-232) from
         the device statistics vector -- same keys.  `mean_belief_ce` / `belief_ce_std` (metrics.py:194-197,217-218):
         cross-entropy of the predicted belief at MrX's node over all reveal steps (belief_quality.py:8-11), scored
-        inside the observe kernel before the reveal collapses the map."""
+        inside the observe kernel before the reveal collapses the map.  by_group=True: one dict per mechanism group
+        (its budget efficiency against its own agent_money).  While groups are set, the aggregate efficiency weighs
+        every group's spending against that group's budget."""
+        if by_group:
+            return [self._metrics_of(st, initial=max(self.number_of_agents * m["agent_money"], 1))
+                    for st, m in zip(self.stats(reduce_group, by_group=True), self._mechanisms)]
         st = self.stats(reduce_group)
+        eff = None
+        if self._mechanisms is not None and self.group_stats_vec is not None:
+            per = self.stats(reduce_group, by_group=True)
+            eff = sum(g["sum_episode_budget_spent"] / max(self.number_of_agents * m["agent_money"], 1)
+                      for g, m in zip(per, self._mechanisms))
+        return self._metrics_of(st, initial=max(self.number_of_agents * self.agent_money, 1), eff_sum=eff)
+
+    def _metrics_of(self, st, initial, eff_sum=None) -> Dict[str, float]:
         n = st["episodes"]
         r = st["reveals"]
         mean_ce = st["sum_belief_ce_q24"] / _cabi.BELIEF_CE_SCALE / r if r else 0.0
@@ -672,13 +785,12 @@ class BatchedScotlandYardEnv:
         ml = st["sum_episode_length"] / n
         var_l = max(st["sum_sq_episode_length"] / n - ml * ml, 0.0)
         spent = st["sum_episode_budget_spent"] / n
-        initial = max(self.number_of_agents * self.agent_money, 1)
         return dict(
             num_episodes=n, mrx_wins=st["mrx_wins"], police_wins=st["police_wins"], win_rate=wr,
             win_rate_std=float(np.sqrt(wr * (1.0 - wr))), mean_episode_length=ml, episode_length_std=float(np.sqrt(var_l)),
             mean_belief_ce=mean_ce, belief_ce_std=float(np.sqrt(var_ce)),
             mean_tolls_paid=self.tolls * st["police_moves"] / n, mean_budget_spent=spent,
-            mean_budget_efficiency=spent / initial,
+            mean_budget_efficiency=spent / initial if eff_sum is None else eff_sum / n,
             mean_time_to_catch=st["sum_length_police_wins"] / st["police_wins"] if st["police_wins"] else 0.0,
             mean_survival_time=st["sum_length_mrx_wins"] / st["mrx_wins"] if st["mrx_wins"] else 0.0,
         )
@@ -688,22 +800,56 @@ class BatchedScotlandYardEnv:
         if self.stats_vec is not None:
             with torch.cuda.device(self.device):
                 _cabi.check(self._lib.sy_stats(self._handle, self.stats_vec.data_ptr(), self._stream()))
+                if self.group_stats_vec is not None:
+                    _cabi.check(self._lib.sy_group_stats(self._handle, self.group_stats_vec.shape[0],
+                                                         self.group_stats_vec.data_ptr(), self._stream()))
 
     def reset_stats(self):
         if self.stats_vec is not None:
             self._fold_stats()
             self.stats_vec.zero_()
+            if self.group_stats_vec is not None:
+                self.group_stats_vec.zero_()
 
     def state_dict(self) -> Dict[str, torch.Tensor]:
         keys = ["pos", "money", "timestep", "graph_id", "episode", "done", "visits", "belief_map", "action_mask",
                 "node_features", "agent_budget", "mrx_revealed", "stats_vec"]
         self._fold_stats()
-        return {k: getattr(self, k).clone() for k in keys if getattr(self, k) is not None}
+        sd = {k: getattr(self, k).clone() for k in keys if getattr(self, k) is not None}
+        if self._group_id is not None:  # mechanism groups: the assignment and the per-group statistics
+            sd["group_id"] = self._group_id.clone()
+            if self.group_stats_vec is not None:
+                sd["group_stats_vec"] = self.group_stats_vec.clone()
+        return sd
 
     def load_state_dict(self, sd: Dict[str, torch.Tensor]):
+        """Restore a `state_dict`.  One taken while mechanism groups were set needs the same groups set first (with
+        `set_mechanisms`).  Mechanism groups cannot be resumed mid-episode: after `set_mechanisms` the library requires a
+        full `reset()` before the next step, which starts new episodes -- what carries over is the statistics, the
+        per-group ones included."""
+        if ("group_id" in sd) != (self._group_id is not None) or (
+                "group_id" in sd and not torch.equal(sd["group_id"].to(self._group_id.device), self._group_id)):
+            raise ValueError("the state dict's mechanism groups differ from this env's: set_mechanisms() first")
         for k, v in sd.items():
-            getattr(self, k).copy_(v)
+            if k != "group_id":
+                getattr(self, k).copy_(v)
         self._is_reset = True
+
+
+class _RolloutGraph:
+    """A captured rollout graph (torch.cuda.CUDAGraph) that refuses to replay once the env's mechanism groups changed:
+    its launches carry the groups -- and the kernels chosen for them -- of the time it was captured."""
+
+    def __init__(self, graph, env):
+        self.graph, self._env, self._generation = graph, env, env._groups_generation
+
+    def replay(self):
+        if self._env._groups_generation != self._generation:
+            raise _cabi.SyError("the mechanism groups changed since this rollout graph was captured: capture it again")
+        self.graph.replay()
+
+    def __getattr__(self, name):
+        return getattr(self.graph, name)
 
 
 class _LazyGather:

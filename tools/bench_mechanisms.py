@@ -1,0 +1,128 @@
+"""Cost of mechanism groups (env.set_mechanisms) at c3 and c2: four variants of the same handle in one process,
+timed alternately, median of 5 passes each -- no groups, one group equal to the config, 16 groups interleaved
+(the default b % 16 assignment) and 1 024 groups, the groups differing in their reward weights only.  Two timings per variant: `sy_step` (K plain steps between a CUDA
+event pair, actions drawn once beforehand) and the replayed `capture_rollout` graph (K steps of the random policy).
+c3 runs with the belief scored at reveal steps (belief_ce), so the per-group cross-entropy atomics are included.
+Writes profiles/r03_mechanisms_c{2,3}.json (or --out-dir) with the card's name and power limit.
+
+    python tools/bench_mechanisms.py [--workloads c3,c2] [--steps 50] [--passes 5]
+"""
+import argparse
+import json
+import os
+import statistics
+import subprocess
+import sys
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+WORKLOADS = {  # bench.py's c2 / c3 (c3 with the belief scored at reveals)
+    "c2": dict(N=50, E=110, P=3, money=10, toll=0, belief=False, reveal=5, B=1024),
+    "c3": dict(N=200, E=400, P=6, money=20, toll=1, belief=True, reveal=5, B=65536),
+}
+VARIANTS = ["no_groups", "one_group_equal", "groups_16", "groups_1024"]
+
+
+def card():
+    try:
+        q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                           capture_output=True, text=True, timeout=30).stdout.strip().splitlines()[0]
+        name, power, sm = [x.strip() for x in q.split(",")]
+        return dict(name=name, power_limit=power, sm_max_clock=sm)
+    except Exception as exc:  # noqa: BLE001
+        import torch
+
+        return dict(name=torch.cuda.get_device_name(0), power_limit=f"unknown ({exc.__class__.__name__})")
+
+
+def run(wl_name, steps, passes):
+    import torch
+
+    from student_mechanism_design_b200 import BatchedScotlandYardEnv
+
+    wl = WORKLOADS[wl_name]
+    envs = {}
+    for v in VARIANTS:
+        env = BatchedScotlandYardEnv(wl["B"], wl["P"], wl["money"], graph_nodes=wl["N"], graph_edges=wl["E"], seed=0,
+                                     num_graphs=1, tolls=wl["toll"], belief=wl["belief"], belief_ce=wl["belief"],
+                                     reveal_interval=wl["reveal"], auto_reset=True, device="cuda:0")
+        if v == "one_group_equal":
+            env.set_mechanisms([{}])
+        elif v in ("groups_16", "groups_1024"):
+            # distinct mechanisms with the config's budget and reveal schedule: only the reward weights differ, so
+            # every variant does the same game work and the difference is the cost of the groups themselves
+            n = 16 if v == "groups_16" else 1024
+            env.set_mechanisms([dict(reward_weights={"Mrx_closest": 0.3 + 0.001 * g, "Police_distance": 0.1 + 0.001 * g})
+                                for g in range(n)])
+        env.reset()
+        acts = env.sample_actions(step_counter=0)
+        graph, _ = env.capture_rollout(steps)
+        for _ in range(3):  # warm every shape of the timed window
+            env.step(acts)
+            graph.replay()
+        envs[v] = (env, acts, graph)
+    torch.cuda.synchronize()
+    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    times = {v: {"sy_step_ms": [], "graph_replay_ms": []} for v in VARIANTS}
+    for p in range(passes):
+        order = VARIANTS if p % 2 == 0 else VARIANTS[::-1]  # alternate, so drift does not favour one variant
+        for v in order:
+            env, acts, graph = envs[v]
+            ev0.record()
+            for _ in range(steps):
+                env.step(acts)
+            ev1.record()
+            torch.cuda.synchronize()
+            times[v]["sy_step_ms"].append(ev0.elapsed_time(ev1) / steps)
+            ev0.record()
+            graph.replay()
+            ev1.record()
+            torch.cuda.synchronize()
+            times[v]["graph_replay_ms"].append(ev0.elapsed_time(ev1) / steps)
+    out = {}
+    for v in VARIANTS:
+        env = envs[v][0]
+        row = {}
+        for k, xs in times[v].items():
+            row[k] = statistics.median(xs)
+            row[k + "_passes"] = [round(x, 5) for x in xs]
+            row[k + "_spread"] = max(xs) - min(xs)
+        row["groups"] = 0 if env.mechanisms is None else len(env.mechanisms)
+        out[v] = row
+    base = out["no_groups"]
+    for v in VARIANTS[1:]:
+        for k in ("sy_step_ms", "graph_replay_ms"):
+            out[v][k + "_vs_no_groups"] = out[v][k] / base[k] - 1.0
+    for env, _, _ in envs.values():
+        env.close()
+    return out
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--workloads", default="c3,c2")
+    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--passes", type=int, default=5)
+    ap.add_argument("--out-dir", default=os.path.join(ROOT, "profiles"))
+    args = ap.parse_args()
+    import torch
+
+    if not torch.cuda.is_available():
+        sys.exit("bench_mechanisms.py needs a CUDA device")
+    info = card()
+    os.makedirs(args.out_dir, exist_ok=True)
+    for w in args.workloads.split(","):
+        res = dict(workload=w, config=WORKLOADS[w], steps_per_pass=args.steps, passes=args.passes, card=info,
+                   note="every variant takes the handle's usual path (c3: dynamics + observation kernels, c2: fused "
+                        "step / one-launch rollout kernel), the grouped ones through its GROUPS instantiation; c3 scores "
+                        "the belief at reveal steps (about 4 us per step over bench.py's c3 line, which does not)",
+                   variants=run(w, args.steps, args.passes))
+        path = os.path.join(args.out_dir, f"r03_mechanisms_{w}.json")
+        with open(path, "w") as f:
+            json.dump(res, f, indent=1)
+        print(json.dumps(res))
+
+
+if __name__ == "__main__":
+    main()
