@@ -26,6 +26,23 @@ def u01(word: int) -> float:
     return float(np.float32(word >> 8) * np.float32(1.0 / 16777216.0))
 
 
+def philox4x32_batched(c0, c1, c2, c3, seed):
+    """`sy_oracle.philox4x32` over arrays of counters (broadcast), one 64-bit key: four uint32 arrays."""
+    m = np.uint64(_M32)
+    c = [np.asarray(x, dtype=np.uint64) & m for x in np.broadcast_arrays(c0, c1, c2, c3)]
+    k0, k1 = np.uint64(seed & _M32), np.uint64((seed >> 32) & _M32)
+    for _ in range(10):
+        p0, p1 = np.uint64(0xD2511F53) * c[0], np.uint64(0xCD9E8D57) * c[2]  # 32 x 32 bits: exact in uint64
+        c = [((p1 >> np.uint64(32)) ^ c[1] ^ k0) & m, p1 & m, ((p0 >> np.uint64(32)) ^ c[3] ^ k1) & m, p0 & m]
+        k0, k1 = (k0 + np.uint64(0x9E3779B9)) & m, (k1 + np.uint64(0xBB67AE85)) & m
+    return [x.astype(np.uint32) for x in c]
+
+
+def u01_batched(words) -> np.ndarray:
+    """float32 [0, 1) of the kernels' u01, elementwise"""
+    return (np.asarray(words, dtype=np.uint32) >> np.uint32(8)).astype(np.float32) * np.float32(1.0 / 16777216.0)
+
+
 # ------------------------------------------------------------------------------------------ GNN
 def graph_features(mode, pos, revealed, n_nodes, n_agents) -> np.ndarray:
     """x [N, K=A].  FEATURES_ENV: the env's node_features (yard.py:283-291, MrX column blank while hidden).
@@ -64,6 +81,62 @@ def gnn_forward(x, edge_links, sd, epsilon=0.1, gamma=0.1) -> np.ndarray:
     return (x @ f("output_layer.weight").T).reshape(-1) + float(f("output_layer.bias").reshape(-1)[0])
 
 
+def graph_features_batched(mode, pos, revealed, n_nodes, n_agents) -> np.ndarray:
+    """`graph_features` of many envs at once: x [B, N, K=A] from pos [B, A] and revealed [B]."""
+    pos, revealed = np.asarray(pos, dtype=np.int64), np.asarray(revealed)
+    B = len(pos)
+    b = np.arange(B)
+    x = np.zeros((B, n_nodes, n_agents), dtype=np.float64)
+    if mode == FEATURES_ENV:
+        for k in range(n_agents):
+            on = revealed >= 0 if k == 0 else np.ones(B, dtype=bool)
+            x[b[on], pos[on, k], k] = 1
+    else:
+        x[b, np.where(revealed >= 0, pos[:, 0], n_nodes - 1), 0] = 1
+        for i in range(n_agents - 2):
+            x[b, pos[:, 1], i + 1] = 1
+    return x
+
+
+def gcn_matrix(edge_links, n_nodes):
+    """GCNConv's normalised propagation as a sparse [N, N] matrix (row = target): one entry per stored edge u -> v with
+    deg[u]^-1/2 deg[v]^-1/2 (parallel edges are separate messages, so their entries add up), self-loops 1/deg[v]."""
+    import scipy.sparse as sp
+
+    src, dst = np.asarray(edge_links)[:, 0].astype(np.int64), np.asarray(edge_links)[:, 1].astype(np.int64)
+    dis = (1.0 + np.bincount(dst, minlength=n_nodes)) ** -0.5
+    v = np.arange(n_nodes)
+    return sp.csr_matrix((np.concatenate([dis[src] * dis[dst], dis * dis]), (np.concatenate([dst, v]), np.concatenate([src, v]))),
+                         shape=(n_nodes, n_nodes))
+
+
+def gnn_forward_batched(mode, pos, revealed, graph_id, edge_links, sds, n_nodes, epsilon=0.1, gamma=0.1,
+                        chunk_floats=1 << 23) -> np.ndarray:
+    """`gnn_forward` of every env and every model in `sds`: q [B, len(sds), N] float64.  Features follow
+    `graph_features_batched`, env b aggregates over graph `edge_links[graph_id[b]]`; envs are processed in chunks of at
+    most `chunk_floats` feature entries so that a full batch fits in host memory."""
+    pos, revealed, graph_id = np.asarray(pos), np.asarray(revealed), np.asarray(graph_id)
+    B, K = pos.shape
+    mats = [gcn_matrix(el, n_nodes) for el in edge_links]
+    f = [{k: np.asarray(sd[k], dtype=np.float64) for k in sd} for sd in sds]
+    q = np.zeros((B, len(sds), n_nodes), dtype=np.float64)
+    step = max(1, chunk_floats // (n_nodes * K))
+    for g, Ahat in enumerate(mats):
+        envs = np.nonzero(graph_id == g)[0]
+        for c0 in range(0, len(envs), step):
+            e = envs[c0: c0 + step]
+            x0 = graph_features_batched(mode, pos[e], revealed[e], n_nodes, K)
+            for m, w in enumerate(f):
+                x = x0
+                for c in ("conv1", "conv2"):
+                    xl = x @ w[f"{c}.phi.lin.weight"].T
+                    agg = (Ahat @ xl.transpose(1, 0, 2).reshape(n_nodes, -1)).reshape(n_nodes, len(e), K).transpose(1, 0, 2)
+                    h = x @ (w[f"{c}.W"] - w[f"{c}.W"].T - gamma * np.eye(K)).T + agg + w[f"{c}.bias"]
+                    x = np.maximum(x + epsilon * np.tanh(h), 0)
+                q[e, m] = (x @ w["output_layer.weight"].T)[..., 0] + float(w["output_layer.bias"].reshape(-1)[0])
+    return q
+
+
 def gnn_select(q, valid_moves, eps, seed, env, step, agent, tie_tol=0.0):
     """GNNAgent.select_action (gnn_agent.py:62-82) with the kernel's Philox draws.  Returns (action or -1, explored,
     set of acceptable argmax nodes within tie_tol)."""
@@ -76,6 +149,22 @@ def gnn_select(q, valid_moves, eps, seed, env, step, agent, tie_tol=0.0):
     qv = q[valid_moves]
     a = int(valid_moves[int(np.argmax(qv))])
     return a, False, {int(m) for m, v in zip(valid_moves, qv) if v >= qv.max() - tie_tol}
+
+
+def gnn_explore_batched(mask, eps_mrx, eps_police, seed, env_ids, step):
+    """The exploration half of `gnn_select` for all envs and agents: (explored [B, A] bool, action [B, A] = the drawn
+    valid move where explored, else -1).  Agents without a valid move never explore."""
+    mask = np.asarray(mask, dtype=bool)
+    B, A, N = mask.shape
+    r = philox4x32_batched(np.asarray(env_ids)[:, None], step, RNG_GNN_POLICY, np.arange(A)[None, :], seed)
+    eps = np.full(A, np.float32(eps_police), dtype=np.float32)
+    eps[0] = np.float32(eps_mrx)
+    n_valid = mask.sum(-1)
+    explored = (u01_batched(r[0]) < eps[None, :]) & (n_valid > 0)
+    target = (r[1].astype(np.uint64) * n_valid.astype(np.uint64)) >> np.uint64(32)  # index into the ascending valid moves
+    rank = np.cumsum(mask, axis=-1, dtype=np.int16) - np.int16(1)
+    hit = mask & (rank == target[..., None].astype(np.int16))
+    return explored, np.where(explored, hit.argmax(-1), -1)
 
 
 # ------------------------------------------------------------------------------------------ MAPPO
@@ -92,6 +181,52 @@ def mappo_probs(obs, sd, mask, dtype=np.float64):
     if s <= 1e-8:
         return m / m.sum() if m.sum() > 1e-8 else np.ones_like(m) / len(m)
     return p / (s + dtype(1e-8))
+
+
+MAPPO_SOFTMAX, MAPPO_UNIFORM_MASK, MAPPO_UNIFORM_ALL = 0, 1, 2
+
+
+def mappo_forward_batched(obs, sd, mask, chunk=8192):
+    """`mappo_probs` for many rows of ONE policy: obs [R, D], mask [R, N].  Returns a dict of float64 / int arrays:
+    `probs` [R, N], `mode` [R] (MAPPO_SOFTMAX: softmax * mask / (Sv + 1e-8); MAPPO_UNIFORM_MASK; MAPPO_UNIFORM_ALL),
+    `masked` [R, N] (the softmax branch's probabilities whichever branch the row takes), `Sv` [R] (the softmax mass on
+    the mask) and `scale` [R] = max_n (|b2_n| + sum_k |W2_nk| (|b1_k| + sum_o |W1_ko x_o|)), the magnitude every
+    rounding error of a float32 evaluation of the logits is proportional to."""
+    f = lambda k: np.asarray(sd[k], dtype=np.float64)  # noqa: E731
+    W1, b1, W2, b2 = f("actor.0.weight"), f("actor.0.bias"), f("actor.2.weight"), f("actor.2.bias")
+    obs, mask = np.asarray(obs, dtype=np.float64), np.asarray(mask, dtype=bool)
+    R, N = mask.shape
+    out = dict(probs=np.zeros((R, N)), masked=np.zeros((R, N)), mode=np.zeros(R, dtype=np.int64), Sv=np.zeros(R), scale=np.zeros(R))
+    aW1, ab1, aW2, ab2 = np.abs(W1), np.abs(b1), np.abs(W2), np.abs(b2)
+    for r0 in range(0, R, chunk):
+        x, m = obs[r0: r0 + chunk], mask[r0: r0 + chunk]
+        h = np.maximum(x @ W1.T + b1, 0)
+        logits = h @ W2.T + b2
+        e = np.exp(logits - logits.max(-1, keepdims=True))
+        p = e / e.sum(-1, keepdims=True)
+        Sv = (p * m).sum(-1)
+        nv = m.sum(-1)
+        mode = np.where(Sv > 1e-8, MAPPO_SOFTMAX, np.where(nv > 0, MAPPO_UNIFORM_MASK, MAPPO_UNIFORM_ALL))
+        masked = p * m / (Sv + 1e-8)[:, None]
+        probs = np.where(mode[:, None] == MAPPO_SOFTMAX, masked,
+                         np.where(mode[:, None] == MAPPO_UNIFORM_MASK, m / np.maximum(nv, 1)[:, None], 1.0 / N))
+        s1 = ab1 + np.abs(x) @ aW1.T  # |b1_k| + sum_o |W1_ko| |x_o|: bounds the hidden unit's partial sums
+        out["probs"][r0: r0 + chunk] = probs
+        out["masked"][r0: r0 + chunk] = masked
+        out["mode"][r0: r0 + chunk] = mode
+        out["Sv"][r0: r0 + chunk] = Sv
+        out["scale"][r0: r0 + chunk] = (ab2 + s1 @ aW2.T).max(-1)
+    return out
+
+
+def critic_value_batched(x, sd):
+    """`critic_value` of every row of x [M, D]: (values [M], scale [M] as in `mappo_forward_batched`)."""
+    f = lambda k: np.asarray(sd[k], dtype=np.float64)  # noqa: E731
+    W1, b1, W2, b2 = f("critic.0.weight"), f("critic.0.bias"), f("critic.2.weight").reshape(-1), f("critic.2.bias").reshape(-1)
+    x = np.asarray(x, dtype=np.float64)
+    v = np.maximum(x @ W1.T + b1, 0) @ W2 + b2[0]
+    scale = abs(b2[0]) + (np.abs(b1) + np.abs(x) @ np.abs(W1).T) @ np.abs(W2)
+    return v, scale
 
 
 def categorical_log_prob(probs, action, dtype=np.float64):

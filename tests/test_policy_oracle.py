@@ -147,3 +147,86 @@ def test_gnn_restatement_against_pyg_golden_when_present():
         sd = {k: gold[f"c{ci}_{k}"] for k in keys}
         for x, q in zip(gold[f"c{ci}_x"], gold[f"c{ci}_q"]):
             np.testing.assert_allclose(po.gnn_forward(x.astype(np.float64), gold[f"c{ci}_edge_links"], sd), q, rtol=2e-5, atol=2e-6)
+
+
+def test_batched_philox_matches_the_scalar_one():
+    rng = np.random.default_rng(5)
+    ctr = rng.integers(0, 2 ** 32, size=(4, 300), dtype=np.uint64)
+    seed = (0xDEADBEEF << 32) | 0x12345678
+    got = po.philox4x32_batched(*ctr, seed)
+    for i in range(300):
+        assert tuple(int(w[i]) for w in got) == so.philox4x32(tuple(int(c[i]) for c in ctr), (seed & 0xFFFFFFFF, seed >> 32))
+    assert all(float(po.u01_batched(got[0])[i]) == po.u01(int(got[0][i])) for i in range(300))
+
+
+def _pool_with_parallel_edges(N, E):
+    """three graphs of one size; the last stores one edge twice and one reversed: both are separate GCN messages"""
+    graphs = [so.philox_sample_graph_once(7, g, 0, 0, N, E) for g in range(3)]
+    links = graphs[2].edge_links.copy()
+    links[-1], links[-2] = links[0], links[1][::-1]
+    return [graphs[0].edge_links, graphs[1].edge_links, links]
+
+
+def test_batched_gnn_oracle_matches_both_scalar_restatements():
+    """gnn_forward_batched (sparse aggregation, env chunks) == gnn_forward == gnn_forward_message_passing to 1e-12 on a
+    few hundred envs of a pool with parallel edges, both feature modes, MrX hidden and revealed, both models."""
+    rng = np.random.default_rng(12)
+    N, E, K, B = 20, 35, 5, 240
+    pool = _pool_with_parallel_edges(N, E)
+    assert len({tuple(r) for r in pool[2].tolist()}) < len(pool[2])  # the pool does hold a parallel edge
+    sds = [_random_gnn_sd(rng, K), _random_gnn_sd(rng, K)]
+    pos = np.stack([rng.choice(N, size=K, replace=False) for _ in range(B)])
+    pos[::7, 2] = pos[::7, 1]  # officers sharing a node
+    rev = np.where(rng.random(B) < 0.5, -1, 3)
+    gid = rng.integers(0, 3, size=B)
+    for mode in (po.FEATURES_ENV, po.FEATURES_REFERENCE):
+        q = po.gnn_forward_batched(mode, pos, rev, gid, pool, sds, N, chunk_floats=37 * N * K)  # several chunks per graph
+        for b in range(B):
+            x = po.graph_features(mode, pos[b], rev[b], N, K)
+            np.testing.assert_array_equal(po.graph_features_batched(mode, pos[b: b + 1], rev[b: b + 1], N, K)[0], x)
+            for m in range(2):
+                np.testing.assert_allclose(q[b, m], po.gnn_forward(x, pool[gid[b]], sds[m]), rtol=1e-12, atol=1e-12)
+                if b % 4 == 0:
+                    np.testing.assert_allclose(q[b, m], po.gnn_forward_message_passing(x, pool[gid[b]], sds[m]), rtol=1e-12,
+                                               atol=1e-12)
+    assert (rev < 0).any() and (rev >= 0).any() and (gid == 2).any()
+
+
+def test_batched_gnn_exploration_matches_gnn_select():
+    rng = np.random.default_rng(2)
+    B, A, N, seed, step, off = 300, 4, 30, (7 << 32) | 99, 17, 1000
+    mask = rng.random((B, A, N)) < 0.12
+    mask[::11, 1] = False  # agents without a move
+    explored, act = po.gnn_explore_batched(mask, 0.4, 0.7, seed, off + np.arange(B), step)
+    q = rng.normal(size=N)
+    for b in range(B):
+        for a in range(A):
+            want, ex, _ = po.gnn_select(q, np.nonzero(mask[b, a])[0], 0.4 if a == 0 else 0.7, seed, off + b, step, a)
+            assert ex == explored[b, a] and (act[b, a] == want if ex else act[b, a] == -1), (b, a)
+    assert explored.any() and (~explored).any()
+
+
+def test_batched_mappo_oracle_matches_mappo_probs():
+    """mappo_forward_batched == mappo_probs to 1e-12 on a few hundred rows that take all three branches; the error scale
+    is the documented sum of magnitudes"""
+    rng = np.random.default_rng(4)
+    R, D, H, N = 400, 6, 24, 33
+    sd = {"actor.0.weight": rng.normal(size=(H, D)) * 0.4, "actor.0.bias": rng.normal(size=H) * 0.2,
+          "actor.2.weight": rng.normal(size=(N, H)) * 0.2, "actor.2.bias": rng.normal(size=N)}
+    sd["actor.2.bias"][:3] += 60.0  # the mass on masks without nodes 0..2 underflows 1e-8: uniform over the mask
+    obs = rng.normal(size=(R, D))
+    mask = rng.random((R, N)) < 0.15
+    mask[::9] = False  # empty masks: uniform over all nodes
+    mask[1::9, :3] = True
+    out = po.mappo_forward_batched(obs, sd, mask, chunk=64)
+    for r in range(R):
+        np.testing.assert_allclose(out["probs"][r], po.mappo_probs(obs[r], sd, mask[r].astype(np.float64)), rtol=1e-12, atol=1e-15)
+        h = np.abs(sd["actor.0.bias"]) + np.abs(sd["actor.0.weight"]) @ np.abs(obs[r])
+        assert abs(out["scale"][r] - (np.abs(sd["actor.2.bias"]) + np.abs(sd["actor.2.weight"]) @ h).max()) <= 1e-12 * out["scale"][r]
+    assert set(out["mode"].tolist()) == {po.MAPPO_SOFTMAX, po.MAPPO_UNIFORM_MASK, po.MAPPO_UNIFORM_ALL}
+    gsd = {"critic.0.weight": rng.normal(size=(H, 3 * D)), "critic.0.bias": rng.normal(size=H), "critic.2.weight": rng.normal(size=(1, H)),
+           "critic.2.bias": rng.normal(size=1)}
+    x = rng.normal(size=(50, 3 * D))
+    v, scale = po.critic_value_batched(x, gsd)
+    np.testing.assert_allclose(v, [po.critic_value(r, gsd) for r in x], rtol=1e-12, atol=1e-12)
+    assert (scale >= np.abs(v)).all()
