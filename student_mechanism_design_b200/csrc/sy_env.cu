@@ -1792,7 +1792,11 @@ __device__ __forceinline__ void belief_env_generic_t(const Params& p, float* sb,
       else ce_record(ce, S, vx);
       _Pragma("unroll 1") for (int j = lane; j < N; j += 32) bel[j] = (j == x) ? 1.0f : 0.0f;
     } else if (p.belief_hint && op == BEL_PROPAGATE && tot != 0.0f) {
-      // observation hint (belief_module.py:102-106) on the row this warp just wrote (every lane re-reads its own stores)
+      // observation hint (belief_module.py:102-106) on the row this warp just wrote.  Lane l re-reads the nodes
+      // j = l (mod 32); the shared-CSR path wrote bel[perm[jj]] in degree order, so those values came from other lanes,
+      // which may still be in the last trip of their gather loop when N % 32 != 0: wait for every lane's stores first
+      // (here and not before the branch, so that the hint-free kernels keep their instruction stream)
+      __syncwarp();
       const uint8_t* hint = p.belief_hint + (size_t)b * N;
       float hs = 0.0f;
       _Pragma("unroll 1") for (int j = lane; j < N; j += 32) hs += bel[j] * (hint[j] ? 1.0f : 0.1f);
