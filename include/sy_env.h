@@ -336,7 +336,8 @@ int sy_stats(SyEnv* env, int64_t* stats, sy_stream_t stream);
 
 /* Mechanism groups: one handle evaluates up to SY_MAX_GROUPS mechanisms side by side.  Every env belongs to one group,
  * and a group replaces, for its envs, the config's reward weights (fp32 reward mode uses (float)w), police start budget
- * (agent_money) and reveal schedule (reveal_interval, reveal_skip_prob).  Everything else stays one value per handle.
+ * (agent_money), reveal schedule (reveal_interval, reveal_skip_prob) and, through sy_set_group_tolls, the toll.  The
+ * number of police and max_timestep stay one value per handle.
  * Group membership enters no random stream, so a group equal to the config reproduces a handle without groups bit for
  * bit.  Every step path runs with groups (its GROUPS instantiation) except the split step of SY_OPT_NF_FILL, which acts
  * as off while groups are set (results are the same).  The statistics are also summed per group (sy_group_stats).
@@ -356,8 +357,18 @@ typedef struct SyGroup {
  * library-owned memory; a rejected call keeps the previous groups.  The new groups take effect at the next sy_reset of
  * every env (NULL reset_mask, or one with every byte set): until then the step and rollout entry points fail with
  * SY_ERR_STATE (so a state saved under groups cannot be resumed mid-episode: the reset starts new episodes).  Fails with
- * SY_ERR_STATE while observations are pending.  Clears the per-group statistics. */
+ * SY_ERR_STATE while observations are pending.  Clears the per-group statistics.  Every group gets the config's toll. */
 int sy_set_groups(SyEnv* env, int32_t num_groups, const SyGroup* groups, const int32_t* group_id, sy_stream_t stream);
+/* Per-group tolls: an env pays its group's toll instead of SyConfig.toll -- a move is legal iff w + toll <= budget (MrX and
+ * police; action_mask, the random sampler and the mobility term of the rewards follow the same rule), and a police move
+ * costs w + toll.  tolls: HOST int32 [num_groups], each in [0, SY_MAX_TOLL] (with edge weights <= 255, w + toll and the
+ * per-step sums of the police charges cannot overflow an int32); num_groups must be the number set by sy_set_groups.
+ * A rejected call keeps the previous tolls.  Like sy_set_groups: fails with SY_ERR_STATE while observations are pending
+ * (or when no groups are set), and the new tolls take effect at the next sy_reset of every env, which the step and
+ * rollout entry points require until then.  A CUDA graph captured before the call must be captured again.  Synchronises
+ * `stream`. */
+#define SY_MAX_TOLL 1048576
+int sy_set_group_tolls(SyEnv* env, int32_t num_groups, const int32_t* tolls, sy_stream_t stream);
 /* Add the per-group statistics accumulated since the last call to `stats` (DEVICE int64 [num_groups, SY_NUM_STATS],
  * caller-owned, cumulative) and clear the accumulators; num_groups must be the number set.  They are collected by the
  * same steps as sy_stats, with the same integer sums, so the sum over groups equals the handle-wide vector. */

@@ -14,6 +14,7 @@ SY_NUM_REWARD_WEIGHTS = 11
 SY_MAX_AGENTS = 16
 SY_NUM_STATS = 16
 SY_MAX_GROUPS = 1024
+SY_MAX_TOLL = 1048576
 SY_REWARD_FP64, SY_REWARD_FP32 = 0, 1
 STAT_NAMES = [
     "env_steps", "episodes", "mrx_wins", "police_wins", "truncations", "out_of_money",
@@ -110,6 +111,7 @@ SIGNATURES = {
     "sy_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "sy_set_groups": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(SyGroup), C.c_void_p, C.c_void_p]),
     "sy_group_stats": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
+    "sy_set_group_tolls": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(C.c_int32), C.c_void_p]),
     "sy_allreduce_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sy_rollout_random_dev": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(SyState), C.POINTER(SyObs),
                                         C.POINTER(SyOut), C.c_void_p]),

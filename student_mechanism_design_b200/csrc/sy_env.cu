@@ -167,8 +167,8 @@ struct Params {
   const int32_t* init_pos;
   const int32_t* init_gid;
   int restart;
-  // mechanism groups (sy_set_groups; read only by the GROUPS instantiations): per-env reward weights, police budget and
-  // reveal schedule.  Appended so that the offsets of every field above stay where the default kernels expect them.
+  // mechanism groups (sy_set_groups; read only by the GROUPS instantiations): per-env reward weights, police budget,
+  // reveal schedule and toll.  Appended so that the offsets of every field above stay where the default kernels expect them.
   const struct GroupRow* grp;        // [grp_n] library-owned table
   const int32_t* grp_id;             // [B] group of each env
   int grp_n, grp_rep;                // groups; replicas of the per-group statistics lines
@@ -181,8 +181,36 @@ struct GroupRow {
   double w64[SY_NUM_REWARD_WEIGHTS];
   float w32[SY_NUM_REWARD_WEIGHTS];
   int agent_money, reveal;
+  int toll;  // sy_set_group_tolls (sy_set_groups: the config's)
   unsigned long long reveal_skip_thresh;
 };
+
+// the toll an env pays per move (yard.py:223-229 and action_mask.py:65-76 with the toll extension: a move is legal iff
+// weight + toll <= budget, and costs weight + toll): the handle's, or (GROUPS) that of the env's mechanism group `gr`
+template <int GROUPS>
+__device__ __forceinline__ int env_toll(const Params& p, const GroupRow* gr) {
+  if constexpr (GROUPS) return __ldg(&gr->toll);
+  else return p.toll;
+}
+// ... of env b, when its group row is not at hand
+template <int GROUPS>
+__device__ __forceinline__ int env_toll_of(const Params& p, int b) {
+  if constexpr (GROUPS) return env_toll<1>(p, p.grp + __ldg(p.grp_id + b));
+  else return p.toll;
+}
+// The observation writers stage one budget per (env, agent) and test `weight + wr_toll <= staged budget`.  Without
+// groups that is the budget and the handle's toll.  With groups a tile mixes tolls, so they stage the headroom
+// money - toll_b (at least -SY_MAX_TOLL: no overflow) and add nothing.
+template <int GROUPS>
+__device__ __forceinline__ int wr_toll(const Params& p) {
+  if constexpr (GROUPS) return 0;
+  else return p.toll;
+}
+template <int GROUPS>
+__device__ __forceinline__ int wr_budget(const Params& p, int money, int b) {
+  if constexpr (GROUPS) return money - env_toll_of<1>(p, b);
+  else return money;
+}
 
 
 #ifdef SY_FUSED_CLOCKS  // profiling builds: per-role time inside the fused kernel, summed over CTAs (sy_debug_fused_clocks)
@@ -369,9 +397,10 @@ __device__ __forceinline__ int edge_weight_sg(const SharedGraph& sg, int u, int 
   return w;
 }
 
-template <int MAXA, typename PosT>
+// GROUPS: the toll of the env's mechanism group `gr`
+template <int MAXA, int GROUPS = 0, typename PosT>
 __device__ __forceinline__ int move_phase(const Params& p, PosT* pos, int* money, const int* act, int g, int t, int& spent, int& moves,
-                                          const SharedGraph* sg = nullptr) {
+                                          const SharedGraph* sg = nullptr, const GroupRow* gr = nullptr) {
   const Tables& tb = p.tb;
   const int N = p.N, P = p.P;
   int rp[MAXA], rm[MAXA], ra[MAXA], wpre[MAXA];
@@ -387,7 +416,7 @@ __device__ __forceinline__ int move_phase(const Params& p, PosT* pos, int* money
     wpre[i] = (i <= P && ra[i] >= 0) ? (sg ? edge_weight_sg(*sg, rp[i], ra[i]) : edge_weight(tb, N, g, rp[i], ra[i])) : 0;
   {  // MrX: legal target or stay; may not step onto a police node (yard.py:161-188)
     int tgt = rp[0];
-    if (ra[0] >= 0 && wpre[0] > 0 && wpre[0] + p.toll <= rm[0]) tgt = ra[0];
+    if (ra[0] >= 0 && wpre[0] > 0 && wpre[0] + env_toll<GROUPS>(p, gr) <= rm[0]) tgt = ra[0];
     bool occupied = false;
 #pragma unroll
     for (int i = 1; i < MAXA; ++i) occupied |= (rp[i] == tgt);
@@ -401,14 +430,14 @@ __device__ __forceinline__ int move_phase(const Params& p, PosT* pos, int* money
       const bool skipped = (ai == -1 || m == 0);  // None / DEFAULT_ACTION / broke: skipped (yard.py:210-215)
       no_money &= skipped;
       // a possible move: adjacent and affordable; otherwise the police stays (yard.py:223-229)
-      const bool can = !skipped && ai >= 0 && ai != rp[i] && w != 0 && w + p.toll <= m;
+      const bool can = !skipped && ai >= 0 && ai != rp[i] && w != 0 && w + env_toll<GROUPS>(p, gr) <= m;
       bool occupied = false;  // may step onto MrX (capture) but not onto police (yard.py:231)
 #pragma unroll
       for (int j = 1; j < MAXA; ++j) occupied |= (rp[j] == ai);
       if (can && !occupied) {
         rp[i] = ai;
-        rm[i] = m - (w + p.toll);
-        spent += w + p.toll;
+        rm[i] = m - (w + env_toll<GROUPS>(p, gr));
+        spent += w + env_toll<GROUPS>(p, gr);
         moves += 1;
       }
     }
@@ -602,7 +631,7 @@ struct LogicSmem {
 // LAG_BAR, LAGT threads: the observation warps arrive, the dynamics warps wait -- long after the arrival in practice).
 constexpr int LAG_BAR = 4;
 constexpr int LAG_CSR_BAR = 6;  // lagged kernel: the writers' staged graph is complete (writers arrive, dynamics warps wait)
-// GROUPS: mechanism groups are set -- every env reads its group's row (reward weights, police budget, reveal schedule)
+// GROUPS: mechanism groups are set -- every env reads its group's row (reward weights, police budget, reveal schedule, toll)
 // once per step through the read-only path, and the statistics are also summed per group
 template <int MODE, int MAXA, int BAR, int LAGT = 0, int CSRT = 0, int GROUPS = 0>
 __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm, int b0, int tid, const SharedGraph* sgp = nullptr,
@@ -691,7 +720,7 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
   int spent = 0, moves = 0;
   [[maybe_unused]] const long long tp1 = PHASE_NOW();
   if (warp == 0) {
-    if (active) sm.status[lane] = move_phase<MAXA>(p, pos, money, act, g, t, spent, moves, sg);
+    if (active) sm.status[lane] = move_phase<MAXA, GROUPS>(p, pos, money, act, g, t, spent, moves, sg, gr);
     PHASE_SPAN(8, tp1);
   } else if (warp == 1 && p.auto_reset && active) {
     const unsigned env_id = (unsigned)(p.env_offset + (unsigned long long)b);
@@ -771,8 +800,8 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
           for (int j = 0; j < MAXA; ++j) in.dj[j] = (j <= P && j != a) ? (int)sm.dmat[lane * DS + a * MAXA + j] : 0;
           // QUIRK reward_calculator.py:190: the police mobility term uses the budget of agent index a-1 (not a)
           const int mny = money[a == 0 ? 0 : a - 1];
-          const int c = min(mny - p.toll, p.tb.wcap);
-          if (c > 0) in.mob = sm.cnt_staged ? (int)sm.cnt[u * (p.tb.wcap + 1) + c] : move_count(p.tb, N, g, u, mny, p.toll);
+          const int c = min(mny - env_toll<GROUPS>(p, gr), p.tb.wcap);
+          if (c > 0) in.mob = sm.cnt_staged ? (int)sm.cnt[u * (p.tb.wcap + 1) + c] : move_count(p.tb, N, g, u, mny, env_toll<GROUPS>(p, gr));
         }
         r64 = agent_reward<MODE, MAXA, GROUPS>(p, sm.rt, in, t, status, a, visits_here, gr);
       }
@@ -946,10 +975,10 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
       const bool use_sg = sg != nullptr && !p.resample_graph;
       int nvalid;
       if (use_sg && sm.cnt_staged) {
-        const int c = min(m - p.toll, p.tb.wcap);
+        const int c = min(m - env_toll_of<GROUPS>(p, b0 + e), p.tb.wcap);
         nvalid = c > 0 ? (int)sm.cnt[u * (p.tb.wcap + 1) + c] : 0;
       } else {
-        nvalid = move_count(p.tb, N, gg, u, m, p.toll);
+        nvalid = move_count(p.tb, N, gg, u, m, env_toll_of<GROUPS>(p, b0 + e));
       }
       long long act = -1;
       if (nvalid > 0) {
@@ -958,7 +987,7 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
         int pick = (int)__umulhi(r.x, (unsigned)nvalid);
         if (use_sg) {
           for (int k = sg->rp[u];; ++k) {  // the pick-th affordable neighbour exists
-            if ((int)sg->wgt[k] + p.toll <= m) {
+            if ((int)sg->wgt[k] + env_toll_of<GROUPS>(p, b0 + e) <= m) {
               if (pick == 0) {
                 act = sg->col[k];
                 break;
@@ -969,7 +998,7 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
         } else {
           const uint8_t* wg = p.tb.wgt + (size_t)gg * p.tb.nnz_stride;
           for (int k = __ldg(p.tb.row_ptr + (size_t)gg * (N + 1) + u);; ++k) {  // the pick-th affordable neighbour exists
-            if (__ldg(wg + k) + p.toll <= m) {
+            if (__ldg(wg + k) + env_toll_of<GROUPS>(p, b0 + e) <= m) {
               if (pick == 0) {
                 act = __ldg(p.tb.col + (size_t)gg * p.tb.nnz_stride + k);
                 break;
@@ -1179,8 +1208,9 @@ __device__ __forceinline__ void warp_write_node_features(float* nf, int n, const
 // memory first (one round trip for the whole tile): agents' nodes and budgets, reveal flags and -- when the tile sits
 // on one graph and its CSR fits -- the graph's row pointers / neighbours / weights.  Each env's action_mask rows are
 // assembled in a per-warp shared-memory image and copied out, node_features are zero-filled and the (at most A) chunks
-// with a one rewritten whole: no byte-sized stores anywhere (they cost 60 % extra time when tried).
-template <int WRW, bool PREFILLED = false, int LAGT = 0, int CSRT = 0>
+// with a one rewritten whole: no byte-sized stores anywhere (they cost 60 % extra time when tried).  GROUPS: budgets are
+// staged as headroom against each env's group toll (wr_budget).
+template <int WRW, bool PREFILLED = false, int LAGT = 0, int CSRT = 0, int GROUPS = 0>
 __device__ __forceinline__ void writer_role(const Params& p, unsigned char* dyn, int tile0, int nEnv, int w, int lane,
                                             int* lag_staged = nullptr) {
   const Tables& tb = p.tb;
@@ -1200,7 +1230,7 @@ __device__ __forceinline__ void writer_role(const Params& p, unsigned char* dyn,
   const bool staged = p.wr_stage_csr && __all_sync(FULL, gl == g0 || gl < 0);
   for (int i = tw; i < nEnv * A; i += WRW * 32) {
     s_pos[i] = p.st.pos[(size_t)tile0 * A + i];
-    s_money[i] = p.st.money[(size_t)tile0 * A + i];
+    s_money[i] = wr_budget<GROUPS>(p, p.st.money[(size_t)tile0 * A + i], tile0 + ((i * p.inv_A) >> 16));
   }
   if (tw < nEnv) {
     s_rev[tw] = p.ob.mrx_revealed[tile0 + tw];
@@ -1265,14 +1295,14 @@ __device__ __forceinline__ void writer_role(const Params& p, unsigned char* dyn,
         if (staged) {
           const int r0 = s_rp[u], r1 = s_rp[u + 1];
           for (int k = r0 + sub; k < r1; k += lpa)
-            if ((int)s_wgt[k] + p.toll <= m) row[s_col[k]] = 1;
+            if ((int)s_wgt[k] + wr_toll<GROUPS>(p) <= m) row[s_col[k]] = 1;
         } else {
           const int32_t* rp = tb.row_ptr + (size_t)g * (N + 1) + u;
           const int r0 = __ldg(rp), r1 = __ldg(rp + 1);
           const uint16_t* cl = tb.col + (size_t)g * tb.nnz_stride;
           const uint8_t* wg = tb.wgt + (size_t)g * tb.nnz_stride;
           for (int k = r0 + sub; k < r1; k += lpa)
-            if ((int)__ldg(wg + k) + p.toll <= m) row[__ldg(cl + k)] = 1;
+            if ((int)__ldg(wg + k) + wr_toll<GROUPS>(p) <= m) row[__ldg(cl + k)] = 1;
         }
       }
       __syncwarp();
@@ -1329,8 +1359,9 @@ struct BulkCtx {
   const uint8_t* wgt;
 };
 
-// ones of the action_mask stream that fall into bytes [lo, lo + len): lane = (env, agent) pair
-template <bool STAGED>
+// ones of the action_mask stream that fall into bytes [lo, lo + len): lane = (env, agent) pair (GROUPS: the staged
+// budgets are headroom, see wr_budget)
+template <bool STAGED, int GROUPS = 0>
 __device__ __forceinline__ void bulk_mask_ones(const Params& p, const BulkCtx& c, uint8_t* img, int lo, int len, int lane, uint8_t v) {
   const int N = p.N, A = p.A, S = A * N;
   const int e_lo = lo / S, e_hi = (lo + len - 1) / S;
@@ -1343,7 +1374,7 @@ __device__ __forceinline__ void bulk_mask_ones(const Params& p, const BulkCtx& c
       const int r0 = c.rp[u], r1 = c.rp[u + 1];
       for (int k = r0; k < r1; ++k) {
         const int off = base + (int)c.col[k];
-        if ((int)c.wgt[k] + p.toll <= m && (unsigned)off < (unsigned)len) img[off] = v;
+        if ((int)c.wgt[k] + wr_toll<GROUPS>(p) <= m && (unsigned)off < (unsigned)len) img[off] = v;
       }
     } else {
       const int g = c.s_gid[e];
@@ -1353,7 +1384,7 @@ __device__ __forceinline__ void bulk_mask_ones(const Params& p, const BulkCtx& c
       const uint8_t* wg = p.tb.wgt + (size_t)g * p.tb.nnz_stride;
       for (int k = r0; k < r1; ++k) {
         const int off = base + (int)__ldg(cl + k);
-        if ((int)__ldg(wg + k) + p.toll <= m && (unsigned)off < (unsigned)len) img[off] = v;
+        if ((int)__ldg(wg + k) + wr_toll<GROUPS>(p) <= m && (unsigned)off < (unsigned)len) img[off] = v;
       }
     }
   }
@@ -1454,7 +1485,7 @@ __device__ __forceinline__ void nf32_ones_piece(const Params& p, const BulkCtx& 
 // writer warp `iw` of `niw`: items iw, iw + niw, ... of [uint8 node_features chunks | action_mask chunks]; with float32
 // node_features every mask chunk also carries the matching piece of that stream.  D = chunks between a piece's fill and
 // its ones.  prefilled: the caller already issued (from this warp's lane 0) the fill of all of this warp's pieces.
-template <int D>
+template <int D, int GROUPS = 0>
 __device__ __forceinline__ void writer_stream_warp(const Params& p, const BulkCtx& c, const ImageStreams& st, bool staged, uint8_t* my_img,
                                                    const uint8_t* zero_page, uint8_t* gnf32, int iw, int niw, int lane, bool prefilled) {
   const int Cm = p.wr_c_mask, Cf = p.wr_c_nf;
@@ -1465,8 +1496,8 @@ __device__ __forceinline__ void writer_stream_warp(const Params& p, const BulkCt
       bulk_nf_ones<1>(p, c, img, lo, min(Cf, st.Tf - lo), lane, v != 0);
     } else {
       const int lo = (item - st.ncf) * Cm, len = min(Cm, st.Tm - lo);
-      if (staged) bulk_mask_ones<true>(p, c, img, lo, len, lane, v);
-      else bulk_mask_ones<false>(p, c, img, lo, len, lane, v);
+      if (staged) bulk_mask_ones<true, GROUPS>(p, c, img, lo, len, lane, v);
+      else bulk_mask_ones<false, GROUPS>(p, c, img, lo, len, lane, v);
     }
   };
   auto piece_ones = [&](int item) {
@@ -1532,8 +1563,8 @@ constexpr int BULK_WARPS = SY_BULK_WARPS;  // writer warps that stream on the bu
 constexpr int BULK_DEPTH = SY_BULK_DEPTH;  // chunks between a float32 piece's fill and its ones
 
 // stage the tile's post-step state (and, when the tile sits on one graph, its CSR) into shared memory: what every
-// writer needs to place the ones.  Returns whether the CSR was staged.
-template <int NTHREADS>
+// writer needs to place the ones (GROUPS: budgets as headroom, see wr_budget).  Returns whether the CSR was staged.
+template <int NTHREADS, int GROUPS = 0>
 __device__ __forceinline__ bool stage_tile_inputs(const Params& p, unsigned char* dyn, int tile0, int nEnv, int tw, int lane,
                                                   int* s_pos, int* s_money, int* s_rev, int* s_gid) {
   const Tables& tb = p.tb;
@@ -1546,7 +1577,7 @@ __device__ __forceinline__ bool stage_tile_inputs(const Params& p, unsigned char
   const bool staged = p.wr_stage_csr && __all_sync(FULL, gl == g0 || gl < 0);
   for (int i = tw; i < nEnv * A; i += NTHREADS) {
     s_pos[i] = p.st.pos[(size_t)tile0 * A + i];
-    s_money[i] = p.st.money[(size_t)tile0 * A + i];
+    s_money[i] = wr_budget<GROUPS>(p, p.st.money[(size_t)tile0 * A + i], tile0 + ((i * p.inv_A) >> 16));
   }
   if (tw < nEnv) {
     s_rev[tw] = p.ob.mrx_revealed[tile0 + tw];
@@ -1583,7 +1614,7 @@ __device__ __forceinline__ bool stage_tile_inputs(const Params& p, unsigned char
   return staged;
 }
 
-template <int WRW>
+template <int WRW, int GROUPS = 0>
 __device__ __forceinline__ void writer_role_bulk(const Params& p, unsigned char* dyn, int tile0, int nEnv, int w, int lane) {
   constexpr int NW = WRW < BULK_WARPS ? WRW : BULK_WARPS;
   const int N = p.N, A = p.A;
@@ -1595,7 +1626,7 @@ __device__ __forceinline__ void writer_role_bulk(const Params& p, unsigned char*
   uint8_t* imgs = zero_page + p.wr_img_bytes;                     // [BULK_WARPS][2][wr_img_bytes]
   for (int i = (w * 32 + lane) * 16; i < (1 + 2 * NW) * p.wr_img_bytes; i += WRW * 32 * 16) *reinterpret_cast<uint4*>(zero_page + i) = make_uint4(0, 0, 0, 0);
   fence_proxy_async_smem();
-  const bool staged = stage_tile_inputs<WRW * 32>(p, dyn, tile0, nEnv, w * 32 + lane, lane, s_pos, s_money, s_rev, s_gid);
+  const bool staged = stage_tile_inputs<WRW * 32, GROUPS>(p, dyn, tile0, nEnv, w * 32 + lane, lane, s_pos, s_money, s_rev, s_gid);
   named_barrier(2, WRW * 32);
   if (p.bel_share_csr) asm volatile("bar.arrive 3, %0;\n" ::"r"(THREADS) : "memory");
   if (w >= NW) return;
@@ -1604,7 +1635,7 @@ __device__ __forceinline__ void writer_role_bulk(const Params& p, unsigned char*
   const BulkCtx c{s_pos, s_money, s_rev, s_gid, s_rp, s_col, reinterpret_cast<uint8_t*>(s_col + p.tb.nnz_stride)};
   const ImageStreams st = image_streams(p, tile0, nEnv);
   uint8_t* gnf32 = p.ob.node_features_u8 ? nullptr : reinterpret_cast<uint8_t*>(p.ob.node_features) + (size_t)tile0 * N * A * 4;
-  writer_stream_warp<BULK_DEPTH>(p, c, st, staged, imgs + (size_t)w * 2 * p.wr_img_bytes, zero_page, gnf32, w, NW, lane, false);
+  writer_stream_warp<BULK_DEPTH, GROUPS>(p, c, st, staged, imgs + (size_t)w * 2 * p.wr_img_bytes, zero_page, gnf32, w, NW, lane, false);
 }
 
 // generic belief path: one warp per env, lane = node; any N, any mix of graphs.  sb: N floats of this warp.
@@ -2002,8 +2033,8 @@ __device__ __forceinline__ void belief_role(const Params& p, unsigned char* dyn,
 // <BW, 0> / <0, WRW>: one role per launch (the split step runs them as two concurrent kernels; the role hand-over
 // barrier of the large-N belief path counts THREADS, so that path keeps both roles in one launch)
 enum { WV_LSU = 0, WV_BULK = 1, WV_ONES = 2 };
-// GROUPS: the belief scores at reveal steps are also summed per mechanism group (only launched while groups are set and
-// the step collects scored statistics)
+// GROUPS (launched while mechanism groups are set): the writers test each env's moves against its group's toll, and the
+// belief scores at reveal steps are also summed per group
 template <int BW, int WRW, int WV = WV_LSU, int GROUPS = 0>
 __global__ void __launch_bounds__((BW + WRW) * 32) sy_observe_kernel(const Params p) {
   static_assert((BW + WRW) * 32 == THREADS || BW == 0 || WRW == 0, "the role hand-over barrier counts THREADS");
@@ -2033,9 +2064,9 @@ __global__ void __launch_bounds__((BW + WRW) * 32) sy_observe_kernel(const Param
   } else if (!(p.dbg_skip & 1)) {
     if constexpr (WRW > 0) {
       if constexpr (WV == WV_BULK) {
-        if constexpr (WRW >= 2) writer_role_bulk<WRW>(p, dyn, tile0, nEnv, warp - nbw, lane);
+        if constexpr (WRW >= 2) writer_role_bulk<WRW, GROUPS>(p, dyn, tile0, nEnv, warp - nbw, lane);
       } else {
-        writer_role<WRW, WV == WV_ONES>(p, dyn, tile0, nEnv, warp - nbw, lane);
+        writer_role<WRW, WV == WV_ONES, 0, 0, GROUPS>(p, dyn, tile0, nEnv, warp - nbw, lane);
       }
       if (warp == nbw) {
         FCLK_ADD(1, FCLK_NOW() - t0);
@@ -2074,7 +2105,7 @@ __global__ void __launch_bounds__((BW + WRW + LOGIC_WARPS) * 32, 2) sy_step_lagg
     if constexpr (BW > 0) belief_role<BW, NT, GROUPS>(p, dyn, tile0, nEnv, warp, lane);
     if (warp == 0) FCLK_ADD(3, FCLK_NOW() - t0);
   } else if (warp < BW + WRW) {
-    writer_role<WRW, false, NT, CSRT>(p, dyn, tile0, nEnv, warp - BW, lane, &staged_flag);
+    writer_role<WRW, false, NT, CSRT, GROUPS>(p, dyn, tile0, nEnv, warp - BW, lane, &staged_flag);
     if (warp == BW) FCLK_ADD(1, FCLK_NOW() - t0);
   } else {
     const int* s_rp = reinterpret_cast<const int*>(dyn + p.wr_off_csr);
@@ -2114,7 +2145,7 @@ __global__ void __launch_bounds__((BW + WRW + LOGIC_WARPS) * 32, 2) sy_rollout_l
       }
     } else if (warp < BW + WRW) {
       if (do_obs) {
-        writer_role<WRW, false, NT, CSRT>(p, dyn, tile0, nEnv, warp - BW, lane, &staged_flag);
+        writer_role<WRW, false, NT, CSRT, GROUPS>(p, dyn, tile0, nEnv, warp - BW, lane, &staged_flag);
       } else {
         if (threadIdx.x == BW * 32) staged_flag = 0;  // nothing staged: the dynamics read the pool tables
         asm volatile("bar.arrive %0, %1;\n" ::"n"(LAG_CSR_BAR), "n"(CSRT) : "memory");
@@ -2200,14 +2231,15 @@ __device__ __forceinline__ PairView pair_of(const Params& p, const int* s_pos, c
 }
 // affordable neighbours of the pair's node into (v = 1) or out of (v = 0) the chunk image (action_mask.py:65-76).
 // s_nbr4[u] = the first four neighbours as {col | wgt << 16}, the degree in the top byte of .x; the rare nodes with
-// more neighbours finish over the staged CSR.
+// more neighbours finish over the staged CSR.  GROUPS: the pair's budget is headroom (wr_budget).
+template <int GROUPS = 0>
 __device__ __forceinline__ void fast_mask_ones(const Params& p, const PairView& pv, const uint4* s_nbr4, const int* s_rp, const uint16_t* s_col,
                                                const uint8_t* s_wgt, uint8_t* img, int epc, int cm, uint8_t v) {
   if (!pv.valid) return;
   const uint4 nb = s_nbr4[pv.u];
   const int deg = (int)(nb.x >> 24);
   uint8_t* row = img + ((pv.e - cm * epc) * p.A + pv.a) * p.N;
-  const int lim = pv.m - p.toll;  // wgt + toll <= m
+  const int lim = pv.m - wr_toll<GROUPS>(p);  // wgt + toll <= m
   if (deg > 0 && (int)((nb.x >> 16) & 0xffu) <= lim) row[nb.x & 0xffffu] = v;
   if (deg > 1 && (int)(nb.y >> 16) <= lim) row[nb.y & 0xffffu] = v;
   if (deg > 2 && (int)(nb.z >> 16) <= lim) row[nb.z & 0xffffu] = v;
@@ -2227,7 +2259,7 @@ __device__ __forceinline__ void fast_nf32_ones(const Params& p, const PairView& 
     __stcs(reinterpret_cast<float*>(gnf + (size_t)pv.e * p.N * A * 4) + pv.u * A + pv.a, 1.0f);
 }
 
-template <int BW>
+template <int BW, int GROUPS = 0>
 __device__ __forceinline__ void fused_writer_role(const Params& p, unsigned char* dyn, const unsigned* tiles_done, int w, int lane) {
   constexpr int D = BULK_DEPTH;
   const Tables& tb = p.tb;
@@ -2283,8 +2315,8 @@ __device__ __forceinline__ void fused_writer_role(const Params& p, unsigned char
       bulk_nf_ones<1>(p, c, img, lo, min(p.wr_c_nf, st.Tf - lo), lane, v != 0);
     } else {
       const int lo = (item - st.ncf) * Cm, len = min(Cm, st.Tm - lo);
-      if (staged) bulk_mask_ones<true>(p, c, img, lo, len, lane, v);
-      else bulk_mask_ones<false>(p, c, img, lo, len, lane, v);
+      if (staged) bulk_mask_ones<true, GROUPS>(p, c, img, lo, len, lane, v);
+      else bulk_mask_ones<false, GROUPS>(p, c, img, lo, len, lane, v);
     }
   };
   auto owed_ones = [&](int k, int item, int fast) {  // float32 ones of an older chunk, after its fill has completed
@@ -2322,7 +2354,7 @@ __device__ __forceinline__ void fused_writer_role(const Params& p, unsigned char
       const bool one_graph = p.wr_stage_csr && __all_sync(FULL, gl == g0 || gl < 0);
       for (int i = tw; i < nEnv * A; i += FUSED_WR * 32) {
         sb[i] = __ldcg(p.st.pos + (size_t)tile0 * A + i);
-        sb[TILE * A + i] = __ldcg(p.st.money + (size_t)tile0 * A + i);
+        sb[TILE * A + i] = wr_budget<GROUPS>(p, __ldcg(p.st.money + (size_t)tile0 * A + i), tile0 + ((i * p.inv_A) >> 16));
       }
       if (tw < nEnv) {
         sb[2 * TILE * A + tw] = __ldcg(p.ob.mrx_revealed + tile0 + tw);
@@ -2382,7 +2414,7 @@ __device__ __forceinline__ void fused_writer_role(const Params& p, unsigned char
         if (pending == D && ring_fast[0]) {  // (after a tile-boundary flush the ring is short: clear the whole image)
           int* ob = sbuf(ring_k[0]);
           const PairView pv = pair_of(p, ob, ob + TILE * A, ring_item[0], p.wr_epc, envs_of(ring_k[0]), lane);
-          fast_mask_ones(p, pv, s_nbr4, s_rp, s_col, s_wgt, img, p.wr_epc, ring_item[0], 0);
+          fast_mask_ones<GROUPS>(p, pv, s_nbr4, s_rp, s_col, s_wgt, img, p.wr_epc, ring_item[0], 0);
         } else {
           for (int i = lane * 16; i < p.wr_img_bytes; i += 32 * 16) *reinterpret_cast<uint4*>(img + i) = make_uint4(0, 0, 0, 0);
         }
@@ -2394,7 +2426,7 @@ __device__ __forceinline__ void fused_writer_role(const Params& p, unsigned char
       const int len = is_nf8 ? min(p.wr_c_nf, st.Tf - lo) : min(Cm, st.Tm - lo);
       if (fast) {
         const PairView pv = pair_of(p, sb, sb + TILE * A, item, p.wr_epc, nEnv, lane);
-        fast_mask_ones(p, pv, s_nbr4, s_rp, s_col, s_wgt, img, p.wr_epc, item, 1);
+        fast_mask_ones<GROUPS>(p, pv, s_nbr4, s_rp, s_col, s_wgt, img, p.wr_epc, item, 1);
       } else {
         generic_img(k, item, st, img, 1);
       }
@@ -2459,7 +2491,7 @@ __global__ void __launch_bounds__((BW + FUSED_WR + LOGIC_WARPS) * 32, 2) sy_step
     }
   } else if (warp < BW + FUSED_WR) {
     const long long t0 = FCLK_NOW();
-    fused_writer_role<BW>(p, dyn, &tiles_done, warp - BW, lane);
+    fused_writer_role<BW, GROUPS>(p, dyn, &tiles_done, warp - BW, lane);
     if (warp == BW) FCLK_ADD(1, FCLK_NOW() - t0);
   } else {
     const int tid = threadIdx.x - (BW + FUSED_WR) * 32;
@@ -2525,7 +2557,8 @@ __global__ void sy_count_unset_kernel(const uint8_t* mask, int B, int* unset) {
 // ---------------------------------------------------------------------------------------------
 // random valid policy: thread per (env, agent)
 // ---------------------------------------------------------------------------------------------
-template <typename ActT>
+// GROUPS: each env's moves are tested against its mechanism group's toll
+template <typename ActT, int GROUPS = 0>
 __global__ void __launch_bounds__(256) sy_sample_actions_kernel(const Params p, unsigned step_counter, ActT* actions,
                                                                 const unsigned* __restrict__ step_base) {
   if (step_base) step_counter += *step_base;  // device-resident counter: a captured CUDA graph keeps advancing
@@ -2535,7 +2568,8 @@ __global__ void __launch_bounds__(256) sy_sample_actions_kernel(const Params p, 
   const Tables& tb = p.tb;
   const int N = p.N;
   const int g = p.st.graph_id[b], u = p.st.pos[i], m = p.st.money[i];
-  const int nvalid = move_count(tb, N, g, u, m, p.toll);  // one table lookup instead of a pass over the row
+  const int toll = env_toll_of<GROUPS>(p, (int)b);
+  const int nvalid = move_count(tb, N, g, u, m, toll);  // one table lookup instead of a pass over the row
   long long act = -1;
   if (nvalid > 0) {
     const unsigned env_id = (unsigned)(p.env_offset + (unsigned long long)b);
@@ -2543,7 +2577,7 @@ __global__ void __launch_bounds__(256) sy_sample_actions_kernel(const Params p, 
     int pick = (int)__umulhi(r.x, (unsigned)nvalid);
     const uint8_t* wg = tb.wgt + (size_t)g * tb.nnz_stride;
     for (int k = __ldg(tb.row_ptr + (size_t)g * (N + 1) + u);; ++k) {  // the pick-th affordable neighbour exists
-      if (__ldg(wg + k) + p.toll <= m) {
+      if (__ldg(wg + k) + toll <= m) {
         if (pick == 0) {
           act = __ldg(tb.col + (size_t)g * tb.nnz_stride + k);
           break;
@@ -2986,6 +3020,7 @@ struct SyEnv {
   void* d_grp_bad = nullptr;     // int: ids out of range
   void* d_grp_stats = nullptr;   // u64 [GROUP_STAT_LINES, SY_NUM_STATS]: [grp_rep, grp_n] lines in use
   bool grp_need_reset = false;  // groups changed: steps are refused until a full sy_reset
+  std::vector<GroupRow> grp_rows;  // host copy of the rows in use (sy_set_group_tolls rewrites their tolls)
 };
 
 namespace {
@@ -3226,7 +3261,7 @@ void launch_observe(const SyEnv* e, const Params& p0, unsigned grid, cudaStream_
       grid = (unsigned)(full + rest * k);
     }
   }
-  if (p.grp_n && p.belief_score && p.out.stats) {  // mechanism groups: belief scores also summed per group
+  if (p.grp_n) {  // mechanism groups: every env's own toll, belief scores also summed per group
     if (p.wr_bulk) {
       if (gen) sy_observe_kernel<GEN_BEL_WARPS, GEN_WR_WARPS, WV_BULK, 1><<<grid, THREADS, e->obs_smem, s>>>(p);
       else sy_observe_kernel<BEL_WARPS, WR_WARPS, WV_BULK, 1><<<grid, THREADS, e->obs_smem, s>>>(p);
@@ -4049,7 +4084,9 @@ int sample_impl(SyEnv* e, const SyState* st, uint32_t step_counter, ActT* action
   if (rc) return rc;
   CUDA_TRY(cudaSetDevice(e->cfg.device));
   const size_t n = (size_t)p.B * p.A;
-  sy_sample_actions_kernel<ActT><<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(p, step_counter, actions, step_base);
+  const unsigned grid = (unsigned)((n + 255) / 256);
+  if (p.grp_n) sy_sample_actions_kernel<ActT, 1><<<grid, 256, 0, (cudaStream_t)stream>>>(p, step_counter, actions, step_base);
+  else sy_sample_actions_kernel<ActT><<<grid, 256, 0, (cudaStream_t)stream>>>(p, step_counter, actions, step_base);
   g_launches++;
   CUDA_TRY(cudaGetLastError());
   return SY_OK;
@@ -4226,6 +4263,7 @@ int sy_set_groups(SyEnv* e, int32_t n, const SyGroup* groups, const int32_t* gro
     rows[g].agent_money = q.agent_money;
     rows[g].reveal = q.reveal_interval;
     rows[g].reveal_skip_thresh = q.reveal_skip_prob > 0.0f ? (unsigned long long)((double)fminf(q.reveal_skip_prob, 1.0f) * 4294967296.0) : 0ull;
+    rows[g].toll = e->cfg.toll;  // every group starts with the config's toll (sy_set_group_tolls changes it)
   }
   CUDA_TRY(cudaSetDevice(e->cfg.device));
   cudaStream_t s = (cudaStream_t)stream;
@@ -4263,8 +4301,28 @@ int sy_set_groups(SyEnv* e, int32_t n, const SyGroup* groups, const int32_t* gro
   CUDA_TRY(cudaMemsetAsync(e->d_grp_stats, 0, (size_t)GROUP_STAT_LINES * SY_NUM_STATS * sizeof(unsigned long long), s));
   CUDA_TRY(cudaStreamSynchronize(s));  // (the host table is a local)
   e->grp_n = n;
+  e->grp_rows = std::move(rows);
   // per-group lines spread like the handle-wide replicas: rep * n <= GROUP_STAT_LINES for every n <= SY_MAX_GROUPS
   e->grp_rep = n ? std::max(1, std::min(STAT_REPLICAS, GROUP_STAT_LINES / n)) : 0;
+  e->grp_need_reset = true;
+  return SY_OK;
+}
+
+int sy_set_group_tolls(SyEnv* e, int32_t n, const int32_t* tolls, sy_stream_t stream) {
+  if (!e) return fail(SY_ERR_INVALID_ARGUMENT, "NULL env");
+  if (e->obs_pending) return fail(SY_ERR_STATE, "sy_set_group_tolls: observations are pending (sy_flush_observations first)");
+  if (e->grp_n == 0) return fail(SY_ERR_STATE, "sy_set_group_tolls: no mechanism groups are set (sy_set_groups first)");
+  if (n != e->grp_n) return fail(SY_ERR_INVALID_ARGUMENT, "sy_set_group_tolls: num_groups %d, but the handle holds %d groups", n, e->grp_n);
+  if (!tolls) return fail(SY_ERR_INVALID_ARGUMENT, "tolls is NULL");
+  for (int g = 0; g < n; ++g)
+    if (tolls[g] < 0 || tolls[g] > SY_MAX_TOLL) return fail(SY_ERR_INVALID_ARGUMENT, "group %d: toll %d outside [0, %d]", g, tolls[g], SY_MAX_TOLL);
+  std::vector<GroupRow> rows = e->grp_rows;
+  for (int g = 0; g < n; ++g) rows[g].toll = tolls[g];
+  CUDA_TRY(cudaSetDevice(e->cfg.device));
+  cudaStream_t s = (cudaStream_t)stream;
+  CUDA_TRY(cudaMemcpyAsync(e->d_grp, rows.data(), (size_t)n * sizeof(GroupRow), cudaMemcpyHostToDevice, s));
+  CUDA_TRY(cudaStreamSynchronize(s));  // (the host table is a local)
+  e->grp_rows = std::move(rows);
   e->grp_need_reset = true;
   return SY_OK;
 }

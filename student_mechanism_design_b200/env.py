@@ -36,13 +36,26 @@ MAX_MONEY_LIMIT = 1000  # yard.py:11
 N_EXP_TABLE = 1100  # exp(-d) underflows to 0 beyond d = 745
 
 
-MECHANISM_KEYS = ("reward_weights", "agent_money", "reveal_interval", "reveal_skip_prob")
+MECHANISM_KEYS = ("reward_weights", "agent_money", "reveal_interval", "reveal_skip_prob", "tolls")
+
+
+def mechanism_toll(mech: Dict, base) -> int:
+    """The toll of one mechanism dict: its `tolls` (the constructor's rule: integral and >= 0, so 1.0 is accepted; at most
+    SY_MAX_TOLL), else `base.tolls`.  Raises ValueError on what sy_set_group_tolls would refuse."""
+    toll = mech["tolls"] if "tolls" in mech else base.tolls
+    if isinstance(toll, torch.Tensor):
+        toll = toll.item()
+    if isinstance(toll, bool) or not isinstance(toll, (int, float, np.integer, np.floating)) or not np.isfinite(toll) \
+            or int(toll) != toll or not 0 <= int(toll) <= _cabi.SY_MAX_TOLL:
+        raise ValueError(f"tolls must be an integer in [0, {_cabi.SY_MAX_TOLL}], got {toll!r}")
+    return int(toll)
 
 
 def pack_mechanism(mech: Dict, base) -> "_cabi.SyGroup":
     """One mechanism dict (keys of MECHANISM_KEYS, all optional) as the SyGroup of sy_set_groups; missing keys and
     missing reward-weight names take `base`'s values (an env, or anything with `reward_weights`, `agent_money`,
-    `reveal_interval` and `config.reveal_skip_prob`).  Raises ValueError / KeyError on what the library would refuse."""
+    `reveal_interval` and `config.reveal_skip_prob`).  Raises ValueError / KeyError on what the library would refuse.
+    A `tolls` key is validated here (mechanism_toll) but travels separately, through sy_set_group_tolls."""
     if not isinstance(mech, dict):
         raise TypeError(f"a mechanism is a dict, got {type(mech).__name__}")
     unknown = set(mech) - set(MECHANISM_KEYS)
@@ -66,6 +79,8 @@ def pack_mechanism(mech: Dict, base) -> "_cabi.SyGroup":
         raise ValueError(f"reveal_interval must be a non-negative integer, got {reveal}")
     if not 0.0 <= skip <= 1.0:
         raise ValueError(f"reveal_skip_prob must be in [0, 1], got {skip}")
+    if "tolls" in mech:
+        mechanism_toll(mech, base)
     g = _cabi.SyGroup()
     g.struct_bytes = C.sizeof(_cabi.SyGroup)
     for i, v in enumerate(w):
@@ -74,11 +89,54 @@ def pack_mechanism(mech: Dict, base) -> "_cabi.SyGroup":
     return g
 
 
-def unpack_mechanism(g: "_cabi.SyGroup") -> Dict:
-    """The complete mechanism dict of a SyGroup (float weights)"""
-    return dict(reward_weights={k: float(g.reward_weights[i]) for i, k in enumerate(REWARD_WEIGHT_NAMES)},
-                agent_money=int(g.agent_money), reveal_interval=int(g.reveal_interval),
-                reveal_skip_prob=float(g.reveal_skip_prob))
+def unpack_mechanism(g: "_cabi.SyGroup", tolls: Optional[int] = None) -> Dict:
+    """The complete mechanism dict of a SyGroup (float weights), with `tolls` when given"""
+    d = dict(reward_weights={k: float(g.reward_weights[i]) for i, k in enumerate(REWARD_WEIGHT_NAMES)},
+             agent_money=int(g.agent_money), reveal_interval=int(g.reveal_interval),
+             reveal_skip_prob=float(g.reveal_skip_prob))
+    if tolls is not None:
+        d["tolls"] = int(tolls)
+    return d
+
+
+def group_metrics(per: Sequence[Dict], mechanisms: Sequence[Dict], number_of_agents: int):
+    """What metrics() needs while mechanism groups are set, from the per-group statistics `per` (stats(by_group=True))
+    and the mechanism dicts: (efficiency sum, tolls paid, per-group metrics).  A group's budget efficiency uses its own agent_money and its
+    mean_tolls_paid its own toll; the aggregate weighs every group against its own budget and sums the tolls paid as
+    the integer sum over groups of toll * police_moves (divided once: groups with the constructor's toll give exactly
+    the float of a handle without groups)."""
+    by_group = [metrics_of(g, initial=max(number_of_agents * m["agent_money"], 1), tolls_paid=m["tolls"] * g["police_moves"])
+                for g, m in zip(per, mechanisms)]
+    eff = sum(g["sum_episode_budget_spent"] / max(number_of_agents * m["agent_money"], 1) for g, m in zip(per, mechanisms))
+    paid = sum(int(m["tolls"]) * int(g["police_moves"]) for g, m in zip(per, mechanisms))
+    return eff, paid, by_group
+
+
+def metrics_of(st: Dict, initial: int, tolls_paid: int, eff_sum=None) -> Dict[str, float]:
+    """MetricsTracker.get_aggregated_metrics (src/eval/metrics.py:168-232) of one statistics dict; `initial` = the police
+    budget of an episode, `tolls_paid` = the tolls paid over all episodes (an integer)"""
+    n = st["episodes"]
+    r = st["reveals"]
+    mean_ce = st["sum_belief_ce_q24"] / _cabi.BELIEF_CE_SCALE / r if r else 0.0
+    var_ce = max(st["sum_sq_belief_ce_q24"] / _cabi.BELIEF_CE_SCALE / r - mean_ce * mean_ce, 0.0) if r else 0.0
+    if n == 0:  # metrics.py:170-186
+        return dict(num_episodes=0, mrx_wins=0, police_wins=0, win_rate=0.5, win_rate_std=0.0, mean_episode_length=0.0,
+                    episode_length_std=0.0, mean_belief_ce=mean_ce, belief_ce_std=float(np.sqrt(var_ce)),
+                    mean_tolls_paid=0.0, mean_budget_spent=0.0, mean_budget_efficiency=0.0,
+                    mean_time_to_catch=0.0, mean_survival_time=0.0)
+    wr = st["mrx_wins"] / n
+    ml = st["sum_episode_length"] / n
+    var_l = max(st["sum_sq_episode_length"] / n - ml * ml, 0.0)
+    spent = st["sum_episode_budget_spent"] / n
+    return dict(
+        num_episodes=n, mrx_wins=st["mrx_wins"], police_wins=st["police_wins"], win_rate=wr,
+        win_rate_std=float(np.sqrt(wr * (1.0 - wr))), mean_episode_length=ml, episode_length_std=float(np.sqrt(var_l)),
+        mean_belief_ce=mean_ce, belief_ce_std=float(np.sqrt(var_ce)),
+        mean_tolls_paid=tolls_paid / n, mean_budget_spent=spent,
+        mean_budget_efficiency=spent / initial if eff_sum is None else eff_sum / n,
+        mean_time_to_catch=st["sum_length_police_wins"] / st["police_wins"] if st["police_wins"] else 0.0,
+        mean_survival_time=st["sum_length_mrx_wins"] / st["mrx_wins"] if st["mrx_wins"] else 0.0,
+    )
 
 
 def numpy_reward_tables(max_timestep: int = 250):
@@ -252,6 +310,7 @@ class BatchedScotlandYardEnv:
         self._is_reset = False
         self._need_full_reset = False
         self._mechanisms, self._group_id, self.group_stats_vec = None, None, None  # set_mechanisms
+        self._env_toll = None  # int32 [B, 1] while some mechanism group's toll differs from `tolls`
         self._groups_generation = 0  # set_mechanisms calls: captured rollout graphs check it
 
     # ------------------------------------------------------------------ plumbing
@@ -423,26 +482,33 @@ class BatchedScotlandYardEnv:
     def set_mechanisms(self, mechanisms, group_id=None):
         """Evaluate several mechanisms in this one batch (sy_set_groups).  `mechanisms`: a sequence of dicts with the
         optional keys `reward_weights` (a dict keyed by REWARD_WEIGHT_NAMES, floats or 0-dim tensors; missing names keep
-        the constructor's weight), `agent_money`, `reveal_interval` and `reveal_skip_prob` (a missing key keeps the
-        constructor's value).  `group_id`: int tensor [B] (env -> index into `mechanisms`), or None for
+        the constructor's weight), `agent_money`, `reveal_interval`, `reveal_skip_prob` and `tolls` (a missing key keeps
+        the constructor's value).  `group_id`: int tensor [B] (env -> index into `mechanisms`), or None for
         (env_offset + b) % len(mechanisms).  `mechanisms=None` clears the groups.  Pending observations are flushed
         first; the new mechanisms take effect at the next full `reset()`, which `step` and the rollouts require."""
         self.flush_observations()
         if mechanisms is None:
-            table, gid = [], None
+            table, tolls, gid = [], [], None
         else:
             table = [pack_mechanism(m, self) for m in mechanisms]
+            tolls = [mechanism_toll(m, self) for m in mechanisms]
             if not 1 <= len(table) <= _cabi.SY_MAX_GROUPS:
                 raise ValueError(f"between 1 and {_cabi.SY_MAX_GROUPS} mechanisms, got {len(table)}")
             gid = None if group_id is None else self._dev(group_id, torch.int32, (self.num_envs,))
         arr = (_cabi.SyGroup * max(len(table), 1))(*table)
+        own_tolls = any(t != self.tolls for t in tolls)
         with torch.cuda.device(self.device):
             _cabi.check(self._lib.sy_set_groups(self._handle, len(table), arr, _ptr(gid), self._stream()))
-        self._mechanisms = None if mechanisms is None else tuple(unpack_mechanism(g) for g in table)
-        self._group_id = None
+            if own_tolls:  # (sy_set_groups gave every group the constructor's toll)
+                _cabi.check(self._lib.sy_set_group_tolls(self._handle, len(tolls), (C.c_int32 * len(tolls))(*tolls),
+                                                         self._stream()))
+        self._mechanisms = None if mechanisms is None else tuple(unpack_mechanism(g, t) for g, t in zip(table, tolls))
+        self._group_id, self._env_toll = None, None
         if table:
             self._group_id = gid.clone() if gid is not None else (
                 (torch.arange(self.num_envs, device=self.device, dtype=torch.int64) + self.env_offset) % len(table)).to(torch.int32)
+            if own_tolls:  # int32 [B, 1] toll of each env (the policies' legality test, see policy._PolicyBase._state)
+                self._env_toll = torch.tensor(tolls, dtype=torch.int32, device=self.device)[self._group_id.long()].view(-1, 1)
         self.group_stats_vec = torch.zeros(len(table), _cabi.SY_NUM_STATS, dtype=torch.int64, device=self.device) \
             if table and self.stats_vec is not None else None
         self._need_full_reset = True  # the next reset() covers every env
@@ -761,39 +827,12 @@ class BatchedScotlandYardEnv:
         (its budget efficiency against its own agent_money).  While groups are set, the aggregate efficiency weighs
         every group's spending against that group's budget."""
         if by_group:
-            return [self._metrics_of(st, initial=max(self.number_of_agents * m["agent_money"], 1))
-                    for st, m in zip(self.stats(reduce_group, by_group=True), self._mechanisms)]
+            return group_metrics(self.stats(reduce_group, by_group=True), self._mechanisms, self.number_of_agents)[2]
         st = self.stats(reduce_group)
-        eff = None
+        eff, paid = None, self.tolls * st["police_moves"]
         if self._mechanisms is not None and self.group_stats_vec is not None:
-            per = self.stats(reduce_group, by_group=True)
-            eff = sum(g["sum_episode_budget_spent"] / max(self.number_of_agents * m["agent_money"], 1)
-                      for g, m in zip(per, self._mechanisms))
-        return self._metrics_of(st, initial=max(self.number_of_agents * self.agent_money, 1), eff_sum=eff)
-
-    def _metrics_of(self, st, initial, eff_sum=None) -> Dict[str, float]:
-        n = st["episodes"]
-        r = st["reveals"]
-        mean_ce = st["sum_belief_ce_q24"] / _cabi.BELIEF_CE_SCALE / r if r else 0.0
-        var_ce = max(st["sum_sq_belief_ce_q24"] / _cabi.BELIEF_CE_SCALE / r - mean_ce * mean_ce, 0.0) if r else 0.0
-        if n == 0:  # metrics.py:170-186
-            return dict(num_episodes=0, mrx_wins=0, police_wins=0, win_rate=0.5, win_rate_std=0.0, mean_episode_length=0.0,
-                        episode_length_std=0.0, mean_belief_ce=mean_ce, belief_ce_std=float(np.sqrt(var_ce)),
-                        mean_tolls_paid=0.0, mean_budget_spent=0.0, mean_budget_efficiency=0.0,
-                        mean_time_to_catch=0.0, mean_survival_time=0.0)
-        wr = st["mrx_wins"] / n
-        ml = st["sum_episode_length"] / n
-        var_l = max(st["sum_sq_episode_length"] / n - ml * ml, 0.0)
-        spent = st["sum_episode_budget_spent"] / n
-        return dict(
-            num_episodes=n, mrx_wins=st["mrx_wins"], police_wins=st["police_wins"], win_rate=wr,
-            win_rate_std=float(np.sqrt(wr * (1.0 - wr))), mean_episode_length=ml, episode_length_std=float(np.sqrt(var_l)),
-            mean_belief_ce=mean_ce, belief_ce_std=float(np.sqrt(var_ce)),
-            mean_tolls_paid=self.tolls * st["police_moves"] / n, mean_budget_spent=spent,
-            mean_budget_efficiency=spent / initial if eff_sum is None else eff_sum / n,
-            mean_time_to_catch=st["sum_length_police_wins"] / st["police_wins"] if st["police_wins"] else 0.0,
-            mean_survival_time=st["sum_length_mrx_wins"] / st["mrx_wins"] if st["mrx_wins"] else 0.0,
-        )
+            eff, paid, _ = group_metrics(self.stats(reduce_group, by_group=True), self._mechanisms, self.number_of_agents)
+        return metrics_of(st, initial=max(self.number_of_agents * self.agent_money, 1), tolls_paid=paid, eff_sum=eff)
 
     def _fold_stats(self):
         """sy_stats: add what the kernels accumulated since the last call to `stats_vec`"""

@@ -74,6 +74,7 @@ class _PolicyBase:
         self._lib = pc.load_library()
         self.env = env
         self._tables: Optional[_GraphTables] = None
+        self._headroom: Optional[torch.Tensor] = None  # int32 [B, A] money - toll of the env's mechanism group
 
     def _graphs(self) -> pc.SyPolicyGraphs:
         # a refreshed device pool (env.regenerate_graphs) bumps the generation; `id(list)` alone can be recycled by a
@@ -88,6 +89,13 @@ class _PolicyBase:
         s = pc.SyPolicyState()
         s.num_envs, s.num_agents, s.toll, s.env_offset = e.num_envs, e.num_agents, int(e.tolls), e.env_offset
         s.pos, s.money, s.graph_id = e.pos.data_ptr(), e.money.data_ptr(), e.graph_id.data_ptr()
+        if e._env_toll is not None:
+            # mechanism groups with their own tolls: the kernels read budgets only to test w + toll <= money, so they get
+            # the headroom money - toll_b and toll 0 (the same test, in exact integers)
+            if self._headroom is None or self._headroom.shape != e.money.shape or self._headroom.device != e.money.device:
+                self._headroom = torch.empty_like(e.money)
+            torch.sub(e.money, e._env_toll, out=self._headroom)
+            s.money, s.toll = self._headroom.data_ptr(), 0
         s.mrx_revealed = e.mrx_revealed.data_ptr()
         return s
 

@@ -5,7 +5,11 @@ event pair, actions drawn once beforehand) and the replayed `capture_rollout` gr
 c3 runs with the belief scored at reveal steps (belief_ce), so the per-group cross-entropy atomics are included.
 Writes profiles/r03_mechanisms_c{2,3}.json (or --out-dir) with the card's name and power limit.
 
-    python tools/bench_mechanisms.py [--workloads c3,c2] [--steps 50] [--passes 5]
+--tolls (opt-in): no groups, the same 16 groups, and those 16 groups with their own tolls cycling 0..3 (group g pays
+g % 4), timed the same way; writes profiles/r04_group_tolls_c{2,3}.json.  Other tolls change the games themselves (which
+moves are legal, how long episodes last), so that variant does not do exactly the same game work.
+
+    python tools/bench_mechanisms.py [--workloads c3,c2] [--steps 50] [--passes 5] [--tolls]
 """
 import argparse
 import json
@@ -22,6 +26,7 @@ WORKLOADS = {  # bench.py's c2 / c3 (c3 with the belief scored at reveals)
     "c3": dict(N=200, E=400, P=6, money=20, toll=1, belief=True, reveal=5, B=65536),
 }
 VARIANTS = ["no_groups", "one_group_equal", "groups_16", "groups_1024"]
+TOLL_VARIANTS = ["no_groups", "groups_16", "groups_16_tolls"]
 
 
 def card():
@@ -36,25 +41,29 @@ def card():
         return dict(name=torch.cuda.get_device_name(0), power_limit=f"unknown ({exc.__class__.__name__})")
 
 
-def run(wl_name, steps, passes):
+def run(wl_name, steps, passes, variants=VARIANTS):
     import torch
 
     from student_mechanism_design_b200 import BatchedScotlandYardEnv
 
     wl = WORKLOADS[wl_name]
     envs = {}
-    for v in VARIANTS:
+    for v in variants:
         env = BatchedScotlandYardEnv(wl["B"], wl["P"], wl["money"], graph_nodes=wl["N"], graph_edges=wl["E"], seed=0,
                                      num_graphs=1, tolls=wl["toll"], belief=wl["belief"], belief_ce=wl["belief"],
                                      reveal_interval=wl["reveal"], auto_reset=True, device="cuda:0")
         if v == "one_group_equal":
             env.set_mechanisms([{}])
-        elif v in ("groups_16", "groups_1024"):
+        elif v in ("groups_16", "groups_1024", "groups_16_tolls"):
             # distinct mechanisms with the config's budget and reveal schedule: only the reward weights differ, so
             # every variant does the same game work and the difference is the cost of the groups themselves
-            n = 16 if v == "groups_16" else 1024
-            env.set_mechanisms([dict(reward_weights={"Mrx_closest": 0.3 + 0.001 * g, "Police_distance": 0.1 + 0.001 * g})
-                                for g in range(n)])
+            n = 1024 if v == "groups_1024" else 16
+            mechs = [dict(reward_weights={"Mrx_closest": 0.3 + 0.001 * g, "Police_distance": 0.1 + 0.001 * g})
+                     for g in range(n)]
+            if v == "groups_16_tolls":
+                for g, m in enumerate(mechs):
+                    m["tolls"] = g % 4
+            env.set_mechanisms(mechs)
         env.reset()
         acts = env.sample_actions(step_counter=0)
         graph, _ = env.capture_rollout(steps)
@@ -64,9 +73,9 @@ def run(wl_name, steps, passes):
         envs[v] = (env, acts, graph)
     torch.cuda.synchronize()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    times = {v: {"sy_step_ms": [], "graph_replay_ms": []} for v in VARIANTS}
+    times = {v: {"sy_step_ms": [], "graph_replay_ms": []} for v in variants}
     for p in range(passes):
-        order = VARIANTS if p % 2 == 0 else VARIANTS[::-1]  # alternate, so drift does not favour one variant
+        order = variants if p % 2 == 0 else variants[::-1]  # alternate, so drift does not favour one variant
         for v in order:
             env, acts, graph = envs[v]
             ev0.record()
@@ -81,7 +90,7 @@ def run(wl_name, steps, passes):
             torch.cuda.synchronize()
             times[v]["graph_replay_ms"].append(ev0.elapsed_time(ev1) / steps)
     out = {}
-    for v in VARIANTS:
+    for v in variants:
         env = envs[v][0]
         row = {}
         for k, xs in times[v].items():
@@ -91,9 +100,11 @@ def run(wl_name, steps, passes):
         row["groups"] = 0 if env.mechanisms is None else len(env.mechanisms)
         out[v] = row
     base = out["no_groups"]
-    for v in VARIANTS[1:]:
+    for v in variants[1:]:
         for k in ("sy_step_ms", "graph_replay_ms"):
             out[v][k + "_vs_no_groups"] = out[v][k] / base[k] - 1.0
+            if v == "groups_16_tolls":
+                out[v][k + "_vs_groups_16"] = out[v][k] / out["groups_16"][k] - 1.0
     for env, _, _ in envs.values():
         env.close()
     return out
@@ -105,6 +116,7 @@ def main():
     ap.add_argument("--steps", type=int, default=50)
     ap.add_argument("--passes", type=int, default=5)
     ap.add_argument("--out-dir", default=os.path.join(ROOT, "profiles"))
+    ap.add_argument("--tolls", action="store_true", help="16 groups with and without their own tolls (r04 profiles)")
     args = ap.parse_args()
     import torch
 
@@ -113,12 +125,15 @@ def main():
     info = card()
     os.makedirs(args.out_dir, exist_ok=True)
     for w in args.workloads.split(","):
-        res = dict(workload=w, config=WORKLOADS[w], steps_per_pass=args.steps, passes=args.passes, card=info,
-                   note="every variant takes the handle's usual path (c3: dynamics + observation kernels, c2: fused "
-                        "step / one-launch rollout kernel), the grouped ones through its GROUPS instantiation; c3 scores "
-                        "the belief at reveal steps (about 4 us per step over bench.py's c3 line, which does not)",
-                   variants=run(w, args.steps, args.passes))
-        path = os.path.join(args.out_dir, f"r03_mechanisms_{w}.json")
+        note = ("every variant takes the handle's usual path (c3: dynamics + observation kernels, c2: fused "
+                "step / one-launch rollout kernel), the grouped ones through its GROUPS instantiation; c3 scores "
+                "the belief at reveal steps (about 4 us per step over bench.py's c3 line, which does not)")
+        if args.tolls:
+            note += (f"; groups_16_tolls: group g pays toll g % 4 (config toll {WORKLOADS[w]['toll']}), so its games "
+                     "differ from the other variants'")
+        res = dict(workload=w, config=WORKLOADS[w], steps_per_pass=args.steps, passes=args.passes, card=info, note=note,
+                   variants=run(w, args.steps, args.passes, TOLL_VARIANTS if args.tolls else VARIANTS))
+        path = os.path.join(args.out_dir, f"r04_group_tolls_{w}.json" if args.tolls else f"r03_mechanisms_{w}.json")
         with open(path, "w") as f:
             json.dump(res, f, indent=1)
         print(json.dumps(res))
