@@ -111,11 +111,17 @@ typedef struct SyConfig {
  * size with SY_ERR_INVALID_ARGUMENT instead of reading past the caller's memory (a binding written against an older
  * header would otherwise hand the kernels garbage pointers). */
 
-/* Per-env state, device pointers, caller-owned (yard.py:111-127 state, batched). */
+/* Per-env state, device pointers, caller-owned (yard.py:111-127 state, batched).
+ * Absent agents: an env whose mechanism group plays with fewer police than the config (sy_set_group_rules, P_g <
+ * num_police) keeps the [B, A, ...] layout; its agents P_g + 1 .. A - 1 are absent and carry exactly these values:
+ * pos -1, money 0, agent_budget 0.0f, reward (and reward64) 0.0, terminated / truncated / done equal to the env's own
+ * flags, an all-zero action_mask row and node_features column (both dtypes); sy_sample_actions and the in-kernel
+ * action draws give them -1, their actions are ignored whatever they hold, and their init_pos entries (sy_reset) are
+ * ignored and come back as -1. */
 typedef struct SyState {
   uint64_t struct_bytes; /* = sizeof(SyState) */
-  int32_t* pos;      /* [B, A]  MrX_pos + police_positions */
-  int32_t* money;    /* [B, A]  agents_money */
+  int32_t* pos;      /* [B, A]  MrX_pos + police_positions (-1: absent agent, see above) */
+  int32_t* money;    /* [B, A]  agents_money (0: absent agent) */
   int32_t* timestep; /* [B] */
   int32_t* graph_id; /* [B] index into the graph pool */
   int32_t* episode;  /* [B] episodes started (Philox counter) */
@@ -130,7 +136,8 @@ typedef struct SyState {
 
 /* Dynamic observation tensors written every reset/step (yard.py:271-335).  Static graph
  * tensors (adjacency_matrix, edge_index, edge_features) are per-graph and are built once by
- * the host from the same CSR; belief_map is SyState.belief; agent_position is SyState.pos. */
+ * the host from the same CSR; belief_map is SyState.belief; agent_position is SyState.pos.
+ * Absent agents (see SyState) have all-zero action_mask rows and node_features columns and agent_budget 0.0f. */
 typedef struct SyObs {
   uint64_t struct_bytes; /* = sizeof(SyObs) */
   uint8_t* action_mask;  /* [B, A, N] bool */
@@ -336,8 +343,8 @@ int sy_stats(SyEnv* env, int64_t* stats, sy_stream_t stream);
 
 /* Mechanism groups: one handle evaluates up to SY_MAX_GROUPS mechanisms side by side.  Every env belongs to one group,
  * and a group replaces, for its envs, the config's reward weights (fp32 reward mode uses (float)w), police start budget
- * (agent_money), reveal schedule (reveal_interval, reveal_skip_prob) and, through sy_set_group_tolls, the toll.  The
- * number of police and max_timestep stay one value per handle.
+ * (agent_money), reveal schedule (reveal_interval, reveal_skip_prob), through sy_set_group_tolls the toll, and through
+ * sy_set_group_rules the number of police and the episode horizon (max_timestep), each bounded by the config's.
  * Group membership enters no random stream, so a group equal to the config reproduces a handle without groups bit for
  * bit.  Every step path runs with groups (its GROUPS instantiation) except the split step of SY_OPT_NF_FILL, which acts
  * as off while groups are set (results are the same).  The statistics are also summed per group (sy_group_stats).
@@ -357,7 +364,8 @@ typedef struct SyGroup {
  * library-owned memory; a rejected call keeps the previous groups.  The new groups take effect at the next sy_reset of
  * every env (NULL reset_mask, or one with every byte set): until then the step and rollout entry points fail with
  * SY_ERR_STATE (so a state saved under groups cannot be resumed mid-episode: the reset starts new episodes).  Fails with
- * SY_ERR_STATE while observations are pending.  Clears the per-group statistics.  Every group gets the config's toll. */
+ * SY_ERR_STATE while observations are pending.  Clears the per-group statistics.  Every group gets the config's toll,
+ * num_police and max_timestep. */
 int sy_set_groups(SyEnv* env, int32_t num_groups, const SyGroup* groups, const int32_t* group_id, sy_stream_t stream);
 /* Per-group tolls: an env pays its group's toll instead of SyConfig.toll -- a move is legal iff w + toll <= budget (MrX and
  * police; action_mask, the random sampler and the mobility term of the rewards follow the same rule), and a police move
@@ -369,6 +377,19 @@ int sy_set_groups(SyEnv* env, int32_t num_groups, const SyGroup* groups, const i
  * `stream`. */
 #define SY_MAX_TOLL 1048576
 int sy_set_group_tolls(SyEnv* env, int32_t num_groups, const int32_t* tolls, sy_stream_t stream);
+/* Per-group police count and episode horizon.  num_police / max_timestep: HOST int32 [num_groups], either may be NULL
+ * (= the config's value for every group); num_police[g] in [1, config.num_police], max_timestep[g] in
+ * [0, config.max_timestep] (the bounds keep the coverage table, the u16 visit counters and every buffer sized by the
+ * handle valid).  Agents 0 .. num_police[g] of an env of group g play exactly as in a handle built with
+ * num_police = num_police[g], max_timestep = max_timestep[g] and the group's other fields (start nodes, moves, capture,
+ * "every police skipped", rewards in both modes, visits, belief, reveals and statistics, bit for bit; budget spent and
+ * police moves count its police only); the timeout is timestep > max_timestep[g].  The other agents are absent (see
+ * SyState).  num_groups must be the number set by sy_set_groups; a rejected call keeps the previous values.  Like
+ * sy_set_group_tolls: fails with SY_ERR_STATE while observations are pending (or when no groups are set), the new
+ * values take effect at the next sy_reset of every env, which the step and rollout entry points require until then,
+ * and a CUDA graph captured before the call must be captured again.  Clears nothing else.  Synchronises `stream`. */
+int sy_set_group_rules(SyEnv* env, int32_t num_groups, const int32_t* num_police, const int32_t* max_timestep,
+                       sy_stream_t stream);
 /* Add the per-group statistics accumulated since the last call to `stats` (DEVICE int64 [num_groups, SY_NUM_STATS],
  * caller-owned, cumulative) and clear the accumulators; num_groups must be the number set.  They are collected by the
  * same steps as sy_stats, with the same integer sums, so the sum over groups equals the handle-wide vector. */

@@ -112,6 +112,7 @@ SIGNATURES = {
     "sy_set_groups": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(SyGroup), C.c_void_p, C.c_void_p]),
     "sy_group_stats": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
     "sy_set_group_tolls": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(C.c_int32), C.c_void_p]),
+    "sy_set_group_rules": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_void_p]),
     "sy_allreduce_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sy_rollout_random_dev": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(SyState), C.POINTER(SyObs),
                                         C.POINTER(SyOut), C.c_void_p]),

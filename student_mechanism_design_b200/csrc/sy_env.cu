@@ -182,8 +182,29 @@ struct GroupRow {
   float w32[SY_NUM_REWARD_WEIGHTS];
   int agent_money, reveal;
   int toll;  // sy_set_group_tolls (sy_set_groups: the config's)
+  int num_police, max_t;  // sy_set_group_rules (sy_set_groups: the config's), in [1, P] / [0, max_timestep]
   unsigned long long reveal_skip_thresh;
 };
+
+// the number of police an env plays with and its episode horizon: the handle's, or (GROUPS) those of the env's
+// mechanism group `gr`.  Agents num_police + 1 .. A - 1 of an env are absent: pos -1, budget 0, reward 0, no action,
+// and no kernel looks up a graph table at their node.
+template <int GROUPS>
+__device__ __forceinline__ int env_police(const Params& p, const GroupRow* gr) {
+  if constexpr (GROUPS) return __ldg(&gr->num_police);
+  else return p.P;
+}
+template <int GROUPS>
+__device__ __forceinline__ int env_max_t(const Params& p, const GroupRow* gr) {
+  if constexpr (GROUPS) return __ldg(&gr->max_t);
+  else return p.max_t;
+}
+// ... whether agent a of env b is absent, when the env's group row is not at hand (false without groups)
+template <int GROUPS>
+__device__ __forceinline__ bool agent_absent(const Params& p, int b, int a) {
+  if constexpr (GROUPS) return a > env_police<1>(p, p.grp + __ldg(p.grp_id + b));
+  else return false;
+}
 
 // the toll an env pays per move (yard.py:223-229 and action_mask.py:65-76 with the toll extension: a move is legal iff
 // weight + toll <= budget, and costs weight + toll): the handle's, or (GROUPS) that of the env's mechanism group `gr`
@@ -242,7 +263,9 @@ __device__ __forceinline__ unsigned word_of(const uint4& r, int i) {
   return i == 0 ? r.x : (i == 1 ? r.y : (i == 2 ? r.z : r.w));
 }
 
-// A distinct uniform nodes (distribution of np.random.choice(N, A, replace=False), yard.py:112-116)
+// A distinct uniform nodes (distribution of np.random.choice(N, A, replace=False), yard.py:112-116).  Draw a depends
+// only on draws 0..a-1, so the first n of them are the start nodes of a handle with n agents (an env whose mechanism
+// group plays with fewer police uses the first num_police + 1 and ignores the rest).
 template <typename T>
 __device__ void philox_start_positions(const Params& p, unsigned env, unsigned episode, T* out, T* chosen /*A entries of scratch*/) {
   uint4 r = make_uint4(0, 0, 0, 0);
@@ -397,12 +420,12 @@ __device__ __forceinline__ int edge_weight_sg(const SharedGraph& sg, int u, int 
   return w;
 }
 
-// GROUPS: the toll of the env's mechanism group `gr`
+// GROUPS: the toll, police count and horizon of the env's mechanism group `gr`
 template <int MAXA, int GROUPS = 0, typename PosT>
 __device__ __forceinline__ int move_phase(const Params& p, PosT* pos, int* money, const int* act, int g, int t, int& spent, int& moves,
                                           const SharedGraph* sg = nullptr, const GroupRow* gr = nullptr) {
   const Tables& tb = p.tb;
-  const int N = p.N, P = p.P;
+  const int N = p.N, P = env_police<GROUPS>(p, gr);
   int rp[MAXA], rm[MAXA], ra[MAXA], wpre[MAXA];
 #pragma unroll
   for (int i = 0; i < MAXA; ++i) {
@@ -453,7 +476,7 @@ __device__ __forceinline__ int move_phase(const Params& p, PosT* pos, int* money
     }
   }
   // reward_calculator.py:63-79; `timestep` is the pre-increment value (yard.py:345,355)
-  return capture ? ST_CAPTURE : (t > p.max_t ? ST_TIMEOUT : (no_money ? ST_NO_MONEY : ST_RUNNING));
+  return capture ? ST_CAPTURE : (t > env_max_t<GROUPS>(p, gr) ? ST_TIMEOUT : (no_money ? ST_NO_MONEY : ST_RUNNING));
 }
 
 struct RewardTables {  // shared-memory copies of the head of the two float64 tables (built by NumPy on the host)
@@ -472,14 +495,14 @@ struct RewardInputs {
 };
 
 // reward of agent a (reward_calculator.py:26-92 endings, :94-266 shaped), float64 value (fp32 mode: the float, widened)
-// GROUPS: the weights of the env's mechanism group `gr` instead of the handle's
+// GROUPS: the weights and police count of the env's mechanism group `gr` instead of the handle's
 template <int MODE, int MAXA, int GROUPS = 0>
 __device__ __forceinline__ double agent_reward(const Params& p, const RewardTables& rt, const RewardInputs<MAXA>& in, int t, int status,
                                                int a, int visits_here, const GroupRow* gr = nullptr) {
   const Tables& tb = p.tb;
   auto w64 = [&](int k) { return GROUPS ? __ldg(&gr->w64[k]) : p.w64[k]; };
   auto w32 = [&](int k) { return GROUPS ? __ldg(&gr->w32[k]) : p.w32[k]; };
-  const int P = p.P;
+  const int P = env_police<GROUPS>(p, gr);
   if (status == ST_CAPTURE) return (a == 0) ? -1.0 : 1.0;
   if (status != ST_RUNNING) return (a == 0) ? 1.0 : 0.0;
   const double tt = (double)t;
@@ -631,15 +654,16 @@ struct LogicSmem {
 // LAG_BAR, LAGT threads: the observation warps arrive, the dynamics warps wait -- long after the arrival in practice).
 constexpr int LAG_BAR = 4;
 constexpr int LAG_CSR_BAR = 6;  // lagged kernel: the writers' staged graph is complete (writers arrive, dynamics warps wait)
-// GROUPS: mechanism groups are set -- every env reads its group's row (reward weights, police budget, reveal schedule, toll)
-// once per step through the read-only path, and the statistics are also summed per group
+// GROUPS: mechanism groups are set -- every env reads its group's row (reward weights, police budget, reveal schedule, toll,
+// police count, horizon) once per step through the read-only path, and the statistics are also summed per group
 template <int MODE, int MAXA, int BAR, int LAGT = 0, int CSRT = 0, int GROUPS = 0>
 __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm, int b0, int tid, const SharedGraph* sgp = nullptr,
                                            const int* sg_valid = nullptr, unsigned extra_ctr = 0, bool draw_next = true) {
   constexpr int DS = LogicSmem<MAXA>::DS;
   const int lane = tid & 31, warp = tid >> 5;
   const int nEnv = min(32, p.B - b0);
-  const int N = p.N, A = p.A, P = p.P;
+  const int N = p.N, A = p.A;
+  int P = p.P;  // (GROUPS: the env's police count, below; loaded here the instantiations without groups keep their code)
 #ifdef SY_PHASE_CLOCKS
   long long _t0 = clock64();
 #endif
@@ -710,6 +734,7 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
     grp = live ? __ldg(p.grp_id + b) : -1;
     gr = p.grp + max(grp, 0);
   }
+  if constexpr (GROUPS) P = env_police<1>(p, gr);  // police of this env: agents P + 1 .. A - 1 are absent
 
   // ---- P1, four warps in parallel:
   //   warp 0    the order-dependent moves + ending
@@ -726,7 +751,7 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
     const unsigned env_id = (unsigned)(p.env_offset + (unsigned long long)b);
     const unsigned ep = (unsigned)(sm.episode[lane] + 1);
     sm.reset_gid[lane] = p.resample_graph ? philox_graph_choice(p, env_id, ep) : g;
-    philox_start_positions(p, env_id, ep, sm.reset_pos + lane * HS, sm.dmat + lane * HS);
+    philox_start_positions(p, env_id, ep, sm.reset_pos + lane * HS, sm.dmat + lane * HS);  // (absent agents: unused)
     PHASE_SPAN(9, tp1);  // (lane-divergent branch: no warp-level synchronisation in here)
   }
   named_barrier(BAR, LOGIC_THREADS);
@@ -752,7 +777,7 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
       dq[k] = 0;
       if (shaped && q < npairs) {
         const int ij = sm.pair_ij[q];
-        dq[k] = __ldg(Dg + (size_t)pos[ij >> 8] * N + pos[ij & 0xff]);
+        if (!GROUPS || (ij & 0xff) <= P) dq[k] = __ldg(Dg + (size_t)pos[ij >> 8] * N + pos[ij & 0xff]);  // (i < j)
       }
     }
 #pragma unroll
@@ -785,8 +810,8 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
   if (live) {
 #pragma unroll 1
     for (int a = (warp + LOGIC_WARPS - 1) % LOGIC_WARPS; a < A; a += LOGIC_WARPS) {  // warp 0 (moves, next state) gets the fewest
-      double r64 = 0.0;
-      if (active) {
+      double r64 = 0.0;  // (absent agents: 0)
+      if (active && (!GROUPS || a <= P)) {
         int visits_here = 0;
         const int u = pos[a];
         if (a > 0) {  // police never share a node (yard.py:231): the P counters of an env are distinct addresses
@@ -845,7 +870,7 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
             gnew = sm.reset_gid[lane];
             money[0] = p.mrx_money;
             pos[0] = sm.reset_pos[lane * HS];
-            for (int i = 1; i <= P; ++i) {
+            for (int i = 1; i <= P; ++i) {  // (absent agents keep pos / money: P4 stores their fixed values)
               money[i] = agent_money;
               pos[i] = sm.reset_pos[lane * HS + i];
             }
@@ -943,8 +968,9 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
   for (int i = tid; i < nEnv * A; i += LOGIC_THREADS) {
     const int e = (i * p.inv_A) >> 16, a = i - e * A;  // i / A without a division (i < 512, A <= 16)
     const size_t o = (size_t)b0 * A + i;
-    const int m = sm.money[e * AS + a];
-    p.st.pos[o] = (int)sm.pos[e * HS + a];
+    const bool absent = agent_absent<GROUPS>(p, b0 + e, a);
+    const int m = absent ? 0 : sm.money[e * AS + a];
+    p.st.pos[o] = absent ? -1 : (int)sm.pos[e * HS + a];
     p.st.money[o] = m;
     p.ob.agent_budget[o] = (float)m;  // yard.py:329-331
   }
@@ -970,6 +996,10 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
     const unsigned ctr = p.next_counter + (p.next_counter_base ? *p.next_counter_base : 0u) + extra_ctr;
     for (int i = tid; i < nEnv * A; i += LOGIC_THREADS) {
       const int e = (i * p.inv_A) >> 16, a = i - e * A;
+      if (agent_absent<GROUPS>(p, b0 + e, a)) {  // no action, no table lookup
+        p.next_actions[(size_t)b0 * A + i] = -1;
+        continue;
+      }
       const int gg = sm.gid[e], u = (int)sm.pos[e * HS + a], m = sm.money[e * AS + a];
       // a same-step auto-reset with resample_graph may have moved the env to another graph than the staged one
       const bool use_sg = sg != nullptr && !p.resample_graph;
@@ -1054,7 +1084,7 @@ __global__ void __launch_bounds__(FILL_THREADS) sy_fill_kernel(uint8_t* dst, siz
 // ---------------------------------------------------------------------------------------------
 // reset kernel (yard.py:80-142): re-initialise the masked envs (same warp = 32 envs layout)
 // ---------------------------------------------------------------------------------------------
-// GROUPS: police budgets and reveal schedule of each env's mechanism group
+// GROUPS: police budgets, police count and reveal schedule of each env's mechanism group
 template <int GROUPS = 0>
 __global__ void __launch_bounds__(LOGIC_THREADS) sy_reset_kernel(const Params p) {
   __shared__ WarpTile wts[LOGIC_THREADS / 32];
@@ -1071,7 +1101,10 @@ __global__ void __launch_bounds__(LOGIC_THREADS) sy_reset_kernel(const Params p)
   for (int i = lane; i < nEnv * A; i += 32) {
     const int e = (i * p.inv_A) >> 16, a = i - e * A;  // i / A without a division (i < 512, A <= 16)
     const size_t o = (size_t)b0 * A + i;
-    if ((rst_mask >> e) & 1u) {
+    if (agent_absent<GROUPS>(p, b0 + e, a)) {  // (init_pos entries of absent agents are ignored)
+      wt.money[e * AS + a] = 0;
+      wt.pos[e * AS + a] = -1;
+    } else if ((rst_mask >> e) & 1u) {
       const int agent_money = GROUPS ? __ldg(&p.grp[__ldg(p.grp_id + b0 + e)].agent_money) : p.agent_money;
       wt.money[e * AS + a] = (a == 0) ? p.mrx_money : agent_money;  // yard.py:117-119
       wt.pos[e * AS + a] = p.init_pos ? p.init_pos[o] : 0;
@@ -1091,6 +1124,8 @@ __global__ void __launch_bounds__(LOGIC_THREADS) sy_reset_kernel(const Params p)
         const unsigned env_id = (unsigned)(p.env_offset + (unsigned long long)b);
         if (p.resample_graph && p.init_gid == nullptr) g = philox_graph_choice(p, env_id, (unsigned)episode);
         philox_start_positions(p, env_id, (unsigned)episode, wt.pos + lane * AS, wt.act + lane * AS);
+        if constexpr (GROUPS)  // the draws past the env's police are not used
+          for (int a = env_police<1>(p, p.grp + __ldg(p.grp_id + b)) + 1; a < A; ++a) wt.pos[lane * AS + a] = -1;
       }
     } else {
       t = p.st.timestep[b];
@@ -1292,7 +1327,9 @@ __device__ __forceinline__ void writer_role(const Params& p, unsigned char* dyn,
       if (ag < A && lane / lpa < R && !(p.dbg_skip & 2)) {
         const int u = s_pos[e * A + ag], m = s_money[e * A + ag], g = s_gid[e];
         uint8_t* row = img + (ag - a0) * N;
-        if (staged) {
+        if (GROUPS && u < 0) {
+          // absent agent: an all-zero row
+        } else if (staged) {
           const int r0 = s_rp[u], r1 = s_rp[u + 1];
           for (int k = r0 + sub; k < r1; k += lpa)
             if ((int)s_wgt[k] + wr_toll<GROUPS>(p) <= m) row[s_col[k]] = 1;
@@ -1370,6 +1407,7 @@ __device__ __forceinline__ void bulk_mask_ones(const Params& p, const BulkCtx& c
     const int de = (q * p.inv_A) >> 16, a = q - de * A, e = e_lo + de;
     const int u = c.s_pos[e * A + a], m = c.s_money[e * A + a];
     const int base = e * S + a * N - lo;
+    if (GROUPS && u < 0) continue;  // absent agent: an all-zero row
     if (STAGED) {
       const int r0 = c.rp[u], r1 = c.rp[u + 1];
       for (int k = r0; k < r1; ++k) {
@@ -1391,8 +1429,8 @@ __device__ __forceinline__ void bulk_mask_ones(const Params& p, const BulkCtx& c
 }
 
 // ones of the node_features stream (ELEM = 4: float32 1.0f, 1: uint8 1) in bytes [lo, lo + len); the MrX column stays
-// blank while he is hidden (yard.py:279-290 with the reveal schedule)
-template <int ELEM>
+// blank while he is hidden (yard.py:279-290 with the reveal schedule), and (GROUPS) an absent agent's column too
+template <int ELEM, int GROUPS = 0>
 __device__ __forceinline__ void bulk_nf_ones(const Params& p, const BulkCtx& c, uint8_t* img, int lo, int len, int lane, bool set) {
   const int N = p.N, A = p.A, S = N * A * ELEM;
   const int e_lo = lo / S, e_hi = (lo + len - 1) / S;
@@ -1400,6 +1438,7 @@ __device__ __forceinline__ void bulk_nf_ones(const Params& p, const BulkCtx& c, 
   for (int q = lane; q < npairs; q += 32) {
     const int de = (q * p.inv_A) >> 16, a = q - de * A, e = e_lo + de;
     if (a == 0 && c.s_rev[e] < 0) continue;
+    if (GROUPS && c.s_pos[e * A + a] < 0) continue;
     const int off = e * S + (c.s_pos[e * A + a] * A + a) * ELEM - lo;
     if ((unsigned)off < (unsigned)len) {
       if (ELEM == 4) *reinterpret_cast<unsigned*>(img + off) = set ? 0x3f800000u : 0u;
@@ -1447,7 +1486,9 @@ __device__ __forceinline__ void nf32_fill_piece(uint8_t* gnf, int lo, int hi, co
 
 // ones of the float32 node_features stream that fall into bytes [lo, hi) (yard.py:279-290; the MrX column stays blank
 // while he is hidden): lane = (env, agent) pair.  Env rows that are whole 16-byte granules get the granule rewritten
-// (assembled from every agent of the env that falls into it), others a 4-byte store.
+// (assembled from every agent of the env that falls into it), others a 4-byte store.  GROUPS: absent agents (pos -1)
+// have no one (their negative flat index never shares a granule with a present agent's).
+template <int GROUPS = 0>
 __device__ __forceinline__ void nf32_ones_piece(const Params& p, const BulkCtx& c, uint8_t* gnf, int lo, int hi, int lane) {
   const int A = p.A, S = p.N * A * 4;
   const int e_lo = lo / S, e_hi = (hi - 1) / S;
@@ -1458,6 +1499,7 @@ __device__ __forceinline__ void nf32_ones_piece(const Params& p, const BulkCtx& 
     const bool hidden = c.s_rev[e] < 0;
     if (a == 0 && hidden) continue;
     const int* pos = c.s_pos + e * A;
+    if (GROUPS && pos[a] < 0) continue;
     const int f = pos[a] * A + a;  // element index inside the env's row
     const int off = e * S + f * 4;
     if (off < lo || off >= hi) continue;
@@ -1493,7 +1535,7 @@ __device__ __forceinline__ void writer_stream_warp(const Params& p, const BulkCt
   auto ones = [&](int item, uint8_t* img, uint8_t v) {
     if (item < st.ncf) {
       const int lo = item * Cf;
-      bulk_nf_ones<1>(p, c, img, lo, min(Cf, st.Tf - lo), lane, v != 0);
+      bulk_nf_ones<1, GROUPS>(p, c, img, lo, min(Cf, st.Tf - lo), lane, v != 0);
     } else {
       const int lo = (item - st.ncf) * Cm, len = min(Cm, st.Tm - lo);
       if (staged) bulk_mask_ones<true, GROUPS>(p, c, img, lo, len, lane, v);
@@ -1503,7 +1545,7 @@ __device__ __forceinline__ void writer_stream_warp(const Params& p, const BulkCt
   auto piece_ones = [&](int item) {
     if (gnf32 && item >= st.ncf) {
       const int lo = 4 * (item - st.ncf) * Cm;
-      nf32_ones_piece(p, c, gnf32, lo, min(Tf32, lo + 4 * Cm), lane);
+      nf32_ones_piece<GROUPS>(p, c, gnf32, lo, min(Tf32, lo + 4 * Cm), lane);
     }
   };
   const int total = st.ncf + st.ncm;
@@ -2218,6 +2260,8 @@ struct PairView {
   int e, a;     // env inside the tile, agent
   int u, m;     // node, budget
 };
+// (GROUPS: an absent agent's pair is not valid: no mask ones, no node_features one)
+template <int GROUPS = 0>
 __device__ __forceinline__ PairView pair_of(const Params& p, const int* s_pos, const int* s_money, int cm, int epc, int nEnv, int lane) {
   PairView v;
   const int A = p.A;
@@ -2226,6 +2270,7 @@ __device__ __forceinline__ PairView pair_of(const Params& p, const int* s_pos, c
   v.e = cm * epc + de;
   v.valid = de < epc && v.e < nEnv;
   v.u = v.valid ? s_pos[v.e * A + v.a] : 0;
+  if (GROUPS && v.u < 0) v.valid = false, v.u = 0;
   v.m = v.valid ? s_money[v.e * A + v.a] : 0;
   return v;
 }
@@ -2312,7 +2357,7 @@ __device__ __forceinline__ void fused_writer_role(const Params& p, unsigned char
     const BulkCtx c = ctx_of(k);
     if (item < st.ncf) {
       const int lo = item * p.wr_c_nf;
-      bulk_nf_ones<1>(p, c, img, lo, min(p.wr_c_nf, st.Tf - lo), lane, v != 0);
+      bulk_nf_ones<1, GROUPS>(p, c, img, lo, min(p.wr_c_nf, st.Tf - lo), lane, v != 0);
     } else {
       const int lo = (item - st.ncf) * Cm, len = min(Cm, st.Tm - lo);
       if (staged) bulk_mask_ones<true, GROUPS>(p, c, img, lo, len, lane, v);
@@ -2323,13 +2368,13 @@ __device__ __forceinline__ void fused_writer_role(const Params& p, unsigned char
     if (nf8) return;
     int* b = sbuf(k);
     if (fast) {
-      const PairView pv = pair_of(p, b, b + TILE * A, item, p.wr_epc, envs_of(k), lane);
+      const PairView pv = pair_of<GROUPS>(p, b, b + TILE * A, item, p.wr_epc, envs_of(k), lane);
       fast_nf32_ones(p, pv, b + 2 * TILE * A, gnf_of(k), lane);
     } else {
       const ImageStreams so = image_streams(p, tile_of(k) * TILE, envs_of(k));
       if (item >= so.ncf) {
         const int lo = 4 * (item - so.ncf) * Cm;
-        nf32_ones_piece(p, ctx_of(k), gnf_of(k), lo, min(4 * so.Tm, lo + 4 * Cm), lane);
+        nf32_ones_piece<GROUPS>(p, ctx_of(k), gnf_of(k), lo, min(4 * so.Tm, lo + 4 * Cm), lane);
       }
     }
   };
@@ -2413,7 +2458,7 @@ __device__ __forceinline__ void fused_writer_role(const Params& p, unsigned char
         static_assert(D == 2, "the image ring and the owed-ones ring are the same two chunks");
         if (pending == D && ring_fast[0]) {  // (after a tile-boundary flush the ring is short: clear the whole image)
           int* ob = sbuf(ring_k[0]);
-          const PairView pv = pair_of(p, ob, ob + TILE * A, ring_item[0], p.wr_epc, envs_of(ring_k[0]), lane);
+          const PairView pv = pair_of<GROUPS>(p, ob, ob + TILE * A, ring_item[0], p.wr_epc, envs_of(ring_k[0]), lane);
           fast_mask_ones<GROUPS>(p, pv, s_nbr4, s_rp, s_col, s_wgt, img, p.wr_epc, ring_item[0], 0);
         } else {
           for (int i = lane * 16; i < p.wr_img_bytes; i += 32 * 16) *reinterpret_cast<uint4*>(img + i) = make_uint4(0, 0, 0, 0);
@@ -2425,7 +2470,7 @@ __device__ __forceinline__ void fused_writer_role(const Params& p, unsigned char
       const int lo = is_nf8 ? item * p.wr_c_nf : (item - st.ncf) * Cm;
       const int len = is_nf8 ? min(p.wr_c_nf, st.Tf - lo) : min(Cm, st.Tm - lo);
       if (fast) {
-        const PairView pv = pair_of(p, sb, sb + TILE * A, item, p.wr_epc, nEnv, lane);
+        const PairView pv = pair_of<GROUPS>(p, sb, sb + TILE * A, item, p.wr_epc, nEnv, lane);
         fast_mask_ones<GROUPS>(p, pv, s_nbr4, s_rp, s_col, s_wgt, img, p.wr_epc, item, 1);
       } else {
         generic_img(k, item, st, img, 1);
@@ -2557,7 +2602,7 @@ __global__ void sy_count_unset_kernel(const uint8_t* mask, int B, int* unset) {
 // ---------------------------------------------------------------------------------------------
 // random valid policy: thread per (env, agent)
 // ---------------------------------------------------------------------------------------------
-// GROUPS: each env's moves are tested against its mechanism group's toll
+// GROUPS: each env's moves are tested against its mechanism group's toll; its absent agents get -1
 template <typename ActT, int GROUPS = 0>
 __global__ void __launch_bounds__(256) sy_sample_actions_kernel(const Params p, unsigned step_counter, ActT* actions,
                                                                 const unsigned* __restrict__ step_base) {
@@ -2565,6 +2610,10 @@ __global__ void __launch_bounds__(256) sy_sample_actions_kernel(const Params p, 
   const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;  // B * A < 2^31 (checked at sy_create)
   if (i >= (unsigned)p.B * (unsigned)p.A) return;
   const unsigned b = i / (unsigned)p.A, a = i - b * (unsigned)p.A;
+  if (agent_absent<GROUPS>(p, (int)b, (int)a)) {  // before any table lookup at its node (-1)
+    actions[i] = (ActT)-1;
+    return;
+  }
   const Tables& tb = p.tb;
   const int N = p.N;
   const int g = p.st.graph_id[b], u = p.st.pos[i], m = p.st.money[i];
@@ -4263,7 +4312,9 @@ int sy_set_groups(SyEnv* e, int32_t n, const SyGroup* groups, const int32_t* gro
     rows[g].agent_money = q.agent_money;
     rows[g].reveal = q.reveal_interval;
     rows[g].reveal_skip_thresh = q.reveal_skip_prob > 0.0f ? (unsigned long long)((double)fminf(q.reveal_skip_prob, 1.0f) * 4294967296.0) : 0ull;
-    rows[g].toll = e->cfg.toll;  // every group starts with the config's toll (sy_set_group_tolls changes it)
+    rows[g].toll = e->cfg.toll;  // every group starts with the config's toll (sy_set_group_tolls changes it) ...
+    rows[g].num_police = e->cfg.num_police;  // ... police count and horizon (sy_set_group_rules)
+    rows[g].max_t = e->cfg.max_timestep;
   }
   CUDA_TRY(cudaSetDevice(e->cfg.device));
   cudaStream_t s = (cudaStream_t)stream;
@@ -4318,6 +4369,32 @@ int sy_set_group_tolls(SyEnv* e, int32_t n, const int32_t* tolls, sy_stream_t st
     if (tolls[g] < 0 || tolls[g] > SY_MAX_TOLL) return fail(SY_ERR_INVALID_ARGUMENT, "group %d: toll %d outside [0, %d]", g, tolls[g], SY_MAX_TOLL);
   std::vector<GroupRow> rows = e->grp_rows;
   for (int g = 0; g < n; ++g) rows[g].toll = tolls[g];
+  CUDA_TRY(cudaSetDevice(e->cfg.device));
+  cudaStream_t s = (cudaStream_t)stream;
+  CUDA_TRY(cudaMemcpyAsync(e->d_grp, rows.data(), (size_t)n * sizeof(GroupRow), cudaMemcpyHostToDevice, s));
+  CUDA_TRY(cudaStreamSynchronize(s));  // (the host table is a local)
+  e->grp_rows = std::move(rows);
+  e->grp_need_reset = true;
+  return SY_OK;
+}
+
+int sy_set_group_rules(SyEnv* e, int32_t n, const int32_t* num_police, const int32_t* max_timestep, sy_stream_t stream) {
+  if (!e) return fail(SY_ERR_INVALID_ARGUMENT, "NULL env");
+  if (e->obs_pending) return fail(SY_ERR_STATE, "sy_set_group_rules: observations are pending (sy_flush_observations first)");
+  if (e->grp_n == 0) return fail(SY_ERR_STATE, "sy_set_group_rules: no mechanism groups are set (sy_set_groups first)");
+  if (n != e->grp_n) return fail(SY_ERR_INVALID_ARGUMENT, "sy_set_group_rules: num_groups %d, but the handle holds %d groups", n, e->grp_n);
+  const int P = e->cfg.num_police, T = e->cfg.max_timestep;
+  for (int g = 0; g < n; ++g) {
+    if (num_police && (num_police[g] < 1 || num_police[g] > P))
+      return fail(SY_ERR_INVALID_ARGUMENT, "group %d: num_police %d outside [1, %d]", g, num_police[g], P);
+    if (max_timestep && (max_timestep[g] < 0 || max_timestep[g] > T))
+      return fail(SY_ERR_INVALID_ARGUMENT, "group %d: max_timestep %d outside [0, %d]", g, max_timestep[g], T);
+  }
+  std::vector<GroupRow> rows = e->grp_rows;
+  for (int g = 0; g < n; ++g) {
+    rows[g].num_police = num_police ? num_police[g] : P;
+    rows[g].max_t = max_timestep ? max_timestep[g] : T;
+  }
   CUDA_TRY(cudaSetDevice(e->cfg.device));
   cudaStream_t s = (cudaStream_t)stream;
   CUDA_TRY(cudaMemcpyAsync(e->d_grp, rows.data(), (size_t)n * sizeof(GroupRow), cudaMemcpyHostToDevice, s));

@@ -12,7 +12,7 @@ device raises.
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, List, Optional, Sequence
+from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -36,26 +36,43 @@ MAX_MONEY_LIMIT = 1000  # yard.py:11
 N_EXP_TABLE = 1100  # exp(-d) underflows to 0 beyond d = 745
 
 
-MECHANISM_KEYS = ("reward_weights", "agent_money", "reveal_interval", "reveal_skip_prob", "tolls")
+MECHANISM_KEYS = ("reward_weights", "agent_money", "reveal_interval", "reveal_skip_prob", "tolls", "number_of_agents",
+                  "max_timestep")
+
+
+def _integral(name: str, v, lo: int, hi: int) -> int:
+    """`v` as an int in [lo, hi]: integral numbers (2.0 too) and 0-dim tensors, never bools"""
+    if isinstance(v, torch.Tensor):
+        v = v.item()
+    if isinstance(v, bool) or not isinstance(v, (int, float, np.integer, np.floating)) or not np.isfinite(v) \
+            or int(v) != v or not lo <= int(v) <= hi:
+        raise ValueError(f"{name} must be an integer in [{lo}, {hi}], got {v!r}")
+    return int(v)
 
 
 def mechanism_toll(mech: Dict, base) -> int:
     """The toll of one mechanism dict: its `tolls` (the constructor's rule: integral and >= 0, so 1.0 is accepted; at most
     SY_MAX_TOLL), else `base.tolls`.  Raises ValueError on what sy_set_group_tolls would refuse."""
-    toll = mech["tolls"] if "tolls" in mech else base.tolls
-    if isinstance(toll, torch.Tensor):
-        toll = toll.item()
-    if isinstance(toll, bool) or not isinstance(toll, (int, float, np.integer, np.floating)) or not np.isfinite(toll) \
-            or int(toll) != toll or not 0 <= int(toll) <= _cabi.SY_MAX_TOLL:
-        raise ValueError(f"tolls must be an integer in [0, {_cabi.SY_MAX_TOLL}], got {toll!r}")
-    return int(toll)
+    return _integral("tolls", mech["tolls"] if "tolls" in mech else base.tolls, 0, _cabi.SY_MAX_TOLL)
+
+
+def mechanism_rules(mech: Dict, base) -> Tuple[int, int]:
+    """(police count, episode horizon) of one mechanism dict: its `number_of_agents` (the number of POLICE, named as in
+    the constructor; the reference trainer's `num_police_agents: k` is an env with k + 1 police) in
+    [1, base.number_of_agents], and its `max_timestep` in [0, base.config.max_timestep]; a missing key takes `base`'s
+    value.  Raises ValueError on what sy_set_group_rules would refuse."""
+    top_p, top_t = base.number_of_agents, base.config.max_timestep
+    police = _integral("number_of_agents", mech["number_of_agents"], 1, top_p) if "number_of_agents" in mech else top_p
+    horizon = _integral("max_timestep", mech["max_timestep"], 0, top_t) if "max_timestep" in mech else top_t
+    return police, horizon
 
 
 def pack_mechanism(mech: Dict, base) -> "_cabi.SyGroup":
     """One mechanism dict (keys of MECHANISM_KEYS, all optional) as the SyGroup of sy_set_groups; missing keys and
     missing reward-weight names take `base`'s values (an env, or anything with `reward_weights`, `agent_money`,
     `reveal_interval` and `config.reveal_skip_prob`).  Raises ValueError / KeyError on what the library would refuse.
-    A `tolls` key is validated here (mechanism_toll) but travels separately, through sy_set_group_tolls."""
+    `tolls`, `number_of_agents` and `max_timestep` keys are validated here (mechanism_toll, mechanism_rules) but travel
+    separately, through sy_set_group_tolls / sy_set_group_rules."""
     if not isinstance(mech, dict):
         raise TypeError(f"a mechanism is a dict, got {type(mech).__name__}")
     unknown = set(mech) - set(MECHANISM_KEYS)
@@ -81,6 +98,8 @@ def pack_mechanism(mech: Dict, base) -> "_cabi.SyGroup":
         raise ValueError(f"reveal_skip_prob must be in [0, 1], got {skip}")
     if "tolls" in mech:
         mechanism_toll(mech, base)
+    if "number_of_agents" in mech or "max_timestep" in mech:
+        mechanism_rules(mech, base)
     g = _cabi.SyGroup()
     g.struct_bytes = C.sizeof(_cabi.SyGroup)
     for i, v in enumerate(w):
@@ -89,25 +108,29 @@ def pack_mechanism(mech: Dict, base) -> "_cabi.SyGroup":
     return g
 
 
-def unpack_mechanism(g: "_cabi.SyGroup", tolls: Optional[int] = None) -> Dict:
-    """The complete mechanism dict of a SyGroup (float weights), with `tolls` when given"""
+def unpack_mechanism(g: "_cabi.SyGroup", tolls: Optional[int] = None, rules: Optional[Tuple[int, int]] = None) -> Dict:
+    """The complete mechanism dict of a SyGroup (float weights), with `tolls` and (`rules` = (police, horizon))
+    `number_of_agents` / `max_timestep` when given"""
     d = dict(reward_weights={k: float(g.reward_weights[i]) for i, k in enumerate(REWARD_WEIGHT_NAMES)},
              agent_money=int(g.agent_money), reveal_interval=int(g.reveal_interval),
              reveal_skip_prob=float(g.reveal_skip_prob))
     if tolls is not None:
         d["tolls"] = int(tolls)
+    if rules is not None:
+        d["number_of_agents"], d["max_timestep"] = int(rules[0]), int(rules[1])
     return d
 
 
 def group_metrics(per: Sequence[Dict], mechanisms: Sequence[Dict], number_of_agents: int):
     """What metrics() needs while mechanism groups are set, from the per-group statistics `per` (stats(by_group=True))
-    and the mechanism dicts: (efficiency sum, tolls paid, per-group metrics).  A group's budget efficiency uses its own agent_money and its
-    mean_tolls_paid its own toll; the aggregate weighs every group against its own budget and sums the tolls paid as
-    the integer sum over groups of toll * police_moves (divided once: groups with the constructor's toll give exactly
-    the float of a handle without groups)."""
-    by_group = [metrics_of(g, initial=max(number_of_agents * m["agent_money"], 1), tolls_paid=m["tolls"] * g["police_moves"])
-                for g, m in zip(per, mechanisms)]
-    eff = sum(g["sum_episode_budget_spent"] / max(number_of_agents * m["agent_money"], 1) for g, m in zip(per, mechanisms))
+    and the mechanism dicts: (efficiency sum, tolls paid, per-group metrics).  A group's budget efficiency uses its own
+    police budget P_g * agent_money_g (P_g = its `number_of_agents`, else `number_of_agents`) and its mean_tolls_paid
+    its own toll; the aggregate weighs every group against its own budget and sums the tolls paid as the integer sum
+    over groups of toll * police_moves (divided once: groups with the constructor's toll give exactly the float of a
+    handle without groups)."""
+    budgets = [max(int(m.get("number_of_agents", number_of_agents)) * m["agent_money"], 1) for m in mechanisms]
+    by_group = [metrics_of(g, initial=b, tolls_paid=m["tolls"] * g["police_moves"]) for g, m, b in zip(per, mechanisms, budgets)]
+    eff = sum(g["sum_episode_budget_spent"] / b for g, b in zip(per, budgets))
     paid = sum(int(m["tolls"]) * int(g["police_moves"]) for g, m in zip(per, mechanisms))
     return eff, paid, by_group
 
@@ -311,6 +334,7 @@ class BatchedScotlandYardEnv:
         self._need_full_reset = False
         self._mechanisms, self._group_id, self.group_stats_vec = None, None, None  # set_mechanisms
         self._env_toll = None  # int32 [B, 1] while some mechanism group's toll differs from `tolls`
+        self._env_police = None  # int32 [B, 1] while some mechanism group's police count differs from number_of_agents
         self._groups_generation = 0  # set_mechanisms calls: captured rollout graphs check it
 
     # ------------------------------------------------------------------ plumbing
@@ -410,8 +434,12 @@ class BatchedScotlandYardEnv:
         gi = None if graph_id is None else self._dev(graph_id, torch.int32, (B,))
         if gi is not None and (int(gi.min()) < 0 or int(gi.max()) >= self.num_graphs):
             raise ValueError("graph_id out of range")
-        if ip is not None and (int(ip.min()) < 0 or int(ip.max()) >= self.graph_nodes):
-            raise ValueError("init_pos out of range")
+        if ip is not None:
+            # (agents beyond a mechanism group's police count are absent: their entries are ignored)
+            live = ip if self._env_police is None else \
+                ip[torch.arange(A, device=self.device).view(1, -1) <= self._env_police]
+            if live.numel() and (int(live.min()) < 0 or int(live.max()) >= self.graph_nodes):
+                raise ValueError("init_pos out of range")
         if restart is None:
             restart = not self._is_reset
         if not self._is_reset and m is not None:
@@ -482,33 +510,48 @@ class BatchedScotlandYardEnv:
     def set_mechanisms(self, mechanisms, group_id=None):
         """Evaluate several mechanisms in this one batch (sy_set_groups).  `mechanisms`: a sequence of dicts with the
         optional keys `reward_weights` (a dict keyed by REWARD_WEIGHT_NAMES, floats or 0-dim tensors; missing names keep
-        the constructor's weight), `agent_money`, `reveal_interval`, `reveal_skip_prob` and `tolls` (a missing key keeps
-        the constructor's value).  `group_id`: int tensor [B] (env -> index into `mechanisms`), or None for
+        the constructor's weight), `agent_money`, `reveal_interval`, `reveal_skip_prob`, `tolls`, `number_of_agents` and
+        `max_timestep` (a missing key keeps the constructor's value).  `number_of_agents` is the group's number of POLICE
+        in [1, number_of_agents] -- the reference trainer's `num_police_agents: k` (agent_configurations) plays k + 1
+        police, so that entry is `number_of_agents=k + 1` -- and `max_timestep` its horizon in [0, max_timestep].  An env
+        of a group with fewer police keeps the [B, A] layout; its agents past the group's police are absent (pos -1,
+        budget 0, reward 0, all-zero mask row and node_features column, sampled action -1; include/sy_env.h, SyState).
+        `group_id`: int tensor [B] (env -> index into `mechanisms`), or None for
         (env_offset + b) % len(mechanisms).  `mechanisms=None` clears the groups.  Pending observations are flushed
         first; the new mechanisms take effect at the next full `reset()`, which `step` and the rollouts require."""
         self.flush_observations()
         if mechanisms is None:
-            table, tolls, gid = [], [], None
+            table, tolls, rules, gid = [], [], [], None
         else:
             table = [pack_mechanism(m, self) for m in mechanisms]
             tolls = [mechanism_toll(m, self) for m in mechanisms]
+            rules = [mechanism_rules(m, self) for m in mechanisms]
             if not 1 <= len(table) <= _cabi.SY_MAX_GROUPS:
                 raise ValueError(f"between 1 and {_cabi.SY_MAX_GROUPS} mechanisms, got {len(table)}")
             gid = None if group_id is None else self._dev(group_id, torch.int32, (self.num_envs,))
         arr = (_cabi.SyGroup * max(len(table), 1))(*table)
         own_tolls = any(t != self.tolls for t in tolls)
+        police, horizon = [r[0] for r in rules], [r[1] for r in rules]
+        own_police = any(n != self.number_of_agents for n in police)
+        own_rules = own_police or any(t != self.config.max_timestep for t in horizon)
         with torch.cuda.device(self.device):
             _cabi.check(self._lib.sy_set_groups(self._handle, len(table), arr, _ptr(gid), self._stream()))
-            if own_tolls:  # (sy_set_groups gave every group the constructor's toll)
+            if own_tolls:  # (sy_set_groups gave every group the constructor's toll, police count and horizon)
                 _cabi.check(self._lib.sy_set_group_tolls(self._handle, len(tolls), (C.c_int32 * len(tolls))(*tolls),
                                                          self._stream()))
-        self._mechanisms = None if mechanisms is None else tuple(unpack_mechanism(g, t) for g, t in zip(table, tolls))
-        self._group_id, self._env_toll = None, None
+            if own_rules:
+                _cabi.check(self._lib.sy_set_group_rules(self._handle, len(rules), (C.c_int32 * len(rules))(*police),
+                                                         (C.c_int32 * len(rules))(*horizon), self._stream()))
+        self._mechanisms = None if mechanisms is None else tuple(
+            unpack_mechanism(g, t, r) for g, t, r in zip(table, tolls, rules))
+        self._group_id, self._env_toll, self._env_police = None, None, None
         if table:
             self._group_id = gid.clone() if gid is not None else (
                 (torch.arange(self.num_envs, device=self.device, dtype=torch.int64) + self.env_offset) % len(table)).to(torch.int32)
             if own_tolls:  # int32 [B, 1] toll of each env (the policies' legality test, see policy._PolicyBase._state)
                 self._env_toll = torch.tensor(tolls, dtype=torch.int32, device=self.device)[self._group_id.long()].view(-1, 1)
+            if own_police:  # int32 [B, 1] police count of each env (init_pos checks, the policies' refusal)
+                self._env_police = torch.tensor(police, dtype=torch.int32, device=self.device)[self._group_id.long()].view(-1, 1)
         self.group_stats_vec = torch.zeros(len(table), _cabi.SY_NUM_STATS, dtype=torch.int64, device=self.device) \
             if table and self.stats_vec is not None else None
         self._need_full_reset = True  # the next reset() covers every env

@@ -84,6 +84,15 @@ class _PolicyBase:
             self._tables = _GraphTables(self.env)
         return self._tables.struct
 
+    def _refuse_mixed_police(self):
+        """Raise ValueError (before anything is launched) while some mechanism group's police count differs from the
+        env's: the GNN's feature width and MAPPO's per-agent actors depend on the police count, and the policy kernels
+        index with every agent's pos, so mixed police counts need one handle (and model) per count, as the reference
+        trainer builds them."""
+        if self.env._env_police is not None:
+            raise ValueError("mechanism groups with their own number_of_agents: the policies need one handle per police "
+                             "count (set every group's number_of_agents to the env's)")
+
     def _state(self) -> pc.SyPolicyState:
         e = self.env
         s = pc.SyPolicyState()
@@ -168,6 +177,7 @@ class GNNPolicy(_PolicyBase):
 
     def q_values(self) -> torch.Tensor:
         """float32 [B, 2, N]: GNNModel.forward of MrX's model ([:, 0]) and the police model ([:, 1]) per env."""
+        self._refuse_mixed_police()
         e = self.env
         q = torch.empty(e.num_envs, 2, e.graph_nodes, dtype=torch.float32, device=e.device)
         with torch.cuda.device(e.device):
@@ -178,6 +188,7 @@ class GNNPolicy(_PolicyBase):
     def act(self, epsilon_mrx: float = 0.0, epsilon_police: Optional[float] = None, step_counter: Optional[int] = None,
             out: Optional[torch.Tensor] = None, return_q: bool = False):
         """int64 [B, A] actions (epsilon-greedy over the valid moves, -1 without one); optionally the chosen Q."""
+        self._refuse_mixed_police()
         e = self.env
         if step_counter is None:
             step_counter = self.step_counter
@@ -266,6 +277,7 @@ class MappoPolicy(_PolicyBase):
         obs=None: the kernel builds MappoTrainer's own observations from the env state (mappo_trainer.py:171-199: MrX
         sees his node, every officer the officers' nodes; raw node ids, zero-padded to obs_size >= P) without any
         observation tensor being materialised."""
+        self._refuse_mixed_police()
         e = self.env
         if obs is None:
             if self.obs_size < e.number_of_agents:

@@ -9,8 +9,15 @@ Writes profiles/r03_mechanisms_c{2,3}.json (or --out-dir) with the card's name a
 g % 4), timed the same way; writes profiles/r04_group_tolls_c{2,3}.json.  Other tolls change the games themselves (which
 moves are legal, how long episodes last), so that variant does not do exactly the same game work.
 
-    python tools/bench_mechanisms.py [--workloads c3,c2] [--steps 50] [--passes 5] [--tolls]
+--rules (opt-in): no groups, the same 16 groups, and those 16 groups with `number_of_agents` / `max_timestep` given
+explicitly through sy_set_group_rules with the handle's own values (the same game work: any difference is the cost of
+the per-env police count and horizon), timed the same way; plus, for information, the 16 groups with police counts
+cycling P, P-1, ..., 1 (group g plays P - g % P police: less game work per env, different games).  Writes
+profiles/r05_group_rules_c{2,3}.json.
+
+    python tools/bench_mechanisms.py [--workloads c3,c2] [--steps 50] [--passes 5] [--tolls | --rules]
 """
+import ctypes as C
 import argparse
 import json
 import os
@@ -27,6 +34,7 @@ WORKLOADS = {  # bench.py's c2 / c3 (c3 with the belief scored at reveals)
 }
 VARIANTS = ["no_groups", "one_group_equal", "groups_16", "groups_1024"]
 TOLL_VARIANTS = ["no_groups", "groups_16", "groups_16_tolls"]
+RULE_VARIANTS = ["no_groups", "groups_16", "groups_16_rules", "groups_16_police"]
 
 
 def card():
@@ -54,7 +62,7 @@ def run(wl_name, steps, passes, variants=VARIANTS):
                                      reveal_interval=wl["reveal"], auto_reset=True, device="cuda:0")
         if v == "one_group_equal":
             env.set_mechanisms([{}])
-        elif v in ("groups_16", "groups_1024", "groups_16_tolls"):
+        elif v in ("groups_16", "groups_1024", "groups_16_tolls", "groups_16_rules", "groups_16_police"):
             # distinct mechanisms with the config's budget and reveal schedule: only the reward weights differ, so
             # every variant does the same game work and the difference is the cost of the groups themselves
             n = 1024 if v == "groups_1024" else 16
@@ -63,7 +71,14 @@ def run(wl_name, steps, passes, variants=VARIANTS):
             if v == "groups_16_tolls":
                 for g, m in enumerate(mechs):
                     m["tolls"] = g % 4
+            if v == "groups_16_police":
+                for g, m in enumerate(mechs):
+                    m["number_of_agents"] = wl["P"] - g % wl["P"]
             env.set_mechanisms(mechs)
+            if v == "groups_16_rules":  # the handle's values, explicitly (set_mechanisms only calls when one differs)
+                arr = lambda x: (C.c_int32 * n)(*([x] * n))  # noqa: E731
+                rc = env._lib.sy_set_group_rules(env._handle, n, arr(wl["P"]), arr(env.config.max_timestep), env._stream())
+                assert rc == 0, rc
         env.reset()
         acts = env.sample_actions(step_counter=0)
         graph, _ = env.capture_rollout(steps)
@@ -103,7 +118,7 @@ def run(wl_name, steps, passes, variants=VARIANTS):
     for v in variants[1:]:
         for k in ("sy_step_ms", "graph_replay_ms"):
             out[v][k + "_vs_no_groups"] = out[v][k] / base[k] - 1.0
-            if v == "groups_16_tolls":
+            if v in ("groups_16_tolls", "groups_16_rules", "groups_16_police"):
                 out[v][k + "_vs_groups_16"] = out[v][k] / out["groups_16"][k] - 1.0
     for env, _, _ in envs.values():
         env.close()
@@ -117,6 +132,7 @@ def main():
     ap.add_argument("--passes", type=int, default=5)
     ap.add_argument("--out-dir", default=os.path.join(ROOT, "profiles"))
     ap.add_argument("--tolls", action="store_true", help="16 groups with and without their own tolls (r04 profiles)")
+    ap.add_argument("--rules", action="store_true", help="16 groups with the police count / horizon machinery (r05 profiles)")
     args = ap.parse_args()
     import torch
 
@@ -131,9 +147,15 @@ def main():
         if args.tolls:
             note += (f"; groups_16_tolls: group g pays toll g % 4 (config toll {WORKLOADS[w]['toll']}), so its games "
                      "differ from the other variants'")
+        if args.rules:
+            note += (f"; groups_16_rules: the 16 groups with number_of_agents = {WORKLOADS[w]['P']} and max_timestep = 250 "
+                     "given through sy_set_group_rules (same games as groups_16); groups_16_police (information only): "
+                     f"group g plays {WORKLOADS[w]['P']} - g % {WORKLOADS[w]['P']} police, so its games differ")
+        variants = TOLL_VARIANTS if args.tolls else (RULE_VARIANTS if args.rules else VARIANTS)
         res = dict(workload=w, config=WORKLOADS[w], steps_per_pass=args.steps, passes=args.passes, card=info, note=note,
-                   variants=run(w, args.steps, args.passes, TOLL_VARIANTS if args.tolls else VARIANTS))
-        path = os.path.join(args.out_dir, f"r04_group_tolls_{w}.json" if args.tolls else f"r03_mechanisms_{w}.json")
+                   variants=run(w, args.steps, args.passes, variants))
+        name = "r04_group_tolls" if args.tolls else ("r05_group_rules" if args.rules else "r03_mechanisms")
+        path = os.path.join(args.out_dir, f"{name}_{w}.json")
         with open(path, "w") as f:
             json.dump(res, f, indent=1)
         print(json.dumps(res))
