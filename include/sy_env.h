@@ -89,9 +89,9 @@ typedef struct SyConfig {
   int32_t num_police;      /* P  (number_of_agents, yard.py:33) */
   int32_t agent_money;     /* yard.py:42,117-119 */
   int32_t mrx_money;       /* MAX_MONEY_LIMIT = 1000, yard.py:11 */
-  int32_t max_timestep;    /* 250, reward_calculator.py:68 */
+  int32_t max_timestep;    /* 250, reward_calculator.py:68; in [0, SY_MAX_TIMESTEP] */
   int32_t reveal_interval; /* 0 = MrX always visible (reference behaviour) */
-  int32_t toll;            /* 0 = reference behaviour; else legality and police charge use w + toll */
+  int32_t toll;            /* 0 = reference behaviour; else legality and police charge use w + toll; in [0, SY_MAX_TOLL] */
   int32_t belief;          /* 0 off | 1 maintain belief_map | SY_BELIEF_SCORED (2): also score it at reveal steps */
   int32_t reward_mode;     /* SY_REWARD_FP64 (python-float weights) | SY_REWARD_FP32 (0-dim fp32 tensors) */
   int32_t auto_reset;      /* 0/1: same-step auto-reset of finished envs (Philox start nodes) */
@@ -106,6 +106,12 @@ typedef struct SyConfig {
   float reveal_skip_prob;
   int32_t reserved0;
 } SyConfig;
+/* Bounds sy_create enforces (sy_set_group_tolls / sy_set_group_rules hold groups to the same ones).
+ * SY_MAX_TIMESTEP: an episode lasts at most max_timestep + 2 steps (the visit counters are incremented before the
+ * timeout test), so a police that never moves counts at most 65 535 visits, exactly what the u16 counters hold.
+ * SY_MAX_TOLL (below): with edge weights <= 255, w + toll and a step's police charges stay far inside int32.
+ * The episode statistics sum the squared lengths and the budget spent per episode (up to 15 x (2^31 - 1)) in 64 bits. */
+#define SY_MAX_TIMESTEP 65533
 
 /* Every pointer struct below starts with `struct_bytes` = sizeof(the struct): the library rejects a struct of another
  * size with SY_ERR_INVALID_ARGUMENT instead of reading past the caller's memory (a binding written against an older
@@ -369,8 +375,9 @@ typedef struct SyGroup {
 int sy_set_groups(SyEnv* env, int32_t num_groups, const SyGroup* groups, const int32_t* group_id, sy_stream_t stream);
 /* Per-group tolls: an env pays its group's toll instead of SyConfig.toll -- a move is legal iff w + toll <= budget (MrX and
  * police; action_mask, the random sampler and the mobility term of the rewards follow the same rule), and a police move
- * costs w + toll.  tolls: HOST int32 [num_groups], each in [0, SY_MAX_TOLL] (with edge weights <= 255, w + toll and the
- * per-step sums of the police charges cannot overflow an int32); num_groups must be the number set by sy_set_groups.
+ * costs w + toll.  tolls: HOST int32 [num_groups], each in [0, SY_MAX_TOLL] (the bound of SyConfig.toll: with edge
+ * weights <= 255, w + toll and the per-step sums of the police charges cannot overflow an int32); num_groups must be the
+ * number set by sy_set_groups.
  * A rejected call keeps the previous tolls.  Like sy_set_groups: fails with SY_ERR_STATE while observations are pending
  * (or when no groups are set), and the new tolls take effect at the next sy_reset of every env, which the step and
  * rollout entry points require until then.  A CUDA graph captured before the call must be captured again.  Synchronises

@@ -718,35 +718,53 @@ def philox_random_valid_action(seed, env, step, agent, moves: np.ndarray) -> int
     return int(moves[(r * len(moves)) >> 32])
 
 
+SY_NUM_STATS = 16  # include/sy_env.h: the statistics vector of sy_stats / sy_group_stats
+(STAT_ENV_STEPS, STAT_EPISODES, STAT_MRX_WINS, STAT_POLICE_WINS, STAT_TRUNCATIONS, STAT_OUT_OF_MONEY, STAT_SUM_LENGTH,
+ STAT_SUM_BUDGET_SPENT, STAT_SUM_SQ_LENGTH, STAT_SUM_LENGTH_POLICE_WINS, STAT_SUM_LENGTH_MRX_WINS,
+ STAT_SUM_EPISODE_BUDGET_SPENT, STAT_POLICE_MOVES, STAT_REVEALS) = range(14)
+
+
 class OracleBatch:
     """B independent OracleEnv with the batched env's conventions: graph pool + graph_id,
     same-step auto-reset keyed by Philox(seed; global env index, episode)."""
 
     def __init__(self, cfg: OracleConfig, graphs: List[Graph], graph_id, start_positions, seed=0,
-                 auto_reset=False, env_offset=0, resample_graph=False):
+                 auto_reset=False, env_offset=0, resample_graph=False, groups=None):
+        """groups: (cfgs, group_id) of an OracleGroupBatch; None = every env runs `cfg`"""
         self.cfg, self.graphs, self.seed = cfg, graphs, int(seed)
         self.auto_reset, self.env_offset, self.resample_graph = auto_reset, env_offset, resample_graph
         self.graph_id = [int(g) for g in graph_id]
-        self.envs = [OracleEnv(cfg, graphs[g], sp) for g, sp in zip(self.graph_id, start_positions)]
+        self.cfgs, self.group = (list(groups[0]), [int(g) for g in groups[1]]) if groups else ([cfg], [0] * len(self.graph_id))
+        self.A = cfg.num_police + 1
+        self.envs = [OracleEnv(self.cfgs[gr], graphs[g], list(sp)[: self.cfgs[gr].num_police + 1])
+                     for g, gr, sp in zip(self.graph_id, self.group, start_positions)]
         self.episode = [0] * len(self.envs)
         self.done = [False] * len(self.envs)
+        # (length, winner, budget spent, truncated, group) of every finished episode
         self.finished = []
         self.belief_ces = []  # cross-entropies at reveal steps (not scored when the same step auto-resets the env)
+        self.ce_groups = []  # the group of each entry of belief_ces
+        self.step_stats = [[0, 0, 0] for _ in self.cfgs]  # per group: env steps, budget spent, police moves
 
     @classmethod
     def from_seed(cls, cfg, graphs, num_envs, seed=0, env_offset=0, auto_reset=True, resample_graph=False):
+        gid, sp = cls._seeded_starts(cfg.num_police + 1, graphs, num_envs, seed, env_offset, resample_graph)
+        return cls(cfg, graphs, gid, sp, seed, auto_reset, env_offset, resample_graph)
+
+    @staticmethod
+    def _seeded_starts(A, graphs, num_envs, seed, env_offset, resample_graph):
         N = graphs[0].num_nodes
         gid, sp = [], []
         for b in range(num_envs):
             e = env_offset + b
             g = philox_graph_choice(seed, e, 0, len(graphs)) if resample_graph else (e // 32) % len(graphs)  # blocks of 32 envs
             gid.append(g)
-            sp.append(philox_start_positions(seed, e, 0, N, cfg.num_police + 1))
-        return cls(cfg, graphs, gid, sp, seed, auto_reset, env_offset, resample_graph)
+            sp.append(philox_start_positions(seed, e, 0, N, A))
+        return gid, sp
 
     def _skip_draw(self, b):
         """the device's draw: skip iff Philox(seed; global env, t, RNG_REVEAL_SKIP, episode)[0] < float32(p) * 2^32"""
-        p = float(np.float32(self.cfg.reveal_skip_prob))
+        p = float(np.float32(self.envs[b].cfg.reveal_skip_prob))
         if p <= 0.0:
             return None
         thresh = int(min(p, 1.0) * 4294967296.0)
@@ -757,7 +775,7 @@ class OracleBatch:
         """actions int [B, A] (-1 == None); hints: optional bool/uint8 [B, N] observation hints (belief_module.py:
         102-106).  Returns dict of arrays for this step, then applies the same-step auto-reset (observations afterwards
         describe the fresh episode)."""
-        B, A = len(self.envs), self.cfg.num_police + 1
+        B, A = len(self.envs), self.A
         f = np.float32 if self.cfg.reward_mode == "fp32" else np.float64
         out = dict(
             reward=np.zeros((B, A), dtype=f),
@@ -769,39 +787,81 @@ class OracleBatch:
             if self.done[b]:  # frozen until reset (no auto-reset): zero reward, flags stay
                 continue
             hint = None if hints is None else [int(j) for j in np.nonzero(np.asarray(hints[b]))[0]]
-            r, te, tr, win = env.step([int(x) for x in actions[b]], hint=hint, skip_reveal=self._skip_draw(b))
-            out["reward"][b] = r
+            money0, moves0 = sum(env.money[1:]), env.moves
+            r, te, tr, win = env.step([int(x) for x in actions[b][: env.A]], hint=hint, skip_reveal=self._skip_draw(b))
+            out["reward"][b, : env.A] = r
             out["terminated"][b], out["truncated"][b], out["winner"][b] = te, tr, win
+            gs = self.step_stats[self.group[b]]
+            gs[0] += 1
+            gs[1] += money0 - sum(env.money[1:])
+            gs[2] += env.moves - moves0
             if env.last_ce is not None and not ((te or tr) and self.auto_reset):
                 self.belief_ces.append(env.last_ce)
+                self.ce_groups.append(self.group[b])
             if te or tr:
                 # (episode length, winner, budget spent) of the finished episode: what metrics.py:EpisodeMetrics records
-                self.finished.append((env.t, int(win), self.cfg.num_police * self.cfg.agent_money - sum(env.money[1:])))
+                spent = env.cfg.num_police * env.cfg.agent_money - sum(env.money[1:])
+                self.finished.append((env.t, int(win), spent, int(tr), self.group[b]))
                 if self.auto_reset:
                     self.episode[b] += 1
                     e = self.env_offset + b
                     if self.resample_graph:
                         self.graph_id[b] = philox_graph_choice(self.seed, e, self.episode[b], len(self.graphs))
-                    sp = philox_start_positions(self.seed, e, self.episode[b], env.N, A)
+                    sp = philox_start_positions(self.seed, e, self.episode[b], env.N, env.A)
                     env.reset(self.graphs[self.graph_id[b]], sp)
                 else:
                     self.done[b] = True
         return out
 
+    def expected_stats(self):
+        """(total, per_group): the statistics vectors of sy_stats and sy_group_stats (include/sy_env.h SY_STAT_*) as
+        Python ints, from the finished episodes and the per-step counts.  Entries 0..12 are exact; entry 13 counts the
+        scored reveals (what the device counts with belief scoring on); 14 and 15, the device's float32 cross-entropy
+        sums, are left None (compare them with a tolerance against belief_ces)."""
+        per = [[0] * SY_NUM_STATS for _ in self.cfgs]
+        for g, (n, spent, moves) in enumerate(self.step_stats):
+            per[g][STAT_ENV_STEPS], per[g][STAT_SUM_BUDGET_SPENT], per[g][STAT_POLICE_MOVES] = n, spent, moves
+        for length, win, spent, trunc, g in self.finished:
+            v = per[g]
+            v[STAT_EPISODES] += 1
+            v[STAT_SUM_LENGTH] += length
+            v[STAT_SUM_SQ_LENGTH] += length * length
+            v[STAT_SUM_EPISODE_BUDGET_SPENT] += spent
+            if win == WINNER_POLICE:
+                v[STAT_POLICE_WINS] += 1
+                v[STAT_SUM_LENGTH_POLICE_WINS] += length
+            else:
+                v[STAT_MRX_WINS] += 1
+                v[STAT_SUM_LENGTH_MRX_WINS] += length
+                v[STAT_TRUNCATIONS if trunc else STAT_OUT_OF_MONEY] += 1
+        for g in self.ce_groups:
+            per[g][STAT_REVEALS] += 1
+        for v in per:
+            v[14] = v[15] = None
+        total = [sum(v[k] for v in per) for k in range(14)] + [None, None]
+        return total, per
+
     def sample_actions(self, step) -> np.ndarray:
-        B, A = len(self.envs), self.cfg.num_police + 1
+        B, A = len(self.envs), self.A
         acts = np.full((B, A), DEFAULT_ACTION, dtype=np.int64)
         for b, env in enumerate(self.envs):
-            for a in range(A):
+            for a in range(env.A):
                 acts[b, a] = philox_random_valid_action(self.seed, self.env_offset + b, step, a, env.possible_moves(a))
         return acts
 
-    # state views shaped like the device arrays
+    # state views shaped like the device arrays (the agents past an env's police count carry the absent values of
+    # include/sy_env.h: pos -1, money 0, all-zero mask rows and node_features columns)
+    def _padded(self, rows, fill, dtype):
+        out = np.full((len(self.envs), self.A) + np.shape(rows[0])[1:], fill, dtype=dtype)
+        for b, r in enumerate(rows):
+            out[b, : len(r)] = r
+        return out
+
     def pos(self):
-        return np.asarray([e.pos for e in self.envs], dtype=np.int32)
+        return self._padded([e.pos for e in self.envs], -1, np.int32)
 
     def money(self):
-        return np.asarray([e.money for e in self.envs], dtype=np.int32)
+        return self._padded([e.money for e in self.envs], 0, np.int32)
 
     def timestep(self):
         return np.asarray([e.t for e in self.envs], dtype=np.int32)
@@ -810,13 +870,38 @@ class OracleBatch:
         return np.stack([e.visits for e in self.envs]).astype(np.uint16)
 
     def masks(self):
-        return np.stack([e.action_masks() for e in self.envs])
+        return self._padded([e.action_masks() for e in self.envs], False, bool)
 
     def node_features(self):
-        return np.stack([e.node_features() for e in self.envs])
+        return self._padded([e.node_features().T for e in self.envs], 0, np.float32).transpose(0, 2, 1).copy()
 
     def belief(self):
         return np.stack([e.belief for e in self.envs])
 
     def revealed(self):
         return np.asarray([e.revealed for e in self.envs], dtype=np.int32)
+
+
+class OracleGroupBatch(OracleBatch):
+    """A batch of mechanism groups with the conventions of a handle with groups (include/sy_env.h, sy_set_groups,
+    sy_set_group_tolls, sy_set_group_rules): env b runs OracleEnv(cfgs[group_id[b]]) -- that group's police count,
+    horizon, police budget, toll, reveal schedule and reward weights -- inside the handle's layout of A = num_police + 1
+    agents.  Its start nodes are the first P_g + 1 draws of philox_start_positions, its reveal-skip draw uses its
+    group's probability, its absent agents carry the absent values in every view and -1 from sample_actions, and its
+    finished episodes and statistics are recorded with its group.  The handle-wide settings (reward mode, MrX budget,
+    belief) come from each cfg and must agree."""
+
+    def __init__(self, cfgs: Sequence[OracleConfig], group_id, num_police: int, graphs: List[Graph], graph_id,
+                 start_positions, seed=0, auto_reset=False, env_offset=0, resample_graph=False):
+        for c in cfgs:
+            assert 1 <= c.num_police <= num_police, "a group plays with 1 .. num_police police"
+            assert (c.reward_mode, c.mrx_money, c.belief) == (cfgs[0].reward_mode, cfgs[0].mrx_money, cfgs[0].belief)
+        handle = OracleConfig(num_police=num_police, agent_money=0, reward_mode=cfgs[0].reward_mode)
+        super().__init__(handle, graphs, graph_id, start_positions, seed, auto_reset, env_offset, resample_graph,
+                         groups=(cfgs, group_id))
+
+    @classmethod
+    def from_seed(cls, cfgs, group_id, num_police, graphs, num_envs, seed=0, env_offset=0, auto_reset=True,
+                  resample_graph=False):
+        gid, sp = cls._seeded_starts(num_police + 1, graphs, num_envs, seed, env_offset, resample_graph)
+        return cls(cfgs, group_id, num_police, graphs, gid, sp, seed, auto_reset, env_offset, resample_graph)

@@ -15,6 +15,8 @@ SY_MAX_AGENTS = 16
 SY_NUM_STATS = 16
 SY_MAX_GROUPS = 1024
 SY_MAX_TOLL = 1048576
+SY_MAX_TIMESTEP = 65533
+INT32_MAX = 2 ** 31 - 1
 SY_REWARD_FP64, SY_REWARD_FP32 = 0, 1
 STAT_NAMES = [
     "env_steps", "episodes", "mrx_wins", "police_wins", "truncations", "out_of_money",

@@ -359,6 +359,12 @@ __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepc
 __device__ __forceinline__ void named_barrier(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;\n" ::"r"(id), "r"(nthreads) : "memory");
 }
+// sum of `v` over the lanes of `mask`, exact for values below 2^43 per lane: two 32-bit reductions, of the low 16 bits
+// (sum < 2^21) and of the rest (sum < 2^32)
+__device__ __forceinline__ unsigned long long warp_sum_u64(unsigned mask, unsigned long long v) {
+  const unsigned lo = __reduce_add_sync(mask, (unsigned)(v & 0xFFFFu)), hi = __reduce_add_sync(mask, (unsigned)(v >> 16));
+  return ((unsigned long long)hi << 16) + lo;
+}
 
 // bulk asynchronous copy shared -> global (TMA, SASS UBLKCP): one thread moves a whole image; the store stream never
 // touches the LSU or a register.  Source / destination 16-byte aligned, size a multiple of 16.
@@ -638,7 +644,8 @@ struct LogicSmem {
   int reset_gid[32];
   int t[32], gid[32], episode[32], frozen[32], status[32];
   int t_new[32], done[32], bel[32], revealed[32], clear[32];
-  int ep_spent[32], spent[32], moves[32];  // statistics inputs handed from warp 0 to the statistics warp
+  long long ep_spent[32];  // statistics inputs handed from warp 0 to the statistics warp
+  int spent[32], moves[32];
   int cnt_staged;
 };
 
@@ -853,7 +860,7 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
     }
   } else {
     // timestep, reveal schedule, same-step auto-reset, statistics
-    int ep_spent = 0;
+    long long ep_spent = 0;
     int t_new = t, done = frozen, bel = BEL_KEEP, revealed = -1, episode = sm.episode[lane], gnew = g;
     bool clear_visits = false;
     if (live) {
@@ -863,7 +870,7 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
         bel = BEL_PROPAGATE;
         if (status != ST_RUNNING) {
           const int agent_money = GROUPS ? __ldg(&gr->agent_money) : p.agent_money;
-          ep_spent = P * agent_money;  // every police starts an episode with agent_money (yard.py:117-119)
+          ep_spent = (long long)P * agent_money;  // every police starts an episode with agent_money (yard.py:117-119)
           for (int i = 1; i <= P; ++i) ep_spent -= money[i];
           if (p.auto_reset) {  // same-step auto-reset: the observation describes the fresh episode
             episode += 1;
@@ -911,22 +918,28 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
   if (warp == LOGIC_WARPS - 1 && p.out.stats) {
     const int st = sm.status[lane];
     const bool fin = active && st != ST_RUNNING;
+    // Sums over 32 lanes.  The squared length (< 2^32 with max_timestep <= SY_MAX_TIMESTEP) and the budget spent in the
+    // episode (<= 15 x (2^31 - 1)) are summed in 64 bits; every other sum stays below 2^31 in int: counts <= 32,
+    // lengths <= 32 x (SY_MAX_TIMESTEP + 2) < 2^22, a step's police charges <= 32 x 15 x (255 + SY_MAX_TOLL) < 2^29
     const int len = fin ? t + 1 : 0;  // episode length = timestep after the final step (yard.py:355)
     int n_step = active, n_ep = fin, n_pol = fin && st == ST_CAPTURE, n_mrx = fin && st != ST_CAPTURE;
     int n_trunc = fin && st == ST_TIMEOUT, n_broke = fin && st == ST_NO_MONEY;
-    int len_sum = len, len_sq = len * len, len_pol = n_pol ? len : 0, len_mrx = n_mrx ? len : 0;
-    int ep_spent = sm.ep_spent[lane], spent = sm.spent[lane], moves = sm.moves[lane];
+    int len_sum = len, len_pol = n_pol ? len : 0, len_mrx = n_mrx ? len : 0;
+    unsigned long long len_sq = (unsigned long long)len * len, ep_spent = (unsigned long long)sm.ep_spent[lane];
+    int spent = sm.spent[lane], moves = sm.moves[lane];
     if constexpr (GROUPS) {
       // per-group sums: the lanes of each distinct group reduce together, one leader adds them to the group's line
       const int v[SY_STAT_POLICE_MOVES + 1] = {n_step, n_ep, n_mrx, n_pol, n_trunc, n_broke, len_sum, spent,
-                                               len_sq, len_pol, len_mrx, ep_spent, moves};
+                                               0, len_pol, len_mrx, 0, moves};
       const unsigned same = __match_any_sync(FULL, grp);
       const bool leader = grp >= 0 && lane == __ffs(same) - 1;
       unsigned long long* line = p.grp_stats + ((size_t)(blockIdx.x % p.grp_rep) * p.grp_n + max(grp, 0)) * SY_NUM_STATS;
 #pragma unroll
       for (int k = 0; k <= SY_STAT_POLICE_MOVES; ++k) {
-        const int sum = __reduce_add_sync(same, v[k]);
-        if (leader && sum) atomicAdd(line + k, (unsigned long long)sum);
+        const unsigned long long sum = k == SY_STAT_SUM_SQ_EPISODE_LENGTH ? warp_sum_u64(same, len_sq)
+                                       : k == SY_STAT_SUM_EPISODE_BUDGET_SPENT ? warp_sum_u64(same, ep_spent)
+                                       : (unsigned long long)__reduce_add_sync(same, v[k]);
+        if (leader && sum) atomicAdd(line + k, sum);
       }
     }
     // per-tile sums -> one of STAT_REPLICAS library-owned accumulator lines (sy_stats folds them into the caller's
@@ -941,12 +954,12 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
       n_trunc = __reduce_add_sync(FULL, n_trunc);
       n_broke = __reduce_add_sync(FULL, n_broke);
       len_sum = __reduce_add_sync(FULL, len_sum);
-      len_sq = __reduce_add_sync(FULL, len_sq);
+      len_sq = warp_sum_u64(FULL, len_sq);
       len_pol = __reduce_add_sync(FULL, len_pol);
       len_mrx = __reduce_add_sync(FULL, len_mrx);
-      ep_spent = __reduce_add_sync(FULL, ep_spent);
+      ep_spent = warp_sum_u64(FULL, ep_spent);
     }
-    int v = 0;  // every lane holds all sums: lane k adds statistic k (one atomic instruction for the warp)
+    unsigned long long v = 0;  // every lane holds all sums: lane k adds statistic k (one atomic instruction for the warp)
     switch (lane) {
       case SY_STAT_ENV_STEPS: v = n_step; break;
       case SY_STAT_EPISODES: v = n_ep; break;
@@ -963,7 +976,7 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
       case SY_STAT_POLICE_MOVES: v = moves; break;
       default: break;
     }
-    if (v) atomicAdd(p.stats_rep + (size_t)(blockIdx.x % STAT_REPLICAS) * SY_NUM_STATS + lane, (unsigned long long)v);
+    if (v) atomicAdd(p.stats_rep + (size_t)(blockIdx.x % STAT_REPLICAS) * SY_NUM_STATS + lane, v);
   }
   for (int i = tid; i < nEnv * A; i += LOGIC_THREADS) {
     const int e = (i * p.inv_A) >> 16, a = i - e * A;  // i / A without a division (i < 512, A <= 16)
@@ -3457,6 +3470,9 @@ int sy_create(const SyConfig* c, SyEnv** out_env) {
     return fail(SY_ERR_INVALID_ARGUMENT, "num_nodes must be in [num_police + 1, 65534]");  // nodes are staged as u16
   if (c->agent_money < 0 || c->mrx_money < 0 || c->toll < 0 || c->reveal_interval < 0 || c->max_timestep < 0)
     return fail(SY_ERR_INVALID_ARGUMENT, "negative money / toll / reveal_interval / max_timestep");
+  if (c->toll > SY_MAX_TOLL) return fail(SY_ERR_INVALID_ARGUMENT, "toll %d outside [0, %d]", c->toll, SY_MAX_TOLL);
+  if (c->max_timestep > SY_MAX_TIMESTEP)  // longer episodes would saturate the u16 visit counters
+    return fail(SY_ERR_INVALID_ARGUMENT, "max_timestep %d outside [0, %d]", c->max_timestep, SY_MAX_TIMESTEP);
   if (!(c->reveal_skip_prob >= 0.0f && c->reveal_skip_prob <= 1.0f)) return fail(SY_ERR_INVALID_ARGUMENT, "reveal_skip_prob must be in [0, 1]");
   if (c->reward_mode != SY_REWARD_FP64 && c->reward_mode != SY_REWARD_FP32)
     return fail(SY_ERR_INVALID_ARGUMENT, "unknown reward_mode %d", c->reward_mode);

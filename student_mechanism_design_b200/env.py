@@ -87,13 +87,9 @@ def pack_mechanism(mech: Dict, base) -> "_cabi.SyGroup":
     w = [float(weights[k].detach()) if isinstance(weights[k], torch.Tensor) else float(weights[k]) for k in REWARD_WEIGHT_NAMES]
     if not all(np.isfinite(w)):
         raise ValueError("reward weights must be finite")
-    money = mech.get("agent_money", base.agent_money)
-    reveal = mech.get("reveal_interval", base.reveal_interval)
+    money = _integral("agent_money", mech.get("agent_money", base.agent_money), 0, _cabi.INT32_MAX)
+    reveal = _integral("reveal_interval", mech.get("reveal_interval", base.reveal_interval), 0, _cabi.INT32_MAX)
     skip = float(mech.get("reveal_skip_prob", base.config.reveal_skip_prob))
-    if int(money) != money or int(money) < 0:
-        raise ValueError(f"agent_money must be a non-negative integer, got {money}")
-    if int(reveal) != reveal or int(reveal) < 0:
-        raise ValueError(f"reveal_interval must be a non-negative integer, got {reveal}")
     if not 0.0 <= skip <= 1.0:
         raise ValueError(f"reveal_skip_prob must be in [0, 1], got {skip}")
     if "tolls" in mech:
@@ -104,7 +100,7 @@ def pack_mechanism(mech: Dict, base) -> "_cabi.SyGroup":
     g.struct_bytes = C.sizeof(_cabi.SyGroup)
     for i, v in enumerate(w):
         g.reward_weights[i] = v
-    g.agent_money, g.reveal_interval, g.reveal_skip_prob = int(money), int(reveal), skip
+    g.agent_money, g.reveal_interval, g.reveal_skip_prob = money, reveal, skip
     return g
 
 
@@ -197,6 +193,13 @@ class BatchedScotlandYardEnv:
                  device="cuda:0", reward_tables=None, keep_reward64: bool = False, collect_stats: bool = True,
                  graph_offset: int = 0, max_edges_per_node: int = 4, max_weight: int = 5,
                  node_features_dtype: torch.dtype = torch.float32, reveal_skip_prob: float = 0.0, guard_bytes: int = 0):
+        # the int32 fields of SyConfig, checked before ctypes would wrap them (2**32 + 5 reads back as 5); the library
+        # refuses the rest (police count, node count)
+        num_envs = _integral("num_envs", num_envs, 1, _cabi.INT32_MAX)
+        agent_money = _integral("agent_money", agent_money, 0, _cabi.INT32_MAX)
+        max_timestep = _integral("max_timestep", max_timestep, 0, _cabi.SY_MAX_TIMESTEP)
+        reveal_interval = _integral("reveal_interval", reveal_interval or 0, 0, _cabi.INT32_MAX)
+        tolls = _integral("tolls", tolls, 0, _cabi.SY_MAX_TOLL)
         if not torch.cuda.is_available():
             raise _cabi.SyError("BatchedScotlandYardEnv needs a CUDA device; there is no CPU fallback")
         self._lib = _cabi.load_library()
@@ -212,8 +215,6 @@ class BatchedScotlandYardEnv:
         self.agent_money = int(agent_money)
         self.possible_agents = ["MrX"] + [f"Police{i}" for i in range(self.number_of_agents)]  # yard.py:54-56
         self.agents = list(self.possible_agents)
-        if float(tolls) != int(tolls):
-            raise ValueError("tolls must be integral so budgets stay integers (mechanism.yaml:12 uses 1.0)")
         reward_weights = dict(DEFAULT_REWARD_WEIGHTS) if reward_weights is None else dict(reward_weights)
         missing = [k for k in REWARD_WEIGHT_NAMES if k not in reward_weights]
         if missing:
