@@ -341,6 +341,48 @@ int sy_sample_actions_i32(SyEnv* env, const SyState* state, uint32_t step_counte
 int sy_sample_actions(SyEnv* env, const SyState* state, uint32_t step_counter, int64_t* actions,
                       sy_stream_t stream);
 
+/* Heuristic opponents for the whole batch: an evading MrX and chasing police, the counterpart of the heuristics of
+ * src/eval/exploitability.py:122,188 (parity unpinned: that source is not available, the rules below are this library's).
+ * One launch; reads the state, SyObs.mrx_revealed, the all-pairs distance table D and the mechanism group rows (toll,
+ * police count), and writes actions int64 [B, A].  Notation for env b: toll_b = its group's toll (else config.toll), P_b =
+ * its police count (agents past P_b are absent); neighbour j of node u is affordable for money m iff w(u, j) + toll_b <= m
+ * (the rule of the step, the mask and the sampler); D[x][y] of 0xFFFF counts as 65 535; police positions are those of
+ * the state read (before the step).
+ *   random draw   = exactly sy_sample_actions(step_counter) for that (env, agent) (-1 without an affordable neighbour).
+ *   exploration   an agent takes the random draw when Philox(env_offset + b, step_counter, 4, agent).x < explore_<side>,
+ *                 with explore_<side> = floor(epsilon * 2^32) in [0, 2^32] (2^32: always, 0: never).
+ *   SY_HEUR_EVADE (MrX) candidates: its own node and every affordable neighbour no present police occupies; score of c:
+ *                 min over present police i of D[c][pos_i]; highest score wins, ties to the own node, then to the lowest
+ *                 id.  The own node means "stay".
+ *   SY_HEUR_CHASE (police) target = mrx_revealed[b] when >= 0, else the env's last_seen entry; unknown (-1): the random
+ *                 draw.  Otherwise: no affordable neighbour -> -1; every affordable neighbour occupied by another present
+ *                 police -> the agent's own node (it stays, but acts: "every police skipped" is not triggered); else the
+ *                 affordable unoccupied neighbour with the smallest D[j][target], ties to the lowest id.
+ *   SY_HEUR_CHASE_BELIEF  as CHASE, but a hidden MrX's target is the first argmax of belief[b, :] (never unknown).  Needs
+ *                 config.belief != 0 and SyState.belief, and is refused with SY_ERR_STATE while observations are pending
+ *                 (the belief map lags the state after sy_step_deferred).
+ *   SY_HEUR_RANDOM  the random draw.  SY_HEUR_NONE  that side's columns of `actions` are left untouched (e.g. written by
+ *                 a learned policy before the call: score it against heuristic opponents).
+ * Absent agents get -1 from every kind but NONE.  Frozen envs get actions by the same rules (the step ignores them).
+ * last_seen: caller-owned DEVICE int32 [B] or NULL.  Per env the call computes ls = rev >= 0 ? rev : (timestep == 0 ? -1 :
+ * last_seen[b]) with rev = mrx_revealed[b] and writes it back (whatever the kinds).  It is MrX's last revealed node of the
+ * current episode when the call has been made at every step of that episode (a plain step loop, RolloutCollector); fill
+ * it with -1 when starting.  NULL: a hidden MrX is never remembered.
+ * Preconditions of sy_sample_actions (graphs and reward tables loaded); SY_ERR_STATE while mechanism groups wait for their
+ * reset, as the step entry points.  SY_ERR_INVALID_ARGUMENT for a wrong struct_bytes, a kind out of range, a threshold
+ * above 2^32, a NULL SyObs.mrx_revealed, or CHASE_BELIEF without a belief map. */
+enum { SY_HEUR_NONE = 0, SY_HEUR_RANDOM = 1, SY_HEUR_EVADE = 2, SY_HEUR_CHASE = 3, SY_HEUR_CHASE_BELIEF = 4 };
+typedef struct SyHeuristic {
+  uint64_t struct_bytes;   /* = sizeof(SyHeuristic) */
+  int32_t mrx_kind;        /* SY_HEUR_NONE | SY_HEUR_RANDOM | SY_HEUR_EVADE */
+  int32_t police_kind;     /* SY_HEUR_NONE | SY_HEUR_RANDOM | SY_HEUR_CHASE | SY_HEUR_CHASE_BELIEF */
+  uint64_t explore_mrx;    /* floor(epsilon_mrx * 2^32), in [0, 2^32] */
+  uint64_t explore_police; /* floor(epsilon_police * 2^32), in [0, 2^32] */
+  int32_t* last_seen;      /* [B] device or NULL */
+} SyHeuristic;
+int sy_heuristic_actions(SyEnv* env, const SyHeuristic* h, const SyState* state, const SyObs* obs,
+                         uint32_t step_counter, int64_t* actions, sy_stream_t stream);
+
 /* Add the statistics accumulated since the last call to `stats` (device, int64 [SY_NUM_STATS], caller-owned and
  * cumulative) and clear the library's internal accumulators.  Asynchronous on `stream`.  Statistics are collected by
  * sy_step only while SyOut.stats is non-NULL (they are kept in per-tile-group lines inside the library so that the

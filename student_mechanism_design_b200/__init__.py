@@ -14,11 +14,11 @@ from .sharding import allreduce_stats, shard_range  # noqa: F401,E402
 from .compat import CustomEnvironment  # noqa: F401,E402
 from .torchrl_env import make_torchrl_env  # noqa: F401,E402
 from .rollout import RolloutCollector, batched_graph_data, masked_sample  # noqa: F401,E402
-from .policy import GNNPolicy, MappoPolicy, gcn_in_edges  # noqa: F401,E402
+from .policy import GNNPolicy, HeuristicPolicy, MappoPolicy, gcn_in_edges  # noqa: F401,E402
 
 __all__ = [
     "allreduce_stats", "shard_range", "CustomEnvironment", "make_torchrl_env", "RolloutCollector", "batched_graph_data",
-    "masked_sample", "GNNPolicy", "MappoPolicy", "gcn_in_edges",
+    "masked_sample", "GNNPolicy", "HeuristicPolicy", "MappoPolicy", "gcn_in_edges",
     "BatchedScotlandYardEnv", "GraphSpec", "generate_connected_graph", "generate_graph_pool", "pack_csr",
     "dense_action_mask", "numpy_reward_tables", "DEFAULT_REWARD_WEIGHTS", "REWARD_WEIGHT_NAMES", "SyError",
     "load_library", "LIB_PATH",

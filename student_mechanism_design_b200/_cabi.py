@@ -73,6 +73,16 @@ class SyGroup(C.Structure):
     ]
 
 
+SY_HEUR_NONE, SY_HEUR_RANDOM, SY_HEUR_EVADE, SY_HEUR_CHASE, SY_HEUR_CHASE_BELIEF = 0, 1, 2, 3, 4
+
+
+class SyHeuristic(C.Structure):
+    _fields_ = [
+        ("struct_bytes", C.c_uint64), ("mrx_kind", C.c_int32), ("police_kind", C.c_int32), ("explore_mrx", C.c_uint64),
+        ("explore_police", C.c_uint64), ("last_seen", C.c_void_p),
+    ]
+
+
 # name -> (restype, argtypes); must list every function include/sy_env.h declares
 SIGNATURES = {
     "sy_abi_version": (C.c_int, []),
@@ -109,6 +119,8 @@ SIGNATURES = {
     "sy_sample_actions_host": (C.c_int, [C.c_void_p, C.POINTER(SyState), C.c_uint32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
     "sy_sample_actions_i32": (C.c_int, [C.c_void_p, C.POINTER(SyState), C.c_uint32, C.c_void_p, C.c_void_p]),
     "sy_sample_actions": (C.c_int, [C.c_void_p, C.POINTER(SyState), C.c_uint32, C.c_void_p, C.c_void_p]),
+    "sy_heuristic_actions": (C.c_int, [C.c_void_p, C.POINTER(SyHeuristic), C.POINTER(SyState), C.POINTER(SyObs), C.c_uint32,
+                                       C.c_void_p, C.c_void_p]),
     "sy_copy_segments": (C.c_int, [C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sy_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "sy_set_groups": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(SyGroup), C.c_void_p, C.c_void_p]),

@@ -2995,6 +2995,141 @@ __global__ void sy_mask_dense_kernel(int N, const double* adj, const double* w, 
   }
 }
 
+// ---------------------------------------------------------------------------------------------
+// heuristic opponents (sy_heuristic_actions): an evading MrX and chasing police, the counterpart of the heuristics of
+// src/eval/exploitability.py:122,188 (parity unpinned: the rules are those of include/sy_env.h, restated by
+// oracle/heuristic_oracle.py).  CTA per 32-env tile: warp per env for the per-env part (MrX's last known node,
+// the chase target, the belief argmax read as coalesced rows), then thread per (env, agent) for the actions.
+// ---------------------------------------------------------------------------------------------
+constexpr unsigned RNG_HEURISTIC = 4;  // Philox purpose of the exploration draws (0..3 and 16..20 are taken)
+constexpr int HEUR_ENVS = 32, HEUR_THREADS = 256;
+
+struct HeurArgs {
+  int mrx_kind, police_kind;
+  unsigned long long thr_mrx, thr_police;  // explore iff Philox word < threshold (epsilon * 2^32)
+  int32_t* last_seen;                      // [B] or NULL
+  long long* actions;                      // int64 [B, A]
+  unsigned step_counter;
+};
+
+// the draw of sy_sample_actions_kernel for a present agent at node u with budget m
+__device__ __forceinline__ int heur_random_action(const Params& p, unsigned b, unsigned a, int g, int u, int m, int toll,
+                                                  unsigned step_counter) {
+  const Tables& tb = p.tb;
+  const int nvalid = move_count(tb, p.N, g, u, m, toll);
+  if (nvalid <= 0) return -1;
+  const unsigned env_id = (unsigned)(p.env_offset + (unsigned long long)b);
+  const uint4 r = philox4x32(make_uint4(env_id, step_counter, RNG_ACTION, a), make_uint2(p.seed_lo, p.seed_hi));
+  int pick = (int)__umulhi(r.x, (unsigned)nvalid);
+  const uint8_t* wg = tb.wgt + (size_t)g * tb.nnz_stride;
+  for (int k = __ldg(tb.row_ptr + (size_t)g * (p.N + 1) + u);; ++k) {  // the pick-th affordable neighbour exists
+    if (__ldg(wg + k) + toll <= m) {
+      if (pick == 0) return __ldg(tb.col + (size_t)g * tb.nnz_stride + k);
+      --pick;
+    }
+  }
+}
+
+template <int GROUPS>
+__global__ void __launch_bounds__(HEUR_THREADS) sy_heuristic_actions_kernel(const Params p, const HeurArgs h) {
+  __shared__ int s_pos[HEUR_ENVS * AS];   // positions of the tile (row = env)
+  __shared__ int s_target[HEUR_ENVS];     // chase target per env, -1 unknown
+  const int b0 = blockIdx.x * HEUR_ENVS, ne = min(HEUR_ENVS, p.B - b0), A = p.A, N = p.N;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  for (int i = tid; i < ne * A; i += HEUR_THREADS) {
+    const int e = i / A;
+    s_pos[e * AS + (i - e * A)] = p.st.pos[(size_t)b0 * A + i];
+  }
+  for (int e = warp; e < ne; e += HEUR_THREADS / 32) {
+    const int b = b0 + e;
+    const int rev = p.ob.mrx_revealed[b];
+    const int ls = rev >= 0 ? rev : ((h.last_seen && p.st.timestep[b] != 0) ? h.last_seen[b] : -1);
+    int target = ls;
+    if (h.police_kind == SY_HEUR_CHASE_BELIEF && rev < 0) {  // first argmax of the belief row
+      const float* row = p.st.belief + (size_t)b * N;
+      float best = -INFINITY;
+      int bi = N;
+      for (int j = lane; j < N; j += 32) {
+        const float v = row[j];
+        if (v > best) best = v, bi = j;
+      }
+#pragma unroll
+      for (int off = 16; off > 0; off >>= 1) {
+        const float ov = __shfl_xor_sync(FULL, best, off);
+        const int oi = __shfl_xor_sync(FULL, bi, off);
+        if (ov > best || (ov == best && oi < bi)) best = ov, bi = oi;
+      }
+      target = bi < N ? bi : 0;  // (a row without an ordered maximum, e.g. all NaN: node 0)
+    }
+    if (lane == 0) {
+      s_target[e] = target;
+      if (h.last_seen) h.last_seen[b] = ls;
+    }
+  }
+  __syncthreads();
+  const Tables& tb = p.tb;
+  for (int i = tid; i < ne * A; i += HEUR_THREADS) {
+    const int e = i / A, a = i - e * A, b = b0 + e;
+    const int kind = a == 0 ? h.mrx_kind : h.police_kind;
+    if (kind == SY_HEUR_NONE) continue;
+    const GroupRow* gr = GROUPS ? p.grp + __ldg(p.grp_id + b) : nullptr;
+    const int P = env_police<GROUPS>(p, gr);
+    long long act = -1;
+    if (a <= P) {  // absent agents: -1
+      const int* sp = s_pos + e * AS;
+      const int g = p.st.graph_id[b], u = sp[a], m = p.st.money[(size_t)b * A + a];
+      const int toll = env_toll<GROUPS>(p, gr);
+      const unsigned long long thr = a == 0 ? h.thr_mrx : h.thr_police;
+      bool random = kind == SY_HEUR_RANDOM || (a > 0 && s_target[e] < 0);
+      if (!random && thr) {
+        const uint4 r = philox4x32(make_uint4((unsigned)(p.env_offset + (unsigned long long)b), h.step_counter, RNG_HEURISTIC,
+                                              (unsigned)a), make_uint2(p.seed_lo, p.seed_hi));
+        random = (unsigned long long)r.x < thr;
+      }
+      if (random) {
+        act = heur_random_action(p, b, a, g, u, m, toll, h.step_counter);
+      } else {
+        const int k0 = __ldg(tb.row_ptr + (size_t)g * (N + 1) + u), k1 = __ldg(tb.row_ptr + (size_t)g * (N + 1) + u + 1);
+        const uint16_t* col = tb.col + (size_t)g * tb.nnz_stride;
+        const uint8_t* wg = tb.wgt + (size_t)g * tb.nnz_stride;
+        const uint16_t* Dg = tb.D + (size_t)g * N * N;
+        if (a == 0) {  // evade: the candidate farthest from the nearest police; ties: stay, then the lowest node
+          int best = u, best_s = INT_MAX;
+          for (int i2 = 1; i2 <= P; ++i2) best_s = min(best_s, (int)__ldg(Dg + (size_t)u * N + sp[i2]));
+          for (int k = k0; k < k1; ++k) {
+            const int c = __ldg(col + k);
+            if (__ldg(wg + k) + toll > m) continue;
+            bool occupied = false;
+            for (int i2 = 1; i2 <= P; ++i2) occupied |= sp[i2] == c;
+            if (occupied) continue;
+            const uint16_t* row = Dg + (size_t)c * N;
+            int s = INT_MAX;
+            for (int i2 = 1; i2 <= P; ++i2) s = min(s, (int)__ldg(row + sp[i2]));
+            if (s > best_s) best = c, best_s = s;
+          }
+          act = best;
+        } else {  // chase: the free affordable neighbour nearest to the target (D symmetric: one row, D[target][.])
+          const uint16_t* row = Dg + (size_t)s_target[e] * N;
+          int best = -1, best_d = INT_MAX;
+          bool affordable = false;
+          for (int k = k0; k < k1; ++k) {
+            const int c = __ldg(col + k);
+            if (__ldg(wg + k) + toll > m) continue;
+            affordable = true;
+            bool occupied = false;
+            for (int i2 = 1; i2 <= P; ++i2) occupied |= sp[i2] == c;
+            if (occupied) continue;
+            const int d = __ldg(row + c);
+            if (d < best_d) best = c, best_d = d;
+          }
+          act = best >= 0 ? best : (affordable ? u : -1);  // boxed in by police: stays, but acts
+        }
+      }
+    }
+    h.actions[(size_t)b * A + a] = act;
+  }
+}
+
 }  // namespace
 
 // =============================================================================================
@@ -4297,6 +4432,35 @@ int sy_sample_actions(SyEnv* e, const SyState* st, uint32_t step_counter, int64_
 
 int sy_sample_actions_i32(SyEnv* e, const SyState* st, uint32_t step_counter, int32_t* actions, sy_stream_t stream) {
   return sample_impl<int>(e, st, step_counter, actions, stream);
+}
+
+int sy_heuristic_actions(SyEnv* e, const SyHeuristic* h, const SyState* st, const SyObs* ob, uint32_t step_counter,
+                         int64_t* actions, sy_stream_t stream) {
+  if (!e || !h || !actions) return fail(SY_ERR_INVALID_ARGUMENT, "NULL env / heuristic / actions");
+  if (h->struct_bytes != sizeof(SyHeuristic)) return fail(SY_ERR_INVALID_ARGUMENT, "SyHeuristic size mismatch: got %llu, library expects %zu (ABI %d)", (unsigned long long)h->struct_bytes, sizeof(SyHeuristic), SY_ABI_VERSION);
+  if (h->mrx_kind != SY_HEUR_NONE && h->mrx_kind != SY_HEUR_RANDOM && h->mrx_kind != SY_HEUR_EVADE)
+    return fail(SY_ERR_INVALID_ARGUMENT, "SyHeuristic.mrx_kind must be SY_HEUR_NONE, SY_HEUR_RANDOM or SY_HEUR_EVADE, got %d", h->mrx_kind);
+  if (h->police_kind != SY_HEUR_NONE && h->police_kind != SY_HEUR_RANDOM && h->police_kind != SY_HEUR_CHASE && h->police_kind != SY_HEUR_CHASE_BELIEF)
+    return fail(SY_ERR_INVALID_ARGUMENT, "SyHeuristic.police_kind must be SY_HEUR_NONE, SY_HEUR_RANDOM, SY_HEUR_CHASE or SY_HEUR_CHASE_BELIEF, got %d", h->police_kind);
+  if (h->explore_mrx > (1ull << 32) || h->explore_police > (1ull << 32))
+    return fail(SY_ERR_INVALID_ARGUMENT, "SyHeuristic exploration thresholds must be at most 2^32");
+  Params p;
+  int rc = fill_params(e, st, ob, nullptr, p);
+  if (rc) return rc;
+  if (!ob || !ob->mrx_revealed) return fail(SY_ERR_INVALID_ARGUMENT, "SyObs.mrx_revealed is NULL");
+  const bool belief = h->police_kind == SY_HEUR_CHASE_BELIEF;
+  if (belief && (!e->cfg.belief || !st->belief)) return fail(SY_ERR_INVALID_ARGUMENT, "SY_HEUR_CHASE_BELIEF needs config.belief and SyState.belief");
+  if (e->grp_need_reset) return fail(SY_ERR_STATE, "mechanism groups changed: a sy_reset of every env (NULL or all-set mask) must come before the next step");
+  if (belief && e->obs_pending) return fail(SY_ERR_STATE, "SY_HEUR_CHASE_BELIEF reads the belief map: observations are pending (sy_flush_observations first)");
+  const HeurArgs a{h->mrx_kind, h->police_kind, h->explore_mrx, h->explore_police, h->last_seen,
+                   reinterpret_cast<long long*>(actions), step_counter};
+  CUDA_TRY(cudaSetDevice(e->cfg.device));
+  const unsigned grid = (unsigned)((p.B + HEUR_ENVS - 1) / HEUR_ENVS);
+  if (p.grp_n) sy_heuristic_actions_kernel<1><<<grid, HEUR_THREADS, 0, (cudaStream_t)stream>>>(p, a);
+  else sy_heuristic_actions_kernel<0><<<grid, HEUR_THREADS, 0, (cudaStream_t)stream>>>(p, a);
+  g_launches++;
+  CUDA_TRY(cudaGetLastError());
+  return SY_OK;
 }
 
 int sy_stats(SyEnv* e, int64_t* stats, sy_stream_t stream) {

@@ -3,6 +3,8 @@
 `GNNPolicy`   = GNNAgent.select_action / GNNModel.forward (src/agent/gnn_agent.py:45-82, 230-257) for MrX's agent and
                 the police agent (gnn_trainer.py:147-165), all envs and agents in one launch.
 `MappoPolicy` = MappoAgent.select_action / AgentPolicy / CentralCritic (src/agent/mappo_agent.py:6-44, 87-142).
+`HeuristicPolicy` = heuristic opponents (evading MrX, chasing police) of libsy_env.so's sy_heuristic_actions, the
+                counterpart of src/eval/exploitability.py:122,188 (parity unpinned).
 
 Parameters use the reference modules' own `state_dict` keys, so checkpoints written by the reference
 (`GNNAgent.save`, `MappoAgent.save`) load unchanged.  The kernels live in libsy_policy.so (include/sy_policy.h);
@@ -17,6 +19,7 @@ from typing import Dict, Optional, Sequence
 import numpy as np
 import torch
 
+from . import _cabi
 from . import _policy_cabi as pc
 from .graphs import GraphSpec, pack_csr
 
@@ -209,6 +212,81 @@ class GNNPolicy(_PolicyBase):
 
     def __call__(self, obs=None):
         return self.act(self.epsilon[0], self.epsilon[1])
+
+
+class HeuristicPolicy:
+    """Heuristic opponents for every env in one launch (sy_heuristic_actions, include/sy_env.h): an evading MrX
+    (`mrx="evade"`: stay or move to the affordable free neighbour farthest from the nearest police) and chasing police
+    (`police="chase"`: step towards MrX's revealed or last revealed node; `"chase_belief"`: towards the belief map's mode
+    while MrX is hidden), or the random-valid policy (`"random"`) per side.  `None` leaves that side's columns of `out`
+    as they are, so a learned policy can be scored against heuristic opponents: `a = gnn.act(); heur.act(out=a)`.
+    Each side explores (takes the random-valid action) with its own probability `epsilon_*`.  Works with every
+    mechanism group field, mixed police counts included.  The counterpart of src/eval/exploitability.py:122,188
+    (parity unpinned).
+
+    The policy owns `last_seen` (int32 [B], MrX's last revealed node per env); it follows the episodes when `act` is
+    called at every step, as RolloutCollector and a plain step loop do.  `reset_memory()` clears it."""
+
+    MRX_KINDS = {None: _cabi.SY_HEUR_NONE, "random": _cabi.SY_HEUR_RANDOM, "evade": _cabi.SY_HEUR_EVADE}
+    POLICE_KINDS = {None: _cabi.SY_HEUR_NONE, "random": _cabi.SY_HEUR_RANDOM, "chase": _cabi.SY_HEUR_CHASE,
+                    "chase_belief": _cabi.SY_HEUR_CHASE_BELIEF}
+    returns_actions = True  # RolloutCollector: act() returns actions
+
+    def __init__(self, env, mrx: Optional[str] = "evade", police: Optional[str] = "chase", epsilon_mrx: float = 0.0,
+                 epsilon_police: float = 0.0):
+        if mrx not in self.MRX_KINDS:
+            raise ValueError(f"mrx must be one of {list(self.MRX_KINDS)}, got {mrx!r}")
+        if police not in self.POLICE_KINDS:
+            raise ValueError(f"police must be one of {list(self.POLICE_KINDS)}, got {police!r}")
+        if police == "chase_belief" and not env.belief_on:
+            raise ValueError("police='chase_belief' needs an env built with belief=True")
+        self._lib = _cabi.load_library()
+        self.env, self.mrx, self.police = env, mrx, police
+        self.epsilon_mrx, self.epsilon_police = float(epsilon_mrx), float(epsilon_police)
+        self.last_seen = torch.full((env.num_envs,), -1, dtype=torch.int32, device=env.device)
+        # the dense belief map lags the state after a deferred step; everything else the kernel reads is compact state
+        self.reads_state_only = police != "chase_belief"
+        self._h = _cabi.SyHeuristic(C.sizeof(_cabi.SyHeuristic), self.MRX_KINDS[mrx], self.POLICE_KINDS[police],
+                                    self.explore_threshold(epsilon_mrx), self.explore_threshold(epsilon_police),
+                                    self.last_seen.data_ptr())
+
+    @staticmethod
+    def explore_threshold(epsilon: float) -> int:
+        """floor(epsilon * 2^32), exact for every double in [0, 1]: an agent explores when its Philox word is below it"""
+        if isinstance(epsilon, bool) or not isinstance(epsilon, (int, float, np.integer, np.floating)):
+            raise ValueError(f"epsilon must be a number in [0, 1], got {epsilon!r}")
+        e = float(epsilon)
+        if not 0.0 <= e <= 1.0:  # (NaN fails both comparisons)
+            raise ValueError(f"epsilon must be in [0, 1], got {epsilon!r}")
+        return int(e * 2 ** 32)
+
+    def reset_memory(self):
+        """forget MrX's last revealed node in every env"""
+        self.last_seen.fill_(-1)
+
+    def act(self, out: Optional[torch.Tensor] = None, step_counter: Optional[int] = None) -> torch.Tensor:
+        """int64 [B, A] actions (-1 = none).  `out`: int64 [B, A] on the env's device, written in place (the columns of
+        a `None` side keep their values); None allocates one filled with -1.  `step_counter` keys the random draws
+        exactly as `env.sample_actions`; None takes the env's sampler counter and advances it."""
+        e = self.env
+        if not e._is_reset:
+            raise _cabi.SyError("act() before reset()")
+        shape = (e.num_envs, e.num_agents)
+        if out is None:
+            out = torch.full(shape, -1, dtype=torch.int64, device=e.device)
+        elif not (isinstance(out, torch.Tensor) and out.dtype == torch.int64 and tuple(out.shape) == shape
+                  and out.device == e.device and out.is_contiguous()):
+            raise ValueError(f"out must be a contiguous int64 tensor of shape {shape} on {e.device}")
+        if step_counter is None:
+            step_counter = e._sample_counter
+            e._sample_counter += 1
+        with torch.cuda.device(e.device):
+            _cabi.check(self._lib.sy_heuristic_actions(e._handle, C.byref(self._h), C.byref(e._state), C.byref(e._obs),
+                                                       int(step_counter) & 0xFFFFFFFF, out.data_ptr(), e._stream()))
+        return out
+
+    def __call__(self, obs=None):
+        return self.act()
 
 
 class MappoPolicy(_PolicyBase):
