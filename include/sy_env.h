@@ -218,7 +218,8 @@ enum { SY_WRITER_BULK = 0, SY_WRITER_LSU = 1 };
 enum { SY_STEP_FUSED = 0, SY_STEP_TWO_KERNELS = 1, SY_STEP_AUTO = 2 };
 enum { SY_LAGGED_OFF = 0, SY_LAGGED_ON = 1, SY_LAGGED_AUTO = 2 };
 int sy_set_option(SyEnv* env, int32_t option, int32_t value);
-/* new Philox key for subsequent (auto-)resets and action sampling (torchrl `set_seed`) */
+/* new Philox key for subsequent (auto-)resets and action sampling (torchrl `set_seed`).  Launches captured in a CUDA
+ * graph carry the key by value: a graph captured before this call keeps drawing with the key of its capture. */
 int sy_set_seed(SyEnv* env, uint64_t seed);
 
 /* Host-built float64 tables so that rewards are bit-identical to NumPy's:

@@ -34,12 +34,13 @@
 #define SYO_INF 0xFFFF
 enum { W_POLICE_DISTANCE, W_POLICE_GROUP, W_POLICE_POSITION, W_POLICE_TIME, W_MRX_CLOSEST, W_MRX_AVERAGE,
        W_MRX_POSITION, W_MRX_TIME, W_POLICE_COVERAGE, W_POLICE_PROXIMITY, W_POLICE_OVERLAP }; /* reward_net.py:5-17 */
-enum { RNG_RESET_POS = 0, RNG_RESET_GRAPH = 1, RNG_ACTION = 2 };
+enum { RNG_RESET_POS = 0, RNG_RESET_GRAPH = 1, RNG_ACTION = 2, RNG_REVEAL_SKIP = 3 };
 enum { WIN_NONE = 0, WIN_MRX = 1, WIN_POLICE = 2 };
 
 typedef struct SyoConfig {
   int32_t num_nodes, num_police, agent_money, mrx_money, max_timestep, reveal_interval, toll, belief;
-  int32_t reward_mode, auto_reset, resample_graph, num_graphs, nnz_stride, n_exp, n_cov, pad;
+  int32_t reward_mode, auto_reset, resample_graph, num_graphs, nnz_stride, n_exp, n_cov;
+  float reveal_skip_prob; /* every scheduled reveal is skipped with this probability (the batched env's draw) */
   int64_t env_offset;
   uint64_t seed;
   double w[11];
@@ -351,7 +352,13 @@ static void step_one(const SyoConfig* c, const SyoState* st, const SyoOut* out, 
   out->truncated[b] = (uint8_t)trunc;
   out->winner[b] = (int8_t)win;
   /* extensions (parity unpinned): reveal schedule + belief on the new timestep */
-  const int rev = is_reveal(st->t[b], c->reveal_interval);
+  int rev = is_reveal(st->t[b], c->reveal_interval);
+  if (rev && c->reveal_skip_prob > 0.0f) { /* skip iff Philox(seed; env, t, RNG_REVEAL_SKIP, episode)[0] < p * 2^32 */
+    const uint32_t ctr[4] = {(uint32_t)(c->env_offset + b), (uint32_t)st->t[b], RNG_REVEAL_SKIP, (uint32_t)st->episode[b]};
+    uint32_t r[4];
+    philox4x32(ctr, (uint32_t)c->seed, (uint32_t)(c->seed >> 32), r);
+    if ((unsigned long long)r[0] < (unsigned long long)((double)fminf(c->reveal_skip_prob, 1.0f) * 4294967296.0)) rev = 0;
+  }
   st->revealed[b] = (c->reveal_interval > 0) ? (rev ? pos[0] : -1) : pos[0];
   if (st->belief)
     belief_update(c, c->row_ptr + (size_t)g * (N + 1), c->col + (size_t)g * c->nnz_stride, st->belief + (size_t)b * N, tmp,

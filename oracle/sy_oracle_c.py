@@ -37,8 +37,8 @@ def available() -> bool:
 class SyoConfig(C.Structure):
     _fields_ = [(n, C.c_int32) for n in (
         "num_nodes", "num_police", "agent_money", "mrx_money", "max_timestep", "reveal_interval", "toll", "belief",
-        "reward_mode", "auto_reset", "resample_graph", "num_graphs", "nnz_stride", "n_exp", "n_cov", "pad")] + [
-        ("env_offset", C.c_int64), ("seed", C.c_uint64), ("w", C.c_double * 11),
+        "reward_mode", "auto_reset", "resample_graph", "num_graphs", "nnz_stride", "n_exp", "n_cov")] + [
+        ("reveal_skip_prob", C.c_float), ("env_offset", C.c_int64), ("seed", C.c_uint64), ("w", C.c_double * 11),
         ("exp_neg", C.c_void_p), ("coverage", C.c_void_p), ("W", C.c_void_p), ("D", C.c_void_p),
         ("row_ptr", C.c_void_p), ("col", C.c_void_p)]
 
@@ -131,6 +131,7 @@ class CBatch:
         c.reward_mode, c.auto_reset, c.resample_graph = int(cfg.reward_mode == "fp32"), int(auto_reset), int(resample_graph)
         c.num_graphs, c.nnz_stride, c.n_exp, c.n_cov = G, stride, len(self._exp), len(self._cov)
         c.env_offset, c.seed = int(env_offset), int(seed) & 0xFFFFFFFFFFFFFFFF
+        c.reveal_skip_prob = float(cfg.reveal_skip_prob)
         for i, k in enumerate(so.REWARD_WEIGHT_NAMES):
             c.w[i] = float(cfg.reward_weights[k])
         c.exp_neg, c.coverage = self._exp.ctypes.data, self._cov.ctypes.data
@@ -152,11 +153,21 @@ class CBatch:
         self._out = SyoOut(*[None if a is None else a.ctypes.data for a in (
             self._reward, self._term, self._trunc, self._winner, self._mask, self._nf)])
         self._actions = z((B, A), np.int64)
+        self.reset(start_positions, graph_id)
+
+    def set_seed(self, seed):
+        """new Philox key for every later draw (the handle's sy_set_seed; the C oracle reads its config on every call)"""
+        self._c.seed = int(seed) & 0xFFFFFFFFFFFFFFFF
+        self.seed = int(seed)
+
+    def reset(self, start_positions=None, graph_id=None):
+        """every env restarts at episode 0 (start nodes Philox(seed; env, 0) unless given), then observes"""
+        B, A = self.B, self.A
         ip = None if start_positions is None else np.ascontiguousarray(start_positions, dtype=np.int32).reshape(B, A)
         gi = None if graph_id is None else np.ascontiguousarray(graph_id, dtype=np.int32).reshape(B)
-        lib.syo_reset_all(C.byref(c), B, C.byref(self._state), None if ip is None else ip.ctypes.data,
-                          None if gi is None else gi.ctypes.data)
-        lib.syo_observe(C.byref(c), B, C.byref(self._state), C.byref(self._out))
+        _lib().syo_reset_all(C.byref(self._c), B, C.byref(self._state), None if ip is None else ip.ctypes.data,
+                             None if gi is None else gi.ctypes.data)
+        _lib().syo_observe(C.byref(self._c), B, C.byref(self._state), C.byref(self._out))
 
     # -- OracleBatch surface
     def step(self, actions):

@@ -12,6 +12,7 @@ device raises.
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
 from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
@@ -416,6 +417,8 @@ class BatchedScotlandYardEnv:
         self._state.belief_hint = _ptr(hint)
 
     def set_seed(self, seed: int):
+        """New Philox key (its low 64 bits; -1 is 2^64 - 1) for every later draw: start nodes and graphs of (auto-)resets,
+        reveal skips and the random actions.  Rollout graphs captured before refuse to replay."""
         self.seed = int(seed)
         self.config.seed = self.seed & 0xFFFFFFFFFFFFFFFF
         _cabi.check(self._lib.sy_set_seed(self._handle, self.config.seed))
@@ -605,7 +608,9 @@ class BatchedScotlandYardEnv:
         `graph.replay()` continues the rollout with fresh draws (sy_rollout_random_dev).  Small batches are
         launch-latency bound; replaying a graph removes most of that.  Returns (graph, counter tensor).  The captured
         launches assume that no observations are pending (what holds when this returns): call `flush_observations()`
-        before a replay that follows `step_deferred`."""
+        before a replay that follows `step_deferred`.  The graph keeps the Philox key and mechanism groups of its
+        capture, so it refuses to replay after `set_seed` (a `reset(seed=...)` or a `load_state_dict` with another seed
+        too) or `set_mechanisms`: capture it again."""
         if not self._is_reset:
             raise _cabi.SyError("step() before reset()")
         self.flush_observations()
@@ -894,41 +899,92 @@ class BatchedScotlandYardEnv:
             if self.group_stats_vec is not None:
                 self.group_stats_vec.zero_()
 
+    _STATE_TENSORS = ("pos", "money", "timestep", "graph_id", "episode", "done", "visits", "belief_map", "action_mask",
+                      "node_features", "agent_budget", "mrx_revealed", "stats_vec", "group_stats_vec")
+    _STATE_SCALARS = ("seed", "sample_counter", "env_offset", "graph_pool_sha256")
+
+    def _state_keys(self):
+        keys = {k for k in self._STATE_TENSORS if getattr(self, k) is not None} | set(self._STATE_SCALARS)
+        return keys | ({"group_id"} if self._group_id is not None else set())
+
+    def _graph_pool_digest(self) -> torch.Tensor:
+        """uint8 [32]: SHA-256 over every pool graph's node count, edge links and edge weights"""
+        h = hashlib.sha256()
+        for g in self.graphs:
+            links, weights = np.asarray(g.edge_links, dtype=np.int64), np.asarray(g.edges, dtype=np.int64)
+            h.update(np.asarray([g.num_nodes, len(weights)], dtype=np.int64).tobytes())
+            h.update(np.ascontiguousarray(links).tobytes())
+            h.update(np.ascontiguousarray(weights).tobytes())
+        return torch.frombuffer(bytearray(h.digest()), dtype=torch.uint8)
+
     def state_dict(self) -> Dict[str, torch.Tensor]:
-        keys = ["pos", "money", "timestep", "graph_id", "episode", "done", "visits", "belief_map", "action_mask",
-                "node_features", "agent_budget", "mrx_revealed", "stats_vec"]
+        """A checkpoint of the batch: clones of the state, the dense observations (the belief map included), the
+        statistics (folded first; per group and the group assignment while mechanism groups are set), and as CPU int64
+        tensors the Philox key (`seed`, the int64 view of its 64 bits), the sampler counter of `sample_actions` /
+        `rollout_random` / `HeuristicPolicy.act`, `env_offset`, and `graph_pool_sha256` (uint8 [32], a digest of the
+        pool).  Pending observations of `step_deferred` are flushed first, so the dict describes the current state.
+        Callers' own counters (policy step counters, the counter tensor of `capture_rollout`, `HeuristicPolicy.last_seen`)
+        are not in it.  `torch.save` / `torch.load` round-trip it."""
+        self.flush_observations()
         self._fold_stats()
-        sd = {k: getattr(self, k).clone() for k in keys if getattr(self, k) is not None}
-        if self._group_id is not None:  # mechanism groups: the assignment and the per-group statistics
+        sd = {k: getattr(self, k).clone() for k in self._STATE_TENSORS if getattr(self, k) is not None}
+        if self._group_id is not None:  # mechanism groups: the assignment
             sd["group_id"] = self._group_id.clone()
-            if self.group_stats_vec is not None:
-                sd["group_stats_vec"] = self.group_stats_vec.clone()
+        seed = self.config.seed
+        sd["seed"] = torch.tensor(seed - (1 << 64) if seed >= 1 << 63 else seed, dtype=torch.int64)
+        sd["sample_counter"] = torch.tensor(self._sample_counter, dtype=torch.int64)
+        sd["env_offset"] = torch.tensor(self.env_offset, dtype=torch.int64)
+        sd["graph_pool_sha256"] = self._graph_pool_digest()
         return sd
 
     def load_state_dict(self, sd: Dict[str, torch.Tensor]):
-        """Restore a `state_dict`.  One taken while mechanism groups were set needs the same groups set first (with
-        `set_mechanisms`).  Mechanism groups cannot be resumed mid-episode: after `set_mechanisms` the library requires a
-        full `reset()` before the next step, which starts new episodes -- what carries over is the statistics, the
-        per-group ones included."""
-        if ("group_id" in sd) != (self._group_id is not None) or (
-                "group_id" in sd and not torch.equal(sd["group_id"].to(self._group_id.device), self._group_id)):
+        """Restore a `state_dict`: the state, observations and statistics, the Philox key (`set_seed`) and the sampler
+        counter, so that the batch continues exactly as the one that was saved.  Raises ValueError, before anything is
+        changed, when the dict comes from a handle with another `env_offset`, graph pool, batch size, node or agent
+        count, node-feature type, or set of keys (belief map, statistics, mechanism groups on in one and off in the
+        other).  Pending observations are flushed and the library's statistics accumulators folded and discarded first,
+        so rewinding a handle to an earlier dict counts the replayed steps once.
+        One taken while mechanism groups were set needs the same groups set first (with `set_mechanisms`).  In the same
+        handle it then resumes mid-episode; in another handle, mechanism groups cannot be resumed mid-episode: after
+        `set_mechanisms` the library requires a full `reset()` before the next step, which starts new episodes -- what
+        carries over is the statistics, the per-group ones included."""
+        want = self._state_keys()
+        if set(sd) != want:
+            raise ValueError(f"the state dict's keys differ from this env's: missing {sorted(want - set(sd))}, "
+                             f"unexpected {sorted(set(sd) - want)}")
+        if int(sd["env_offset"]) != self.env_offset:
+            raise ValueError(f"the state dict was taken at env_offset {int(sd['env_offset'])}, this env has {self.env_offset}")
+        if not torch.equal(sd["graph_pool_sha256"].cpu(), self._graph_pool_digest()):
+            raise ValueError("the state dict was taken on another graph pool")
+        if "group_id" in sd and not torch.equal(sd["group_id"].to(self._group_id.device), self._group_id):
             raise ValueError("the state dict's mechanism groups differ from this env's: set_mechanisms() first")
-        for k, v in sd.items():
-            if k != "group_id":
-                getattr(self, k).copy_(v)
+        for k in want & set(self._STATE_TENSORS):
+            mine = getattr(self, k)
+            if tuple(sd[k].shape) != tuple(mine.shape) or sd[k].dtype != mine.dtype:
+                raise ValueError(f"state dict entry {k!r} is {sd[k].dtype} {tuple(sd[k].shape)}, this env has "
+                                 f"{mine.dtype} {tuple(mine.shape)}")
+        self.flush_observations()
+        self._fold_stats()  # what the kernels accumulated since the last fold belongs to the state being replaced
+        for k in want & set(self._STATE_TENSORS):
+            getattr(self, k).copy_(sd[k])
+        self.set_seed(int(sd["seed"]) & 0xFFFFFFFFFFFFFFFF)
+        self._sample_counter = int(sd["sample_counter"])
         self._is_reset = True
 
 
 class _RolloutGraph:
-    """A captured rollout graph (torch.cuda.CUDAGraph) that refuses to replay once the env's mechanism groups changed:
-    its launches carry the groups -- and the kernels chosen for them -- of the time it was captured."""
+    """A captured rollout graph (torch.cuda.CUDAGraph) that refuses to replay once the env's mechanism groups or its
+    seed changed: its launches carry the groups -- and the kernels chosen for them -- and the Philox key of the time it
+    was captured."""
 
     def __init__(self, graph, env):
-        self.graph, self._env, self._generation = graph, env, env._groups_generation
+        self.graph, self._env, self._generation, self._seed = graph, env, env._groups_generation, env.config.seed
 
     def replay(self):
         if self._env._groups_generation != self._generation:
             raise _cabi.SyError("the mechanism groups changed since this rollout graph was captured: capture it again")
+        if self._env.config.seed != self._seed:
+            raise _cabi.SyError("the seed changed since this rollout graph was captured: capture it again")
         self.graph.replay()
 
     def __getattr__(self, name):
