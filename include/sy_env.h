@@ -143,7 +143,12 @@ typedef struct SyState {
 /* Dynamic observation tensors written every reset/step (yard.py:271-335).  Static graph
  * tensors (adjacency_matrix, edge_index, edge_features) are per-graph and are built once by
  * the host from the same CSR; belief_map is SyState.belief; agent_position is SyState.pos.
- * Absent agents (see SyState) have all-zero action_mask rows and node_features columns and agent_budget 0.0f. */
+ * Absent agents (see SyState) have all-zero action_mask rows and node_features columns and agent_budget 0.0f.
+ * Precondition of the float32 node_features: the buffer passed to a step must hold what the library last wrote there for
+ * the state passed with it.  A step into the buffer the handle's previous call completed, for the same SyState.pos and
+ * SyObs.mrx_revealed, only clears the entry state's ones and stores the new ones (the rest of the one-hot is already
+ * zero); any other buffer is written whole.  A caller that writes into node_features, pos or mrx_revealed outside the
+ * library must sy_reset those envs before the next step (restoring all three together from one checkpoint is fine). */
 typedef struct SyObs {
   uint64_t struct_bytes; /* = sizeof(SyObs) */
   uint8_t* action_mask;  /* [B, A, N] bool */

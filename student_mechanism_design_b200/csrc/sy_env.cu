@@ -149,6 +149,9 @@ struct Params {
   // the SM with one cp.async.bulk.  0 = the LSU writers (unaligned caller buffers, or selected with sy_set_option)
   int wr_bulk, wr_c_mask, wr_c_nf, wr_img_bytes;
   int nf_prefilled;  // float32 node_features were zero-filled by the logic kernel (bulk stores): the writers only store the ones
+  // incremental node_features (two-kernel step, float32): the buffer holds the one-hot of the entry state, the dynamics
+  // kernel zeroes the granules of nf_incr floats (8 or 4) that hold its ones, the writers store only the new ones; 0 = off
+  int nf_incr;
   int f_off_sbuf, f_sbuf_stride, f_off_zero, f_off_imgs;  // fused kernel: staged tile state (x2), zero page, chunk images
   int f_off_nbr4;  // fused kernel: packed neighbour table [N] uint4 + flag (after the staged CSR)
   int wr_epc;      // fused kernel fast geometry: whole envs per chunk (0: chunks cut through envs / more than 32 pairs)
@@ -341,6 +344,15 @@ __device__ __forceinline__ void store_obs16(uint4* ptr, uint4 v) {
 #else
   __stwt(ptr, v);
 #endif
+}
+// 32-byte store (one whole DRAM sector: no read-modify-write when the line has already left L2), eight words w[k]
+__device__ __forceinline__ void store_obs32(void* ptr, const unsigned (&w)[8], bool streaming) {
+  if (streaming)
+    asm volatile("st.global.cs.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};\n" ::"l"(ptr), "r"(w[0]), "r"(w[1]), "r"(w[2]),
+                 "r"(w[3]), "r"(w[4]), "r"(w[5]), "r"(w[6]), "r"(w[7]) : "memory");
+  else
+    asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};\n" ::"l"(ptr), "r"(w[0]), "r"(w[1]), "r"(w[2]),
+                 "r"(w[3]), "r"(w[4]), "r"(w[5]), "r"(w[6]), "r"(w[7]) : "memory");
 }
 __device__ __forceinline__ void cp_async4(void* smem, const void* gmem) {  // LDGSTS: global -> shared, no staging register
   const unsigned sa = (unsigned)__cvta_generic_to_shared(smem);
@@ -760,6 +772,28 @@ __device__ __forceinline__ void logic_tile(const Params& p, LogicSmem<MAXA>& sm,
     sm.reset_gid[lane] = p.resample_graph ? philox_graph_choice(p, env_id, ep) : g;
     philox_start_positions(p, env_id, ep, sm.reset_pos + lane * HS, sm.dmat + lane * HS);  // (absent agents: unused)
     PHASE_SPAN(9, tp1);  // (lane-divergent branch: no warp-level synchronisation in here)
+  }
+  if (LAGT == 0 && p.nf_incr) {  // (the lagged / rollout kernels never take it: no code in them)
+    // incremental node_features (plain two-kernel step only): the buffer holds the one-hot of the ENTRY state, so the
+    // granules that hold its ones are zeroed here and the observation kernel stores only the granules of the new ones
+    // (the kernel boundary orders the two).  Entry positions and reveal flags are re-read from global memory: warp 0
+    // moves the smem copy, and P4 overwrites both arrays only after the barriers below.  Fire-and-forget stores from the
+    // warps that are idle in P1; zeroing any granule is safe, the buffer holds nothing but zeros and entry ones.
+    constexpr int W0 = LOGIC_WARPS > 2 ? 2 : LOGIC_WARPS - 1;
+    if (warp >= W0) {
+      for (int i = tid - W0 * 32; i < nEnv * A; i += LOGIC_THREADS - W0 * 32) {
+        const int e = (i * p.inv_A) >> 16, a = i - e * A;
+        const int u = p.st.pos[(size_t)b0 * A + i];
+        if (u < 0 || (a == 0 && p.ob.mrx_revealed[b0 + e] < 0)) continue;  // absent agent / hidden MrX: no one written
+        float* g = p.ob.node_features + ((((size_t)(b0 + e) * N + u) * A + a) & ~(size_t)(p.nf_incr - 1));
+        if (p.nf_incr == 8) {
+          const unsigned z[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+          store_obs32(g, z, false);
+        } else {
+          *reinterpret_cast<uint4*>(g) = make_uint4(0, 0, 0, 0);
+        }
+      }
+    }
   }
   named_barrier(BAR, LOGIC_THREADS);
   PHASE_MARK(1);
@@ -1183,28 +1217,29 @@ __device__ __forceinline__ void warp_copy_bytes(uint8_t* dst, const uint8_t* src
 // (yard.py:279-290).  The region is zero-filled with 16-byte stores; lane a then overwrites, with one full 16-byte
 // store, the chunk that holds agent a's one (assembled in registers from all agents that fall into it).  Measured:
 // rewriting a handful of whole chunks costs nothing, whereas byte-sized ones after the fill cost 60 %.
-// the same after a completed zero fill of the region (p.nf_prefilled): only the ones -- whole granules when the env rows
-// are granule-aligned, single floats otherwise
+// the same where the rest of the region is already zero -- after the split step's fill (p.nf_prefilled) or after the
+// dynamics kernel retired the entry one-hot (p.nf_incr): only the granules that hold a one, each written whole (all
+// agents that share it merged): 32-byte sectors when the env rows are 32-byte aligned, 16-byte chunks when they are
+// 16-byte aligned, single floats otherwise
 __device__ __forceinline__ void warp_write_node_feature_ones(float* nf, int n, const int* fpos, int A, int lane) {
   if (lane >= A || fpos[lane] < 0) return;
-  if ((n & 3) || (reinterpret_cast<uintptr_t>(nf) & 15u)) {
+  const uintptr_t base = reinterpret_cast<uintptr_t>(nf);
+  const int gs = ((n & 7) == 0 && (base & 31u) == 0) ? 3 : ((n & 3) == 0 && (base & 15u) == 0) ? 2 : 0;  // log2 floats
+  if (gs == 0) {
     nf[fpos[lane]] = 1.0f;
     return;
   }
-  const int myc = fpos[lane] >> 2;
-  uint4 v = make_uint4(0, 0, 0, 0);
+  const int myg = fpos[lane] >> gs;
+  unsigned bits = 0;  // floats of the granule that hold a one
   for (int a = 0; a < A; ++a) {
     const int f = fpos[a];
-    if (f >= 0 && (f >> 2) == myc) {
-      const unsigned one = 0x3f800000u;
-      const int sub = f & 3;
-      v.x = sub == 0 ? one : v.x;
-      v.y = sub == 1 ? one : v.y;
-      v.z = sub == 2 ? one : v.z;
-      v.w = sub == 3 ? one : v.w;
-    }
+    if (f >= 0 && (f >> gs) == myg) bits |= 1u << (f & ((1 << gs) - 1));
   }
-  store_obs16(reinterpret_cast<uint4*>(nf) + myc, v);
+  unsigned w[8];
+#pragma unroll
+  for (int k = 0; k < 8; ++k) w[k] = ((bits >> k) & 1u) ? 0x3f800000u : 0u;
+  if (gs == 3) store_obs32(nf + ((size_t)myg << 3), w, true);
+  else store_obs16(reinterpret_cast<uint4*>(nf) + myg, make_uint4(w[0], w[1], w[2], w[3]));
 }
 
 __device__ __forceinline__ void warp_write_node_features(float* nf, int n, const int* fpos /*smem, A entries, -1 = none*/,
@@ -1380,7 +1415,7 @@ __device__ __forceinline__ void writer_role(const Params& p, unsigned char* dyn,
       __syncwarp();
       warp_copy_bytes(nf8, img8, N * A, lane);
     } else {
-      if constexpr (PREFILLED) warp_write_node_feature_ones(nf, N * A, fpos, A, lane);
+      if (PREFILLED || (LAGT == 0 && p.nf_incr)) warp_write_node_feature_ones(nf, N * A, fpos, A, lane);
       else warp_write_node_features(nf, N * A, fpos, A, lane);
     }
     __syncwarp();
@@ -3189,6 +3224,15 @@ struct SyEnv {
   int fill_grid = 0;
   int opt_writer = SY_WRITER_LSU;  // sy_set_option(SY_OPT_WRITER_PATH) for the stand-alone observe kernel (sy_reset, two-kernel sy_step)
   int bel_warps = BEL_WARPS, wr_warps = WR_WARPS;  // role split of the observe kernel for this pool
+  // The float32 node_features the library last completed an observation write into, with the state it describes: the
+  // buffer holds onehot(*pos, *mrx_revealed) (include/sy_env.h, SyObs).  A plain step whose buffers match it zeroes only
+  // the entry ones and writes only the new ones (Params.nf_incr).  Cleared on entry of every call that launches work,
+  // set when the call completes such a write (an error or pending observations leave it clear).
+  struct NfWritten {
+    const float* nf = nullptr;
+    const int32_t* pos = nullptr;
+    const int32_t* revealed = nullptr;
+  } nf_written;
   size_t obs_smem = 0;  // dynamic smem of the observe kernel: belief scratch + writer staging
   // software-pipelined steps (sy_step_deferred): the dense observations of the current state have not been written yet;
   // the next dynamics launch carries them (sy_step_lagged_kernel), sy_flush_observations / any plain call writes them
@@ -3561,6 +3605,30 @@ int check_obs(const SyObs* ob) {
   if (!ob || !ob->action_mask || (!ob->node_features && !ob->node_features_u8) || !ob->agent_budget || !ob->mrx_revealed)
     return fail(SY_ERR_INVALID_ARGUMENT, "SyObs has NULL members");
   return SY_OK;
+}
+
+// granule (floats) of an incremental node_features write into these buffers -- 8 (32-byte sectors) or 4 (16-byte
+// chunks), every env row aligned to it -- or 0: the full one-hot.  Only where the library last completed a write of the
+// float32 one-hot of exactly this state into exactly this buffer (SyEnv.nf_written).
+int nf_incr_granule(const SyEnv* e, const SyState* st, const SyObs* ob) {
+  const SyEnv::NfWritten& w = e->nf_written;
+  if (!ob || ob->node_features_u8 || !ob->node_features || w.nf != ob->node_features || w.pos != st->pos ||
+      w.revealed != ob->mrx_revealed)
+    return 0;
+  const size_t n = (size_t)e->cfg.num_nodes * e->A;
+  const uintptr_t base = reinterpret_cast<uintptr_t>(ob->node_features);
+  if (n % 8 == 0 && base % 32 == 0) return 8;
+  if (n % 4 == 0 && base % 16 == 0) return 4;
+  return 0;
+}
+// the call completed an observation write of the state in st into ob (the u8 one-hot leaves no float32 buffer behind)
+void nf_written_set(SyEnv* e, const SyState* st, const SyObs* ob) {
+  e->nf_written = SyEnv::NfWritten{};
+  if (ob && ob->node_features && !ob->node_features_u8) {
+    e->nf_written.nf = ob->node_features;
+    e->nf_written.pos = st->pos;
+    e->nf_written.revealed = ob->mrx_revealed;
+  }
 }
 
 }  // namespace
@@ -4024,6 +4092,9 @@ int sy_reset(SyEnv* e, const uint8_t* reset_mask, const int32_t* init_pos, const
   p.init_pos = init_pos;
   p.init_gid = init_gid;
   p.restart = restart;
+  // a partial reset keeps the record only for the buffer it describes (a reset of every env rewrites it whole)
+  const bool nf_kept = !reset_mask || (!e->obs_pending && nf_incr_granule(e, st, ob) != 0);
+  e->nf_written = SyEnv::NfWritten{};
   CUDA_TRY(cudaSetDevice(e->cfg.device));
   cudaStream_t s = (cudaStream_t)stream;
   if (e->obs_pending) {  // deferred observations (belief propagation of the last step) first: a partial reset keeps the other envs
@@ -4053,6 +4124,7 @@ int sy_reset(SyEnv* e, const uint8_t* reset_mask, const int32_t* init_pos, const
   launch_observe(e, p, (unsigned)((p.B + TILE - 1) / TILE), s);
   g_launches++;
   CUDA_TRY(cudaGetLastError());
+  if (nf_kept) nf_written_set(e, st, ob);
   return SY_OK;
 }
 
@@ -4115,6 +4187,8 @@ int step_impl(SyEnv* e, const int64_t* actions, const int32_t* actions32, const 
   p.actions = reinterpret_cast<const long long*>(actions);
   p.actions32 = actions32;
   p.actions16 = actions16;
+  const int nf_gran = e->obs_pending ? 0 : nf_incr_granule(e, st, ob);  // before anything is launched
+  e->nf_written = SyEnv::NfWritten{};
   CUDA_TRY(cudaSetDevice(e->cfg.device));
   cudaStream_t s = (cudaStream_t)stream;
   const unsigned grid = (unsigned)((p.B + TILE - 1) / TILE);
@@ -4157,6 +4231,7 @@ int step_impl(SyEnv* e, const int64_t* actions, const int32_t* actions32, const 
       g_launches++;
       CUDA_TRY(cudaGetLastError());
       e->obs_pending = false;
+      nf_written_set(e, st, ob);
     }
     return SY_OK;
   }
@@ -4183,6 +4258,7 @@ int step_impl(SyEnv* e, const int64_t* actions, const int32_t* actions32, const 
     CUDA_TRY(cudaGetLastError());
     if (after_logic) CUDA_TRY(cudaEventRecord(after_logic, s));
     if (fused_sampled) *fused_sampled = true;
+    nf_written_set(e, st, ob);
     return SY_OK;
   }
   // Split step: the state-independent zero fill of float32 node_features (63 % of the bytes) goes to the TMA engine in
@@ -4210,6 +4286,10 @@ int step_impl(SyEnv* e, const int64_t* actions, const int32_t* actions32, const 
     CUDA_TRY(cudaGetLastError());
     p.nf_prefilled = 1;
     ls = e->split_stream;
+  } else if (nf_gran && !p.wr_bulk && !p.dbg_skip) {
+    // the buffer holds the one-hot of the entry state: the dynamics kernel zeroes its granules, the writers store only
+    // the new ones (every other path above, and a fresh or different buffer, writes the whole one-hot)
+    p.nf_incr = nf_gran;
   }
   if (!(p.dbg_skip & 32)) launch_logic(e, p, grid, ls);
   g_launches++;
@@ -4231,11 +4311,13 @@ int step_impl(SyEnv* e, const int64_t* actions, const int32_t* actions32, const 
     g_launches++;
     CUDA_TRY(cudaGetLastError());
     if (p.belief_on) CUDA_TRY(cudaStreamWaitEvent(s, e->ev_split_belief, 0));
+    nf_written_set(e, st, ob);
     return SY_OK;
   }
   if (!(p.dbg_skip & 16)) launch_observe(e, p, grid, s);
   g_launches++;
   CUDA_TRY(cudaGetLastError());
+  if (!p.dbg_skip) nf_written_set(e, st, ob);
   return SY_OK;
 }
 
@@ -4311,11 +4393,13 @@ int sy_flush_observations(SyEnv* e, const SyState* st, const SyObs* ob, sy_strea
   if (rc) return rc;
   if ((rc = check_obs(ob))) return rc;
   p.out.stats = e->pending_stats;
+  e->nf_written = SyEnv::NfWritten{};
   CUDA_TRY(cudaSetDevice(e->cfg.device));
   launch_observe(e, p, (unsigned)((p.B + TILE - 1) / TILE), (cudaStream_t)stream);
   g_launches++;
   CUDA_TRY(cudaGetLastError());
   e->obs_pending = false;
+  nf_written_set(e, st, ob);
   return SY_OK;
 }
 
@@ -4673,9 +4757,11 @@ int rollout_one_launch(SyEnv* e, int32_t num_steps, int64_t* actions, uint32_t n
   p.next_counter_base = next_counter_base;
   CUDA_TRY(cudaSetDevice(e->cfg.device));
   e->aux_after_logic = false;
+  e->nf_written = SyEnv::NfWritten{};
   rollout_fn(e, p.grp_n > 0)<<<(unsigned)((p.B + TILE - 1) / TILE), lagged_threads(e), e->obs_smem, s>>>(p, (int)num_steps);
   g_launches++;
   CUDA_TRY(cudaGetLastError());
+  nf_written_set(e, st, ob);  // (the last step's observations are written in the launch)
   return SY_OK;
 }
 bool one_launch_rollout(const SyEnv* e, const SyObs* ob) {

@@ -943,7 +943,9 @@ class BatchedScotlandYardEnv:
         changed, when the dict comes from a handle with another `env_offset`, graph pool, batch size, node or agent
         count, node-feature type, or set of keys (belief map, statistics, mechanism groups on in one and off in the
         other).  Pending observations are flushed and the library's statistics accumulators folded and discarded first,
-        so rewinding a handle to an earlier dict counts the replayed steps once.
+        so rewinding a handle to an earlier dict counts the replayed steps once.  `node_features` is restored together
+        with `pos` and `mrx_revealed`, so it holds the one-hot of the restored state: the next step may update it in
+        place (include/sy_env.h, SyObs) -- a caller that writes any of the three outside the library must reset() those envs.
         One taken while mechanism groups were set needs the same groups set first (with `set_mechanisms`).  In the same
         handle it then resumes mid-episode; in another handle, mechanism groups cannot be resumed mid-episode: after
         `set_mechanisms` the library requires a full `reset()` before the next step, which starts new episodes -- what
