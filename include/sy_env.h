@@ -194,11 +194,8 @@ void sy_destroy(SyEnv* env);
  *                       kernels instead; an explicit SY_STEP_FUSED keeps the fused kernel there too.)
  *   SY_OPT_WRITER_PATH  writers of the two-kernel path's observation kernel: SY_WRITER_LSU (default) = 16-byte
  *                       streaming stores; SY_WRITER_BULK = zero-page bulk fill + chunk images + bulk stores.
- *   SY_OPT_NF_FILL      0 (default).  1: split step for batches of >= 8192 envs with float32 node_features: the zero
- *                       fill of node_features (63 % of a step's bytes, independent of the state) is handed to the TMA
- *                       engine by its own small kernel NEXT TO the dynamics kernel (second stream), then the belief
- *                       propagation and the writers of the ones run as two concurrent kernels; all joined on the
- *                       caller's stream before sy_step returns (events; capturable).  Measured slower (DESIGN.md 4c).
+ *   SY_OPT_NF_FILL      0 or 1, accepted and ignored: the split step it selected is gone (it never changed results,
+ *                       and measured slower than the default step, DESIGN.md 4c).
  *   SY_OPT_LAGGED_KERNEL SY_LAGGED_AUTO (default): a deferred step with pending observations is ONE launch
  *                       (sy_step_lagged_kernel: the pending observation roles + the dynamics warps of the next step in
  *                       the same CTA) and sy_rollout_random* step deferred WHEN the batch's 32-env tiles fit one wave of
@@ -400,8 +397,8 @@ int sy_stats(SyEnv* env, int64_t* stats, sy_stream_t stream);
  * (agent_money), reveal schedule (reveal_interval, reveal_skip_prob), through sy_set_group_tolls the toll, and through
  * sy_set_group_rules the number of police and the episode horizon (max_timestep), each bounded by the config's.
  * Group membership enters no random stream, so a group equal to the config reproduces a handle without groups bit for
- * bit.  Every step path runs with groups (its GROUPS instantiation) except the split step of SY_OPT_NF_FILL, which acts
- * as off while groups are set (results are the same).  The statistics are also summed per group (sy_group_stats).
+ * bit.  Every step path runs with groups (its GROUPS instantiation).  The statistics are also summed per group
+ * (sy_group_stats).
  * The library's group buffers are allocated once and updated in place, but a CUDA graph captured before a
  * sy_set_groups call carries the groups of its capture: recapture it after changing the groups. */
 #define SY_MAX_GROUPS 1024

@@ -73,15 +73,6 @@ constexpr int TILE = 32;       // envs per observe CTA / per logic warp (lane = 
 #ifndef SY_WR_WARPS
 #define SY_WR_WARPS 8
 #endif
-#ifndef SY_STORE_HINT
-#define SY_STORE_HINT 0
-#endif
-#ifndef SY_NF_SCALAR_ONES
-#define SY_NF_SCALAR_ONES 0  // 1: node_features ones as 4-byte stores after the zero fill instead of merged 16-byte chunks
-#endif
-#ifndef SY_BULK_HINT
-#define SY_BULK_HINT 0  // 1: L2 evict_first policy on the bulk stores
-#endif
 #ifndef SY_BULK_IMG_BUDGET
 #define SY_BULK_IMG_BUDGET 25344  // bytes of shared memory for the bulk writers' zero page and chunk images of a CTA
 #endif
@@ -148,7 +139,7 @@ struct Params {
   // wr_c_mask / wr_c_nf bytes (multiples of 16); each chunk is assembled in a per-warp shared-memory image and leaves
   // the SM with one cp.async.bulk.  0 = the LSU writers (unaligned caller buffers, or selected with sy_set_option)
   int wr_bulk, wr_c_mask, wr_c_nf, wr_img_bytes;
-  int nf_prefilled;  // float32 node_features were zero-filled by the logic kernel (bulk stores): the writers only store the ones
+  int unused0;  // keeps the offsets of the fields below: shifting them changes how the kernels pair their parameter loads
   // incremental node_features (two-kernel step, float32): the buffer holds the one-hot of the entry state, the dynamics
   // kernel zeroes the granules of nf_incr floats (8 or 4) that hold its ones, the writers store only the new ones; 0 = off
   int nf_incr;
@@ -334,17 +325,7 @@ __device__ __forceinline__ double exp_neg(const Tables& tb, int d) {
 // small device helpers
 // ---------------------------------------------------------------------------------------------
 // streaming 16-byte store of the observation arrays (written once per step, read by the policy much later)
-__device__ __forceinline__ void store_obs16(uint4* ptr, uint4 v) {
-#if SY_STORE_HINT == 0
-  __stcs(ptr, v);
-#elif SY_STORE_HINT == 1
-  *ptr = v;
-#elif SY_STORE_HINT == 2
-  __stcg(ptr, v);
-#else
-  __stwt(ptr, v);
-#endif
-}
+__device__ __forceinline__ void store_obs16(uint4* ptr, uint4 v) { __stcs(ptr, v); }
 // 32-byte store (one whole DRAM sector: no read-modify-write when the line has already left L2), eight words w[k]
 __device__ __forceinline__ void store_obs32(void* ptr, const unsigned (&w)[8], bool streaming) {
   if (streaming)
@@ -383,14 +364,7 @@ __device__ __forceinline__ unsigned long long warp_sum_u64(unsigned mask, unsign
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory"); }
 __device__ __forceinline__ void bulk_store(void* gdst, const void* ssrc, unsigned bytes) {
   const unsigned sa = (unsigned)__cvta_generic_to_shared(ssrc);
-#if SY_BULK_HINT == 1
-  unsigned long long pol;
-  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;\n" : "=l"(pol));
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;\n" ::"l"(gdst), "r"(sa), "r"(bytes), "l"(pol)
-               : "memory");
-#else
   asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;\n" ::"l"(gdst), "r"(sa), "r"(bytes) : "memory");
-#endif
 }
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;\n" ::: "memory"); }
 template <int PENDING>
@@ -1099,36 +1073,6 @@ __global__ void __launch_bounds__(LOGIC_THREADS, SY_LOGIC_MIN_CTAS) sy_logic_ker
 }
 
 // ---------------------------------------------------------------------------------------------
-// fill kernel: the zero fill of the float32 node_features array is 63 % of a step's bytes and does not depend on the
-// state, while the dynamics and the belief propagation are latency / issue bound and leave HBM idle.  In the split step
-// (step_impl) this kernel therefore runs from the first microsecond of the step NEXT TO the dynamics kernel: a handful
-// of threads per SM hand the whole array to the TMA engine (cp.async.bulk from a shared-memory zero page: no LSU, no
-// registers, ~2 % of the issue slots) and wait for completion; the observation writers later only store the 16-byte
-// granules that hold a one (p.nf_prefilled).  Micro-benchmark (tools/exp/tma_fill.cu): 6.1-6.2 TB/s with 1 CTA per SM.
-// ---------------------------------------------------------------------------------------------
-#ifndef SY_FILL_PAGE
-#define SY_FILL_PAGE 8192
-#endif
-constexpr int FILL_THREADS = 64;
-#ifndef SY_SPLIT_MIN_ENVS
-#define SY_SPLIT_MIN_ENVS 8192
-#endif
-constexpr int SPLIT_MIN_ENVS = SY_SPLIT_MIN_ENVS;  // smaller batches are launch-latency bound: two plain launches
-__global__ void __launch_bounds__(FILL_THREADS) sy_fill_kernel(uint8_t* dst, size_t bytes) {
-  __shared__ __align__(128) uint8_t zero_page[SY_FILL_PAGE];
-  for (int i = threadIdx.x * 16; i < SY_FILL_PAGE; i += FILL_THREADS * 16) *reinterpret_cast<uint4*>(zero_page + i) = make_uint4(0, 0, 0, 0);
-  fence_proxy_async_smem();
-  __syncthreads();
-  const size_t body = bytes & ~(size_t)15;
-  const size_t stride = (size_t)gridDim.x * FILL_THREADS * SY_FILL_PAGE;
-  for (size_t o = ((size_t)blockIdx.x * FILL_THREADS + threadIdx.x) * SY_FILL_PAGE; o < body; o += stride)
-    bulk_store(dst + o, zero_page, (unsigned)min((size_t)SY_FILL_PAGE, body - o));
-  bulk_commit();
-  if (blockIdx.x == 0 && threadIdx.x < (int)(bytes - body)) dst[body + threadIdx.x] = 0;
-  asm volatile("cp.async.bulk.wait_group 0;\n" ::: "memory");  // complete before the kernel ends: the ones follow in stream order
-}
-
-// ---------------------------------------------------------------------------------------------
 // reset kernel (yard.py:80-142): re-initialise the masked envs (same warp = 32 envs layout)
 // ---------------------------------------------------------------------------------------------
 // GROUPS: police budgets, police count and reveal schedule of each env's mechanism group
@@ -1217,10 +1161,9 @@ __device__ __forceinline__ void warp_copy_bytes(uint8_t* dst, const uint8_t* src
 // (yard.py:279-290).  The region is zero-filled with 16-byte stores; lane a then overwrites, with one full 16-byte
 // store, the chunk that holds agent a's one (assembled in registers from all agents that fall into it).  Measured:
 // rewriting a handful of whole chunks costs nothing, whereas byte-sized ones after the fill cost 60 %.
-// the same where the rest of the region is already zero -- after the split step's fill (p.nf_prefilled) or after the
-// dynamics kernel retired the entry one-hot (p.nf_incr): only the granules that hold a one, each written whole (all
-// agents that share it merged): 32-byte sectors when the env rows are 32-byte aligned, 16-byte chunks when they are
-// 16-byte aligned, single floats otherwise
+// the same where the rest of the region is already zero -- after the dynamics kernel retired the entry one-hot
+// (p.nf_incr): only the granules that hold a one, each written whole (all agents that share it merged): 32-byte
+// sectors when the env rows are 32-byte aligned, 16-byte chunks when they are 16-byte aligned, single floats otherwise
 __device__ __forceinline__ void warp_write_node_feature_ones(float* nf, int n, const int* fpos, int A, int lane) {
   if (lane >= A || fpos[lane] < 0) return;
   const uintptr_t base = reinterpret_cast<uintptr_t>(nf);
@@ -1258,13 +1201,6 @@ __device__ __forceinline__ void warp_write_node_features(float* nf, int n, const
 #pragma unroll 4
   for (int i = lane; i < nvec; i += 32) store_obs16(body + i, z);
   __syncwarp();  // orders the zero stores before the chunks below (same warp, same addresses)
-#if SY_NF_SCALAR_ONES
-  // one 4-byte store per agent: no merging of ones that share a chunk (A x A loop) is needed; the lines are still in L2
-  if (lane < A) {
-    const int f0 = fpos[lane] - head;
-    if (fpos[lane] >= 0 && f0 >= 0 && f0 < (nvec << 2)) __stcs(reinterpret_cast<float*>(body) + f0, 1.0f);
-  }
-#else
   if (lane < A) {
     const int f0 = fpos[lane] - head;
     if (fpos[lane] >= 0 && f0 >= 0 && f0 < (nvec << 2)) {
@@ -1284,7 +1220,6 @@ __device__ __forceinline__ void warp_write_node_features(float* nf, int n, const
       store_obs16(body + myc, v);  // (match.any + redux instead of this loop was measured 18 % SLOWER per step: MATCH is slow)
     }
   }
-#endif
 }
 
 // writer warps: stream the dense observations of the tile.  Everything the ones depend on is staged into shared
@@ -1293,7 +1228,7 @@ __device__ __forceinline__ void warp_write_node_features(float* nf, int n, const
 // assembled in a per-warp shared-memory image and copied out, node_features are zero-filled and the (at most A) chunks
 // with a one rewritten whole: no byte-sized stores anywhere (they cost 60 % extra time when tried).  GROUPS: budgets are
 // staged as headroom against each env's group toll (wr_budget).
-template <int WRW, bool PREFILLED = false, int LAGT = 0, int CSRT = 0, int GROUPS = 0>
+template <int WRW, int LAGT = 0, int CSRT = 0, int GROUPS = 0>
 __device__ __forceinline__ void writer_role(const Params& p, unsigned char* dyn, int tile0, int nEnv, int w, int lane,
                                             int* lag_staged = nullptr) {
   const Tables& tb = p.tb;
@@ -1415,7 +1350,7 @@ __device__ __forceinline__ void writer_role(const Params& p, unsigned char* dyn,
       __syncwarp();
       warp_copy_bytes(nf8, img8, N * A, lane);
     } else {
-      if (PREFILLED || (LAGT == 0 && p.nf_incr)) warp_write_node_feature_ones(nf, N * A, fpos, A, lane);
+      if (LAGT == 0 && p.nf_incr) warp_write_node_feature_ones(nf, N * A, fpos, A, lane);
       else warp_write_node_features(nf, N * A, fpos, A, lane);
     }
     __syncwarp();
@@ -2117,17 +2052,14 @@ __device__ __forceinline__ void belief_role(const Params& p, unsigned char* dyn,
 
 // BW belief warps + WRW writer warps.  <8, 8> everywhere the belief hides under the write stream (fast path); the
 // large-N generic belief path is the critical role, there the split is <12, 4> (c4: 82 -> 91 M env-steps/s).
-// WV selects the writers at compile time, so the default kernel carries none of the experimental paths' code or
-// registers: WV_LSU = 16-byte streaming stores (default), WV_BULK = zero-page fill + chunk images through the TMA engine,
-// WV_ONES = node_features were zero-filled by sy_fill_kernel, only the ones are stored (split step).
-// <BW, 0> / <0, WRW>: one role per launch (the split step runs them as two concurrent kernels; the role hand-over
-// barrier of the large-N belief path counts THREADS, so that path keeps both roles in one launch)
-enum { WV_LSU = 0, WV_BULK = 1, WV_ONES = 2 };
+// WV selects the writers at compile time, so the default kernel carries none of the bulk path's code or registers:
+// WV_LSU = 16-byte streaming stores (default), WV_BULK = zero-page fill + chunk images through the TMA engine.
+enum { WV_LSU = 0, WV_BULK = 1 };
 // GROUPS (launched while mechanism groups are set): the writers test each env's moves against its group's toll, and the
 // belief scores at reveal steps are also summed per group
 template <int BW, int WRW, int WV = WV_LSU, int GROUPS = 0>
 __global__ void __launch_bounds__((BW + WRW) * 32) sy_observe_kernel(const Params p) {
-  static_assert((BW + WRW) * 32 == THREADS || BW == 0 || WRW == 0, "the role hand-over barrier counts THREADS");
+  static_assert((BW + WRW) * 32 == THREADS, "the role hand-over barrier counts THREADS");
   extern __shared__ __align__(16) unsigned char dyn[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   int tile0 = blockIdx.x * TILE;
@@ -2147,21 +2079,17 @@ __global__ void __launch_bounds__((BW + WRW) * 32) sy_observe_kernel(const Param
   if (warp < nbw && !p.belief_on) return;
   const long long t0 = FCLK_NOW();
   if (warp < nbw) {
-    if constexpr (BW > 0) {
-      if (!(p.dbg_skip & 4)) belief_role<BW, 0, GROUPS>(p, dyn, tile0, nEnv, warp, lane);
-      if (warp == 0) FCLK_ADD(3, FCLK_NOW() - t0);
-    }
+    if (!(p.dbg_skip & 4)) belief_role<BW, 0, GROUPS>(p, dyn, tile0, nEnv, warp, lane);
+    if (warp == 0) FCLK_ADD(3, FCLK_NOW() - t0);
   } else if (!(p.dbg_skip & 1)) {
-    if constexpr (WRW > 0) {
-      if constexpr (WV == WV_BULK) {
-        if constexpr (WRW >= 2) writer_role_bulk<WRW, GROUPS>(p, dyn, tile0, nEnv, warp - nbw, lane);
-      } else {
-        writer_role<WRW, WV == WV_ONES, 0, 0, GROUPS>(p, dyn, tile0, nEnv, warp - nbw, lane);
-      }
-      if (warp == nbw) {
-        FCLK_ADD(1, FCLK_NOW() - t0);
-        FCLK_ADD(6, 1);
-      }
+    if constexpr (WV == WV_BULK) {
+      if constexpr (WRW >= 2) writer_role_bulk<WRW, GROUPS>(p, dyn, tile0, nEnv, warp - nbw, lane);
+    } else {
+      writer_role<WRW, 0, 0, GROUPS>(p, dyn, tile0, nEnv, warp - nbw, lane);
+    }
+    if (warp == nbw) {
+      FCLK_ADD(1, FCLK_NOW() - t0);
+      FCLK_ADD(6, 1);
     }
   }
 }
@@ -2195,7 +2123,7 @@ __global__ void __launch_bounds__((BW + WRW + LOGIC_WARPS) * 32, 2) sy_step_lagg
     if constexpr (BW > 0) belief_role<BW, NT, GROUPS>(p, dyn, tile0, nEnv, warp, lane);
     if (warp == 0) FCLK_ADD(3, FCLK_NOW() - t0);
   } else if (warp < BW + WRW) {
-    writer_role<WRW, false, NT, CSRT, GROUPS>(p, dyn, tile0, nEnv, warp - BW, lane, &staged_flag);
+    writer_role<WRW, NT, CSRT, GROUPS>(p, dyn, tile0, nEnv, warp - BW, lane, &staged_flag);
     if (warp == BW) FCLK_ADD(1, FCLK_NOW() - t0);
   } else {
     const int* s_rp = reinterpret_cast<const int*>(dyn + p.wr_off_csr);
@@ -2235,7 +2163,7 @@ __global__ void __launch_bounds__((BW + WRW + LOGIC_WARPS) * 32, 2) sy_rollout_l
       }
     } else if (warp < BW + WRW) {
       if (do_obs) {
-        writer_role<WRW, false, NT, CSRT, GROUPS>(p, dyn, tile0, nEnv, warp - BW, lane, &staged_flag);
+        writer_role<WRW, NT, CSRT, GROUPS>(p, dyn, tile0, nEnv, warp - BW, lane, &staged_flag);
       } else {
         if (threadIdx.x == BW * 32) staged_flag = 0;  // nothing staged: the dynamics read the pool tables
         asm volatile("bar.arrive %0, %1;\n" ::"n"(LAG_CSR_BAR), "n"(CSRT) : "memory");
@@ -3218,10 +3146,6 @@ struct SyEnv {
   // wave (launch-latency bound: one launch instead of two, c2 runs 19 % faster), else the dynamics + observation kernels
   // (at 65 536 envs the fused kernel is slower: DESIGN.md section 4c)
   int opt_fused = SY_STEP_AUTO;
-  int opt_fill = 0;   // sy_set_option(SY_OPT_NF_FILL): 1 = split step (fill kernel next to the dynamics, belief next to the writers)
-  cudaStream_t split_stream = nullptr;  // split step: dynamics + belief run here, fill + writers on the caller's stream
-  cudaEvent_t ev_split_start = nullptr, ev_split_logic = nullptr, ev_split_belief = nullptr;
-  int fill_grid = 0;
   int opt_writer = SY_WRITER_LSU;  // sy_set_option(SY_OPT_WRITER_PATH) for the stand-alone observe kernel (sy_reset, two-kernel sy_step)
   int bel_warps = BEL_WARPS, wr_warps = WR_WARPS;  // role split of the observe kernel for this pool
   // The float32 node_features the library last completed an observation write into, with the state it describes: the
@@ -3251,9 +3175,7 @@ struct SyEnv {
   int lag_slots = 0;  // resident CTAs of the lagged kernel (occupancy x SMs)
   int opt_pdl = 0;  // sy_set_option(SY_OPT_PDL): dynamics / observation kernels launched with programmatic stream serialisation
   int opt_rollout_kernel = 1;  // sy_set_option(SY_OPT_ROLLOUT_KERNEL): random rollouts of single-wave batches as ONE launch
-  // mechanism groups (sy_set_groups).  While they are set, steps run the GROUPS instantiations of the dynamics kernel (and
-  // of the observation kernel when belief scores are collected) as two launches: the fused / lagged / one-launch rollout
-  // kernels and the split step are not instantiated for groups
+  // mechanism groups (sy_set_groups).  While they are set, every step path runs its GROUPS instantiation
   int grp_n = 0, grp_rep = 0;
   void* d_grp = nullptr;         // GroupRow [SY_MAX_GROUPS], rows [0, grp_n) in use
   void* d_grp_id = nullptr;      // int32 [B]
@@ -3404,6 +3326,17 @@ FusedFn lagged_fn(const SyEnv* e, bool groups = false) {
   if (groups) return e->cfg.belief ? lagged_fn_bw<BEL_WARPS, 1>(e->cfg.reward_mode, e->A) : lagged_fn_bw<0, 1>(e->cfg.reward_mode, e->A);
   return e->cfg.belief ? lagged_fn_bw<BEL_WARPS, 0>(e->cfg.reward_mode, e->A) : lagged_fn_bw<0, 0>(e->cfg.reward_mode, e->A);
 }
+template <int GR>
+FusedFn logic_fn_gr(int reward_mode, int A) {
+  const bool f64 = reward_mode == SY_REWARD_FP64;
+  if (A <= 4) return f64 ? sy_logic_kernel<SY_REWARD_FP64, 4, GR> : sy_logic_kernel<SY_REWARD_FP32, 4, GR>;
+  if (A <= 8) return f64 ? sy_logic_kernel<SY_REWARD_FP64, 8, GR> : sy_logic_kernel<SY_REWARD_FP32, 8, GR>;
+  return f64 ? sy_logic_kernel<SY_REWARD_FP64, 16, GR> : sy_logic_kernel<SY_REWARD_FP32, 16, GR>;
+}
+// the dynamics kernel of the two-launch step; groups: the GROUPS instantiation (mechanism groups are set)
+FusedFn logic_fn(const SyEnv* e, bool groups = false) {
+  return groups ? logic_fn_gr<1>(e->cfg.reward_mode, e->A) : logic_fn_gr<0>(e->cfg.reward_mode, e->A);
+}
 int lagged_threads(const SyEnv* e) { return ((e->cfg.belief ? BEL_WARPS : 0) + WR_WARPS + LOGIC_WARPS) * 32; }
 
 // eligibility of the lagged step kernel for this handle's shape: the default role split, and two CTAs per SM (with one
@@ -3456,8 +3389,6 @@ int raise_observe_smem_limit(int device, size_t bytes) {
   CUDA_TRY(cudaFuncSetAttribute(sy_observe_kernel<GEN_BEL_WARPS, GEN_WR_WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
   CUDA_TRY(cudaFuncSetAttribute(sy_observe_kernel<BEL_WARPS, WR_WARPS, WV_BULK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
   CUDA_TRY(cudaFuncSetAttribute(sy_observe_kernel<GEN_BEL_WARPS, GEN_WR_WARPS, WV_BULK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-  CUDA_TRY(cudaFuncSetAttribute(sy_observe_kernel<BEL_WARPS, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-  CUDA_TRY(cudaFuncSetAttribute(sy_observe_kernel<0, WR_WARPS, WV_ONES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
   CUDA_TRY(cudaFuncSetAttribute(sy_observe_kernel<BEL_WARPS, WR_WARPS, WV_LSU, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
   CUDA_TRY(cudaFuncSetAttribute(sy_observe_kernel<GEN_BEL_WARPS, GEN_WR_WARPS, WV_LSU, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
   CUDA_TRY(cudaFuncSetAttribute(sy_observe_kernel<BEL_WARPS, WR_WARPS, WV_BULK, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
@@ -3713,9 +3644,6 @@ void sy_destroy(SyEnv* e) {
   for (void* ptr : {e->d_grp, e->d_grp_id, e->d_grp_id_new, e->d_grp_bad, e->d_grp_stats})
     if (ptr) cudaFree(ptr);
   if (e->aux_stream) cudaStreamDestroy(e->aux_stream);
-  if (e->split_stream) cudaStreamDestroy(e->split_stream);
-  for (cudaEvent_t ev : {e->ev_split_start, e->ev_split_logic, e->ev_split_belief})
-    if (ev) cudaEventDestroy(ev);
   if (e->ev_main) cudaEventDestroy(e->ev_main);
   if (e->ev_fork) cudaEventDestroy(e->ev_fork);
   if (e->ev_join) cudaEventDestroy(e->ev_join);
@@ -3732,9 +3660,8 @@ int sy_set_option(SyEnv* e, int32_t option, int32_t value) {
         return fail(SY_ERR_INVALID_ARGUMENT, "SY_OPT_STEP_KERNEL: 0 (fused), 1 (two kernels) or 2 (auto)");
       e->opt_fused = value;
       return SY_OK;
-    case SY_OPT_NF_FILL:
+    case SY_OPT_NF_FILL:  // accepted and ignored (include/sy_env.h)
       if (value != 0 && value != 1) return fail(SY_ERR_INVALID_ARGUMENT, "SY_OPT_NF_FILL: 0 or 1");
-      e->opt_fill = value;
       return SY_OK;
     case SY_OPT_WRITER_PATH:
       if (value != SY_WRITER_BULK && value != SY_WRITER_LSU) return fail(SY_ERR_INVALID_ARGUMENT, "SY_OPT_WRITER_PATH: 0 (bulk) or 1 (LSU)");
@@ -4131,33 +4058,11 @@ int sy_reset(SyEnv* e, const uint8_t* reset_mask, const int32_t* init_pos, const
 }  // extern "C"
 
 namespace {
-// after_logic (optional): recorded between the two kernels -- rewards / flags are final once the logic kernel is done
 bool fused_eligible(const SyEnv* e, const SyObs* ob) {
   if (!e->fused_ok || e->opt_fused == SY_STEP_TWO_KERNELS || !ob) return false;
   if (e->opt_fused == SY_STEP_AUTO && (e->cfg.num_envs + TILE - 1) / TILE > e->f_grid) return false;  // more than one wave of tiles
   const uintptr_t bits = reinterpret_cast<uintptr_t>(ob->action_mask) | reinterpret_cast<uintptr_t>(ob->node_features_u8 ? (void*)ob->node_features_u8 : (void*)ob->node_features);
   return (bits & 15u) == 0;  // bulk stores need 16-byte aligned streams
-}
-
-// next_actions (+ counter): a fused launch also draws the next step's random actions; *fused_sampled reports whether it did
-void launch_logic(const SyEnv* e, const Params& p, unsigned grid, cudaStream_t ls) {
-  const bool f64 = e->cfg.reward_mode == SY_REWARD_FP64, pdl = e->opt_pdl != 0;
-  if (p.grp_n) {  // mechanism groups
-    if (p.A <= 4) launch_ex(f64 ? sy_logic_kernel<SY_REWARD_FP64, 4, 1> : sy_logic_kernel<SY_REWARD_FP32, 4, 1>, grid, LOGIC_THREADS, 0, ls, pdl, p);
-    else if (p.A <= 8) launch_ex(f64 ? sy_logic_kernel<SY_REWARD_FP64, 8, 1> : sy_logic_kernel<SY_REWARD_FP32, 8, 1>, grid, LOGIC_THREADS, 0, ls, pdl, p);
-    else launch_ex(f64 ? sy_logic_kernel<SY_REWARD_FP64, 16, 1> : sy_logic_kernel<SY_REWARD_FP32, 16, 1>, grid, LOGIC_THREADS, 0, ls, pdl, p);
-    return;
-  }
-  if (p.A <= 4) {
-    if (f64) launch_ex(sy_logic_kernel<SY_REWARD_FP64, 4>, grid, LOGIC_THREADS, 0, ls, pdl, p);
-    else launch_ex(sy_logic_kernel<SY_REWARD_FP32, 4>, grid, LOGIC_THREADS, 0, ls, pdl, p);
-  } else if (p.A <= 8) {
-    if (f64) launch_ex(sy_logic_kernel<SY_REWARD_FP64, 8>, grid, LOGIC_THREADS, 0, ls, pdl, p);
-    else launch_ex(sy_logic_kernel<SY_REWARD_FP32, 8>, grid, LOGIC_THREADS, 0, ls, pdl, p);
-  } else {
-    if (f64) launch_ex(sy_logic_kernel<SY_REWARD_FP64, 16>, grid, LOGIC_THREADS, 0, ls, pdl, p);
-    else launch_ex(sy_logic_kernel<SY_REWARD_FP32, 16>, grid, LOGIC_THREADS, 0, ls, pdl, p);
-  }
 }
 
 // the lagged kernel carries pending observations: always (option on), or when the batch is one wave of it (auto)
@@ -4167,6 +4072,8 @@ bool use_lagged(const SyEnv* e) {
   return (e->cfg.num_envs + TILE - 1) / TILE <= e->lag_slots;
 }
 
+// after_logic (optional): recorded between the two kernels -- rewards / flags are final once the logic kernel is done.
+// next_actions (+ counter): a fused launch also draws the next step's random actions; *fused_sampled reports whether it did.
 // defer: leave the dense observations of the new state pending (sy_step_deferred); the next call writes them
 int step_impl(SyEnv* e, const int64_t* actions, const int32_t* actions32, const SyState* st, const SyObs* ob, const SyOut* out,
               sy_stream_t stream, cudaEvent_t after_logic = nullptr, const int16_t* actions16 = nullptr,
@@ -4218,7 +4125,7 @@ int step_impl(SyEnv* e, const int64_t* actions, const int32_t* actions32, const 
         g_launches++;
         CUDA_TRY(cudaGetLastError());
       }
-      launch_logic(e, p, grid, s);
+      launch_ex(logic_fn(e, p.grp_n > 0), grid, LOGIC_THREADS, 0, s, e->opt_pdl != 0, p);
     }
     g_launches++;
     CUDA_TRY(cudaGetLastError());
@@ -4261,59 +4168,15 @@ int step_impl(SyEnv* e, const int64_t* actions, const int32_t* actions32, const 
     nf_written_set(e, st, ob);
     return SY_OK;
   }
-  // Split step: the state-independent zero fill of float32 node_features (63 % of the bytes) goes to the TMA engine in
-  // its own tiny kernel on the caller's stream while the dynamics kernel runs on the handle's split stream; afterwards
-  // the belief propagation (split stream) and the writers of the ones (caller's stream) run next to each other.  Both
-  // join on the caller's stream before step_impl returns (events; capturable in a CUDA graph as a DAG).
-  const bool split = e->opt_fill && !ob->node_features_u8 && !p.wr_bulk && (reinterpret_cast<uintptr_t>(ob->node_features) & 15u) == 0 &&
-                     !p.dbg_skip && !e->bel_share_csr && e->cfg.num_envs >= SPLIT_MIN_ENVS && !e->grp_n;
-  cudaStream_t ls = s;  // stream of the dynamics kernel
-  if (split) {
-    if (!e->split_stream) {
-      CUDA_TRY(cudaStreamCreateWithFlags(&e->split_stream, cudaStreamNonBlocking));
-      CUDA_TRY(cudaEventCreateWithFlags(&e->ev_split_start, cudaEventDisableTiming));
-      CUDA_TRY(cudaEventCreateWithFlags(&e->ev_split_logic, cudaEventDisableTiming));
-      CUDA_TRY(cudaEventCreateWithFlags(&e->ev_split_belief, cudaEventDisableTiming));
-      int sms = 0;
-      CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->cfg.device));
-      e->fill_grid = sms;
-    }
-    CUDA_TRY(cudaEventRecord(e->ev_split_start, s));
-    CUDA_TRY(cudaStreamWaitEvent(e->split_stream, e->ev_split_start, 0));
-    sy_fill_kernel<<<(unsigned)e->fill_grid, FILL_THREADS, 0, s>>>(reinterpret_cast<uint8_t*>(ob->node_features),
-                                                                  (size_t)p.B * p.N * p.A * sizeof(float));
-    g_launches++;
-    CUDA_TRY(cudaGetLastError());
-    p.nf_prefilled = 1;
-    ls = e->split_stream;
-  } else if (nf_gran && !p.wr_bulk && !p.dbg_skip) {
+  if (nf_gran && !p.wr_bulk && !p.dbg_skip) {
     // the buffer holds the one-hot of the entry state: the dynamics kernel zeroes its granules, the writers store only
     // the new ones (every other path above, and a fresh or different buffer, writes the whole one-hot)
     p.nf_incr = nf_gran;
   }
-  if (!(p.dbg_skip & 32)) launch_logic(e, p, grid, ls);
+  if (!(p.dbg_skip & 32)) launch_ex(logic_fn(e, p.grp_n > 0), grid, LOGIC_THREADS, 0, s, e->opt_pdl != 0, p);
   g_launches++;
   CUDA_TRY(cudaGetLastError());
-  if (after_logic) CUDA_TRY(cudaEventRecord(after_logic, ls));
-  if (split) {
-    CUDA_TRY(cudaEventRecord(e->ev_split_logic, ls));
-    if (p.belief_on) {  // belief propagation: one role per launch, next to the writers
-      sy_observe_kernel<BEL_WARPS, 0><<<grid, BEL_WARPS * 32, e->bel_smem, ls>>>(p);
-      g_launches++;
-      CUDA_TRY(cudaGetLastError());
-      CUDA_TRY(cudaEventRecord(e->ev_split_belief, ls));
-    }
-    CUDA_TRY(cudaStreamWaitEvent(s, e->ev_split_logic, 0));
-    Params pw = p;  // writers only: their staging area starts at the beginning of the dynamic shared memory
-    pw.wr_off = 0;
-    pw.wr_off_csr = e->wr_off_csr - e->wr_off;
-    sy_observe_kernel<0, WR_WARPS, WV_ONES><<<grid, WR_WARPS * 32, e->obs_smem - (size_t)e->wr_off, s>>>(pw);
-    g_launches++;
-    CUDA_TRY(cudaGetLastError());
-    if (p.belief_on) CUDA_TRY(cudaStreamWaitEvent(s, e->ev_split_belief, 0));
-    nf_written_set(e, st, ob);
-    return SY_OK;
-  }
+  if (after_logic) CUDA_TRY(cudaEventRecord(after_logic, s));
   if (!(p.dbg_skip & 16)) launch_observe(e, p, grid, s);
   g_launches++;
   CUDA_TRY(cudaGetLastError());

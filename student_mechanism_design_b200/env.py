@@ -392,7 +392,7 @@ class BatchedScotlandYardEnv:
         """Tuning knobs of the handle (results are identical for every setting; include/sy_env.h SY_OPT_*):
         `step_kernel` = "auto" (default: the fused persistent kernel for batches of up to ~9 500 envs, else two kernels)
         | "fused" | "two_kernels"; `writer_path` of the two-kernel path's observation kernel = "lsu" (default) | "bulk"
-        (TMA bulk stores); `nf_fill` = "off" (default) | "on" (split step: TMA fill kernel next to the dynamics);
+        (TMA bulk stores); `nf_fill` = "off" | "on": accepted and ignored (the split step it selected is gone);
         `lagged_kernel` = "auto" (default: deferred steps and the random rollouts run observations of step k + dynamics of
         step k+1 as one launch when the batch is one wave of that kernel, <= ~9 500 envs) | "on" | "off"; `tail_split` =
         "on" (default) | "off" (the observation grid's partly filled last wave cut into parts); `rollout_kernel` = "on"

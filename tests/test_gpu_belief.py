@@ -270,7 +270,6 @@ def _with_oracle(pool, B, P, money, reveal, seed, gid=None):
 LAUNCH = {
     "two_kernels": [("step_kernel", "two_kernels")],
     "fused": [("step_kernel", "fused")],
-    "split": [("step_kernel", "two_kernels"), ("nf_fill", "on")],
     "pdl": [("step_kernel", "two_kernels"), ("pdl", "on")],
 }
 

@@ -41,8 +41,7 @@ def _pair(N, E, P, money, B, seed, *, toll, belief, reveal, graphs=1, writer=Non
     env = pkg.BatchedScotlandYardEnv(B, P, money, graphs=pool, seed=seed, auto_reset=True, tolls=toll, belief=belief,
                                      reveal_interval=reveal, keep_reward64=True, **env_kw)
     # "fused": one persistent kernel | two kernels with: "lsu" = all observation stores through the LSU (the default for
-    # large batches) | "bulk" = chunk images + bulk stores in the observation kernel | "split" = TMA fill kernel next to
-    # the dynamics kernel, then belief and writers as two concurrent kernels
+    # large batches) | "bulk" = chunk images + bulk stores in the observation kernel
     if writer == "lsu_lagged":  # rollouts: software-pipelined deferred steps through the lagged kernel
         env.set_option("lagged_kernel", "on")
         writer = "lsu"
@@ -53,7 +52,6 @@ def _pair(N, E, P, money, B, seed, *, toll, belief, reveal, graphs=1, writer=Non
         env.set_option("step_kernel", "fused" if writer == "fused" else "two_kernels")
         if writer != "fused":
             env.set_option("writer_path", "bulk" if writer == "bulk" else "lsu")
-            env.set_option("nf_fill", "on" if writer == "split" else "off")
     cfg = so.OracleConfig(num_police=P, agent_money=money, toll=toll, belief=belief, reveal_interval=reveal)
     # the env's default graph assignment: blocks of 32 consecutive envs share a graph
     gid = (np.arange(B) // 32) % graphs
@@ -113,7 +111,7 @@ def _rollout_against_oracle(env, ob, steps, belief, dense_every=1):
     return done
 
 
-@pytest.mark.parametrize("writer", ["lsu", "lsu_pdl", "fused", "bulk", "split"])
+@pytest.mark.parametrize("writer", ["lsu", "lsu_pdl", "fused", "bulk"])
 def test_config3_full_size_matches_oracle(torch_cuda, writer):
     """BASELINE config 3 exactly as benchmarked: 200 nodes / 400 edges / 6 police, budget 20, toll 1, belief on,
     reveal every 5, 65 536 envs, same-step auto-reset, 25 steps -- every tile of the 2 048-tile grid and all statistics
@@ -151,7 +149,7 @@ def test_config3_ragged_batch_graph_pool(torch_cuda):
     env.close()
 
 
-@pytest.mark.parametrize("writer", ["lsu", "lsu_lagged", "lsu_pdl", "fused", "split"])
+@pytest.mark.parametrize("writer", ["lsu", "lsu_lagged", "lsu_pdl", "fused"])
 def test_timed_path_graph_replay_matches_oracle(torch_cuda, writer):
     """The path bench.py times -- capture_rollout (sy_rollout_random_dev: device-resident step counter; "lsu", the
     default at this size: two launches per step, the sampler of step k+1 forked next to the observation kernel of step

@@ -623,7 +623,7 @@ GUARD_SHAPES = [  # (N, E, P, B, belief, reveal, tolls), as tests/test_gpu_guard
     (200, 400, 6, 4096 + 19, True, 5, 1),
     (333, 600, 4, 300, True, 5, 1),
 ]
-GUARD_VARIANTS = ["default", "bulk", "fused", "split", "lagged"]
+GUARD_VARIANTS = ["default", "bulk", "fused", "two_kernels", "lagged"]
 
 
 @pytest.mark.parametrize("variant", GUARD_VARIANTS)
@@ -644,9 +644,8 @@ def test_guards_with_fewer_police(torch_cuda, shape, variant):
             env.set_option("writer_path", "bulk")
         elif variant == "fused":
             env.set_option("step_kernel", "fused")
-        elif variant == "split":
+        elif variant == "two_kernels":
             env.set_option("step_kernel", "two_kernels")
-            env.set_option("nf_fill", "on")
         elif variant == "lagged":
             env.set_option("step_kernel", "two_kernels")
             env.set_option("lagged_kernel", "on")

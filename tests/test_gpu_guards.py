@@ -21,7 +21,7 @@ SHAPES = [  # (N, E, P, B, belief, reveal, tolls)
     (333, 600, 4, 300, True, 5, 1),
     (1000, 2000, 6, 330 * 32 - 21, True, 5, 1),
 ]
-VARIANTS = ["default", "bulk", "fused", "split", "lagged"]
+VARIANTS = ["default", "bulk", "fused", "two_kernels", "lagged"]
 
 
 def _configure(env, variant):
@@ -30,9 +30,8 @@ def _configure(env, variant):
         env.set_option("writer_path", "bulk")
     elif variant == "fused":
         env.set_option("step_kernel", "fused")
-    elif variant == "split":
+    elif variant == "two_kernels":
         env.set_option("step_kernel", "two_kernels")
-        env.set_option("nf_fill", "on")
     elif variant == "lagged":
         env.set_option("step_kernel", "two_kernels")
         env.set_option("lagged_kernel", "on")

@@ -386,7 +386,7 @@ PATH_ROWS = {  # name: (env kwargs, sequence)
     "plain_full_2mod4": (dict(N=202, P=8), _seq_granule(FULL)),
     "fused": ({}, _seq_option("step_kernel", "fused", "two_kernels")),
     "bulk_writer": ({}, _seq_option("writer_path", "bulk", "lsu")),
-    "nf_fill": (dict(B=8192 + 37), _seq_option("nf_fill", "on", "off")),
+    "nf_fill": (dict(B=8192 + 37), _seq_fast_option("nf_fill", "on")),  # ignored: the fast path at the old split size
     "pdl": ({}, _seq_fast_option("pdl", "on")),
     "tail_split_off": ({}, _seq_fast_option("tail_split", "off")),
     "deferred_then_plain": ({}, _seq_deferred(False)),
